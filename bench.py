@@ -2,12 +2,12 @@
 """Headline benchmark: MCTS simulations/s (and self-play moves/s) of AlphaZero-mode 15x15 Gomoku
 self-play, 400 simulations per move, 4096 concurrent games per GPU (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--games G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--games G] [--dump-outputs DIR]
 
 A "step" is one self-play move for every game on the GPU: Gumbel noise, one full 400-simulation
 search per game, decision, do_move + win/draw detection, restart of finished games.  Rank 0
-prints ONE JSON line.  `--impl reference` times the UNMODIFIED reference (baseline/_ref, installed by
-baseline/install_reference.py; its own AlphaZeroMCTS.search in one process per host core, plus its production
+prints ONE JSON line; with --dump-outputs it also writes the last step's outputs to DIR (dump_last_step).
+`--impl reference` times the UNMODIFIED reference (baseline/_ref, installed by baseline/install_reference.py; its own AlphaZeroMCTS.search in one process per host core, plus its production
 topology universal_worker x W + inference_server_worker at N = 1) on the same config; the C port of the search
 (oracle/) is timed beside it as a second figure, and stands in alone if baseline/_ref is absent.
 """
@@ -25,6 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: the benchmark writes nothing into it
 
 N, N_IN_ROW, S, K_TOP = 15, 5, 400, 16
 A = N * N
@@ -654,6 +655,42 @@ def weight_broadcast_leg(dev, rank, world):
             "ranks_identical_after": bool(lo.item() == hi.item())}
 
 
+DUMP_MAX_GAMES = 4096          # 4096 games x (policy f64 + board f32) = 11 MB: a dump stays small at any --games
+
+
+def dump_last_step(out_dir, G, dev, n_steps):
+    """--dump-outputs: what the timed path computes for rank 0's games in step `n_steps` (= warmup + timed steps), the
+    arrays its caller reads from the TrajectoryStore and the engine: policy f64 [g, A], root value f64 [g], action [g],
+    board after the move f32 [g, A], winner [g] (+-1, 0 draw, 2 game goes on), game index [g] -- all G games, or a
+    fixed seeded sample of DUMP_MAX_GAMES.  The persistent kernel hands the timed moves to the games by a ticket
+    counter, so how many of them each game gets, and so which of its moves falls in the last step, depends on timing.
+    To give the same outputs for the same arguments, the dump replays the games on a fresh engine (same roots, seeds
+    and kernel) in one-move launches, in which every game makes exactly one move, and records the last one."""
+    import torch
+    from datou_gomoku_muzero_b200.engine import SearchEngine
+    from datou_gomoku_muzero_b200.selfplay import SelfPlayEngine
+    from datou_gomoku_muzero_b200.trajectory import TrajectoryStore
+    eng = SearchEngine(G, board_size=N, n_in_row=N_IN_ROW, num_simulations=S, num_top_actions=K_TOP, device=dev)
+    sp = SelfPlayEngine(eng, "e0", seed=E0_SEED, logit_div=LOGIT_DIV, noise_seed=1000)
+    eng.set_roots(*staggered_positions(G, 0))
+    for _ in range(n_steps - 1):
+        sp.play(moves_per_game=1)
+    # a fresh store puts game g's next move in slot g; with no spare slot a game that ends there stays on its final board
+    last = TrajectoryStore(eng, extra_slots=0, max_moves=1)
+    sp.play(moves_per_game=1, traj=last)
+    fin = last.fin_queue[:int(last.fin_count.item())].long()
+    winner = torch.full((G,), 2, dtype=torch.int32, device=dev)
+    winner[fin[:, 1]] = fin[:, 3].int()
+    games = np.arange(G) if G <= DUMP_MAX_GAMES else np.sort(np.random.RandomState(0).choice(G, DUMP_MAX_GAMES, replace=False))
+    sel = torch.as_tensor(games, device=dev)
+    out = {"policy": last.policy[sel, 0], "value": last.value[sel, 0], "action": last.action[sel, 0].double(),
+           "board": eng.get_roots()[0].reshape(G, A)[sel].float(), "winner": winner[sel].double(),
+           "game": torch.as_tensor(games, dtype=torch.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -868,6 +905,8 @@ def run_ours(args):
             out["reanalysis"] = {"error": repr(ex)[:200]}
     if not args.no_cpu_baseline and world == 1:  # reported on rank 0 at N=1 only
         out["cpu_baseline"] = cpu_baseline_leg(args.cpu_seconds)
+    if args.dump_outputs:
+        dump_last_step(args.dump_outputs, G, dev, args.warmup + args.steps)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -890,7 +929,13 @@ def main():
     ap.add_argument("--reanalysis-positions", type=int, default=1_000_000)
     ap.add_argument("--ref-topology-seconds", type=float, default=60.0,
                     help="--impl reference at N = 1: seconds of the reference's universal_worker + inference_server topology (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="--impl ours: write the last step's outputs to DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU arm computes (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)
