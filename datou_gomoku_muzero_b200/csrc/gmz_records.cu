@@ -13,6 +13,7 @@
 
 #include "../../include/gmz.h"
 #include "gmz_common.cuh"
+#include "gmz_tactics.cuh"
 
 extern "C" void gmz_set_error_(const char *msg);
 static int rc_fail(const char *m) { gmz_set_error_(m); return 1; }
@@ -31,6 +32,52 @@ extern "C" size_t gmz_move_record_bytes(int board_size)
 {
     if (board_size < 1 || board_size > GMZ_MAX_BOARD) return 0;
     return rec_stride(board_size * board_size);
+}
+
+// Missed-win flags of packed move records (workers.py:191-203): one CTA per record, one thread per cell.  The record's
+// board (before the move, absolute colours) is classified for the side in the header's to_move -- not move parity,
+// so a game started from a mid-game position gets the right colour -- and reduced to one byte:
+//   bit 0: the mover had a winning move (some cell class > 0), bit 1: the mover had a five (some cell class == 1),
+//   bit 2: the played cell (header action; outside [0, A) counts as class 0) has class > 0.
+__global__ void __launch_bounds__(512)
+k_records_tactics(const unsigned char *records, size_t stride, int N, int n_in_row, uint8_t *out_flags)
+{
+    __shared__ int8_t sb[GMZ_MAX_BOARD * GMZ_MAX_BOARD];
+    const int A = N * N;
+    const unsigned char *rec = records + (size_t)blockIdx.x * stride;
+    const int8_t *brd = reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * A);
+    for (int i = threadIdx.x; i < A; i += blockDim.x) sb[i] = brd[i];
+    const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
+    const int P = h->to_move >= 0 ? 1 : -1, action = h->action;
+    __syncthreads();
+    int any = 0, five = 0, played = 0;
+    for (int cell = threadIdx.x; cell < A; cell += blockDim.x) {
+        const int cls = gmz_tactics_cell_class(sb, N, n_in_row, P, cell);
+        any |= cls > 0;
+        five |= cls == 1;
+        played |= cell == action && cls > 0;
+    }
+    any = __syncthreads_or(any);
+    five = __syncthreads_or(five);
+    played = __syncthreads_or(played);
+    if (threadIdx.x == 0) out_flags[blockIdx.x] = (uint8_t)((any ? 1 : 0) | (five ? 2 : 0) | (played ? 4 : 0));
+}
+
+extern "C" int gmz_records_tactics(const void *records, int64_t n_records, int board_size, int n_in_row, uint8_t *out_flags,
+                                   gmz_stream stream)
+{
+    if (!records || !out_flags) return rc_fail("gmz_records_tactics: null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail("gmz_records_tactics: board_size out of range");
+    if (n_in_row < 1) return rc_fail("gmz_records_tactics: n_in_row must be >= 1");
+    if (n_records < 0 || n_records > 0x7fffffff) return rc_fail("gmz_records_tactics: n_records out of range");
+    if (n_records == 0) return 0;
+    const int A = board_size * board_size;
+    int threads = ((A + 31) / 32) * 32;          // the block-size rule of gmz_tactics_classify
+    if (threads > 512) threads = 512;
+    k_records_tactics<<<(unsigned)n_records, threads, 0, (cudaStream_t)stream>>>((const unsigned char *)records, rec_stride(A),
+                                                                               board_size, n_in_row, out_flags);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : rc_fail(cudaGetErrorString(e));
 }
 
 __device__ __forceinline__ float rec_final_reward(int i, int T, int winner)   // workers.py:183-187

@@ -1,13 +1,11 @@
 // gmz_tactics.cu -- the reference's tactical move classifier find_winning_moves_rebuilt
 // (workers.py:49-123) for a batch of boards: one CTA per board, one thread per cell.
-// Class per empty cell: 1 = 'five' (placing the stone wins, game.py:25-58), 2 = 'open_four',
-// 3 = 'combo' (>= 2 blocked fours, blocked four + open three, or >= 2 open threes), 0 = none.
-// Patterns are matched anywhere inside the 9-cell line centred on the move, off-board cells count
-// as opponent stones, each pattern at most once per direction -- exactly as the reference does.
+// The per-cell classes (gmz_tactics_cell_class) are defined in gmz_tactics.cuh.
 #include <stdint.h>
 
 #include "../../include/gmz.h"
 #include "gmz_common.cuh"
+#include "gmz_tactics.cuh"
 
 extern "C" void gmz_set_error_(const char *msg);
 
@@ -18,46 +16,9 @@ k_tactics(const int8_t *boards, const int8_t *players, int N, int n_in_row, int8
     const int A = N * N, b = blockIdx.x;
     for (int i = threadIdx.x; i < A; i += blockDim.x) sb[i] = boards[(size_t)b * A + i];
     __syncthreads();
-    const int P = players[b] >= 0 ? 1 : -1, O = -P;
-    const int DR[4] = {0, 1, 1, 1}, DC[4] = {1, 0, 1, -1};
+    const int P = players[b] >= 0 ? 1 : -1;
     for (int cell = threadIdx.x; cell < A; cell += blockDim.x) {
-        int cls = 0;
-        if (sb[cell] == 0) {
-            const int r = cell / N, c = cell % N;
-            bool five = false;
-            int open_four = 0, blocked_four = 0, open_three = 0;
-            for (int d = 0; d < 4; ++d) {
-                // check_win with the stone placed: contiguous run through (r,c), up to n_in_row+1 each way
-                int cnt = 1;
-                for (int s = -1; s <= 1; s += 2)
-                    for (int i = 1; i < n_in_row + 2; ++i) {
-                        const int rr = r + s * i * DR[d], cc = c + s * i * DC[d];
-                        if (rr >= 0 && rr < N && cc >= 0 && cc < N && sb[rr * N + cc] == P) ++cnt; else break;
-                    }
-                if (cnt >= n_in_row) five = true;
-                // the 9-cell line as two bit masks (mine / empty); everything else is a block
-                unsigned mine = 0, empty = 0;
-                for (int i = -4; i <= 4; ++i) {
-                    const int rr = r + i * DR[d], cc = c + i * DC[d];
-                    int v = O;
-                    if (rr >= 0 && rr < N && cc >= 0 && cc < N) v = (i == 0) ? P : sb[rr * N + cc];
-                    if (v == P) mine |= 1u << (i + 4); else if (v == 0) empty |= 1u << (i + 4);
-                }
-                const unsigned block = ~(mine | empty) & 0x1ffu;
-                bool of = false, bf = false, ot = false;
-                for (int i = 0; i < 4; ++i)          // (0,P,P,P,P,0)
-                    of = of || ((((empty >> i) & 0x21u) == 0x21u) && (((mine >> i) & 0x1eu) == 0x1eu));
-                for (int i = 0; i < 5; ++i) {
-                    const unsigned m = (mine >> i) & 0x1fu, e = (empty >> i) & 0x1fu, k = (block >> i) & 0x1fu;
-                    bf = bf || (m == 0x0eu && ((k == 0x01u && e == 0x10u) || (e == 0x01u && k == 0x10u)));   // (X,P,P,P,0) / (0,P,P,P,X)
-                    ot = ot || (m == 0x0eu && e == 0x11u);                                                      // (0,P,P,P,0)
-                }
-                open_four += of; blocked_four += bf; open_three += ot;
-            }
-            if (five) cls = 1;
-            else if (open_four > 0) cls = 2;
-            else if (blocked_four >= 2 || (blocked_four >= 1 && open_three >= 1) || open_three >= 2) cls = 3;
-        }
+        const int cls = gmz_tactics_cell_class(sb, N, n_in_row, P, cell);
         out[(size_t)b * A + cell] = (int8_t)cls;
     }
 }

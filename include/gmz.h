@@ -269,6 +269,13 @@ int gmz_traj_pack(const gmz_traj *traj, int board_size, const int32_t *fin, int 
  * (loss.py:37-51).  Outputs as gmz_build_batch. */
 int gmz_records_batch(const void *ring, int64_t capacity, int board_size, const int64_t *positions, int batch, int unroll,
                       int rot_k, int flip, float *obs, int32_t *act, float *rew, double *pi, float *val, gmz_stream stream);
+/* Missed-win flags of n_records consecutive records (a packed block or a stretch of the ring), read in place: the
+ * record's board is classified like gmz_tactics_classify for the side in its to_move, out_flags uint8 [n_records] =
+ * bit 0: the mover had a winning move, bit 1: the mover had a five, bit 2: the played action was one of them
+ * (an action outside [0, A) is not).  A missed win (workers.py:191-203) is bit 0 without bit 2, a missed five
+ * additionally has bit 1.  n_records = 0 is a no-op. */
+int gmz_records_tactics(const void *records, int64_t n_records, int board_size, int n_in_row, uint8_t *out_flags,
+                        gmz_stream stream);
 
 /* ---- tactics classifier (find_winning_moves_rebuilt, workers.py:49-123) ---- */
 /* boards int8 [B,A], players int8 [B] (the side to move) -> out_cls int8 [B,A]: per empty cell
