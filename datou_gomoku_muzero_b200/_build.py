@@ -13,7 +13,7 @@ SOURCES = ["gmz_engine.cu", "gmz_per.cu", "gmz_slices.cu", "gmz_tactics.cu", "gm
 # the persistent play kernel: one object per (MuZero mode, float32 accumulation), built in parallel
 PLAY_SOURCE = "gmz_play_inst.cu"
 PLAY_VARIANTS = [(0, 0), (0, 1), (1, 0), (1, 1)]
-HEADERS = ["gmz_common.cuh", "gmz_tree.cuh", "gmz_play.cuh", "gmz_tactics.cuh", "gmz_internal.h", os.path.join("..", "..", "include", "gmz.h")]
+HEADERS = ["gmz_common.cuh", "gmz_tree.cuh", "gmz_play.cuh", "gmz_tactics.cuh", "gmz_records.cuh", "gmz_internal.h", os.path.join("..", "..", "include", "gmz.h")]
 # -fmad=false: the search's float64 / float32 arithmetic must round once per operation, like the
 # reference's Python floats / NumPy scalars (SURVEY.md App. A.7); an FMA would change visit counts.
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false",

@@ -70,6 +70,9 @@ SIGNATURES = {
     "gmz_traj_pack": (C.c_int, [C.POINTER(GmzTraj), C.c_int, _P, C.c_int, _P, _P, C.c_int, _P, _P]),
     "gmz_records_batch": (C.c_int, [_P, C.c_int64, C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),
     "gmz_records_tactics": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int, _P, _P]),
+    "gmz_set_roots_from_records": (C.c_int, [_P, _P, C.c_int64, C.c_int64, C.c_int64, _P]),
+    "gmz_records_writeback": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_int64, _P, _P, _P]),
+    "gmz_records_retarget": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_int64, _P, C.c_int, _P]),
     "gmz_tactics_classify": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gmz_per_update": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int, _P]),
     "gmz_per_add": (C.c_int, [_P, C.c_int64, C.c_int64, _P, C.c_int, _P, _P]),

@@ -10,6 +10,7 @@
 #include <unordered_set>
 
 #include "gmz_internal.h"
+#include "gmz_records.cuh"
 #include "gmz_tree.cuh"
 #include "gmz_play.cuh"
 
@@ -52,20 +53,18 @@ static bool engine_live(const gmz_engine *e)
 // ---------------------------------------------------------------------------------------------
 // root positions
 // ---------------------------------------------------------------------------------------------
-// boards int8 [G,A] -> bitboards; one warp per game, ballots pack 32 cells at a time.
-__global__ void __launch_bounds__(CTA_THREADS)
-k_set_roots(Params p, const int8_t *boards, const int8_t *players, const int32_t *last_moves, const int32_t *move_counts)
+// board int8 [A] -> game g's bitboards; one warp per game, ballots pack 32 cells at a time.  b == NULL: a full board
+// of +1 stones (an inactive padding root).
+__device__ __forceinline__ void root_load(const Params &p, int g, int lane, const int8_t *b, int player, int last_move,
+                                          int move_count)
 {
-    const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
-    if (g >= p.G) return;
-    const int8_t *b = boards + (size_t)g * p.A;
     u64 P = 0, M = 0, V = 0;
     int nvalid = 0;
     for (int w = 0; w < GMZ_WORDS; ++w) {
         u64 pw = 0, mw = 0, vw = 0;
         for (int h = 0; h < 2; ++h) {
             const int a = 64 * w + 32 * h + lane;
-            const int c = a < p.A ? (int)b[a] : 2;
+            const int c = a < p.A ? (b ? (int)b[a] : 1) : 2;
             pw |= (u64)__ballot_sync(GMZ_FULL, c == 1) << (32 * h);
             mw |= (u64)__ballot_sync(GMZ_FULL, c == -1) << (32 * h);
             vw |= (u64)__ballot_sync(GMZ_FULL, c == 0) << (32 * h);
@@ -76,13 +75,36 @@ k_set_roots(Params p, const int8_t *boards, const int8_t *players, const int32_t
     GState *s = p.gs + g;
     if (lane < GMZ_WORDS) { s->p1[lane] = P; s->m1[lane] = M; s->valid[lane] = V; }
     if (lane == 0) {
-        s->to_move = players[g] >= 0 ? 1 : -1;
-        s->last_move = last_moves[g];
-        s->move_count = move_counts[g];
+        s->to_move = player >= 0 ? 1 : -1;
+        s->last_move = last_move;
+        s->move_count = move_count;
         s->active = nvalid > 0;
         s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
         s->winner = GMZ_WINNER_NONE;
     }
+}
+
+__global__ void __launch_bounds__(CTA_THREADS)
+k_set_roots(Params p, const int8_t *boards, const int8_t *players, const int32_t *last_moves, const int32_t *move_counts)
+{
+    const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
+    if (g >= p.G) return;
+    root_load(p, g, lane, boards + (size_t)g * p.A, players[g], last_moves[g], move_counts[g]);
+}
+
+// Roots from packed move records (re-analysis, workers.py:254-263): game g < n takes the record at ring position
+// (first + g) % capacity -- its board (before the move, absolute colours), and from the header the side to move (not
+// move parity: games started mid-game keep their colour), last move and move count.  Games n..G-1 get the full-board
+// padding root, inactive.
+__global__ void __launch_bounds__(CTA_THREADS)
+k_set_roots_records(Params p, const unsigned char *ring, size_t stride, int64_t capacity, int64_t first, int n)
+{
+    const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
+    if (g >= p.G) return;
+    if (g >= n) { root_load(p, g, lane, nullptr, 1, -1, 0); return; }
+    const unsigned char *rec = ring + (size_t)((first + g) % capacity) * stride;
+    const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
+    root_load(p, g, lane, reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * p.A), h->to_move, h->last_move, h->move_count);
 }
 
 __global__ void __launch_bounds__(CTA_THREADS) k_games_reset(Params p, const uint8_t *mask)
@@ -546,6 +568,18 @@ extern "C" int gmz_set_roots(gmz_engine *e, const int8_t *boards, const int8_t *
     if (!boards || !players || !last_moves || !move_counts) return fail("gmz_set_roots: null argument");
     k_set_roots<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, boards, players, last_moves, move_counts);
     return check_launch("k_set_roots");
+}
+extern "C" int gmz_set_roots_from_records(gmz_engine *e, const void *ring, int64_t capacity, int64_t first, int64_t n,
+                                          gmz_stream stream)
+{
+    if (!ring) return fail("gmz_set_roots_from_records: null argument");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return fail("gmz_set_roots_from_records: %s", m);
+    LIVE(e, "gmz_set_roots_from_records");
+    if (n > e->p.G) return fail("gmz_set_roots_from_records: n exceeds the engine's num_games");
+    if (n == 0) return 0;
+    k_set_roots_records<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, (const unsigned char *)ring, rec_stride(e->p.A), capacity, first,
+                                                              (int)n);
+    return check_launch("k_set_roots_records");
 }
 extern "C" int gmz_games_reset(gmz_engine *e, const uint8_t *mask, gmz_stream stream)
 {

@@ -10,24 +10,16 @@
 //     (workers.py:430-433) is gathered straight from the ring, D4 augmentation (loss.py:37-51) included.
 // Record layout (gmz_move_record_bytes): 64-byte header | policy f64[A] | obs f32[3A] | board i8[A] | pad to 16.
 #include <stdint.h>
+#include <stdio.h>
 
 #include "../../include/gmz.h"
 #include "gmz_common.cuh"
+#include "gmz_records.cuh"
 #include "gmz_tactics.cuh"
 
 extern "C" void gmz_set_error_(const char *msg);
 static int rc_fail(const char *m) { gmz_set_error_(m); return 1; }
 
-struct RecHeader {            // 64 bytes, see include/gmz.h gmz_move_record
-    int32_t game_seq, t, length, winner;
-    int32_t action, to_move, last_move, move_count;
-    float reward, value_target;
-    double search_value;
-    int32_t game, slot, pad0, pad1;
-};
-static_assert(sizeof(RecHeader) == 64, "record header must be 64 bytes");
-
-static inline size_t rec_stride(int A) { return ((size_t)64 + (size_t)21 * A + 15) / 16 * 16; }
 extern "C" size_t gmz_move_record_bytes(int board_size)
 {
     if (board_size < 1 || board_size > GMZ_MAX_BOARD) return 0;
@@ -233,4 +225,86 @@ extern "C" int gmz_records_batch(const void *ring, int64_t capacity, int board_s
                                                                        positions, batch, unroll, rot_k, flip ? 1 : 0, obs, act, rew, pi, val);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : rc_fail(cudaGetErrorString(e));
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Re-analysis of a stretch of the ring in place (workers.py:243-305): record k of the stretch sits at ring position
+// (first + k) % capacity.  gmz_set_roots_from_records (gmz_engine.cu) loads the roots, the search runs, then the two
+// kernels below put the results back.
+static int rc_fail2(const char *name, const char *m)
+{
+    char buf[256];
+    snprintf(buf, sizeof(buf), "%s: %s", name, m);
+    gmz_set_error_(buf);
+    return 1;
+}
+
+// The re-searched policy row k and root value k replace the record's policy bytes and header search_value; nothing
+// else in the record is written.  One warp per record.
+__global__ void __launch_bounds__(128)
+k_records_writeback(unsigned char *ring, size_t stride, int64_t capacity, int64_t first, int64_t n, int A, const double *policy,
+                    const double *value)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t k = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (k >= n) return;
+    unsigned char *rec = ring + (size_t)((first + k) % capacity) * stride;
+    double *pol = reinterpret_cast<double *>(rec + 64);
+    const double *src = policy + (size_t)k * A;
+    for (int c = lane; c < A; c += 32) pol[c] = src[c];
+    if (lane == 0) reinterpret_cast<RecHeader *>(rec)->search_value = value[k];
+}
+
+extern "C" int gmz_records_writeback(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *policy,
+                                     const double *value, gmz_stream stream)
+{
+    const char *name = "gmz_records_writeback";
+    if (!ring || !policy || !value) return rc_fail2(name, "null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return rc_fail2(name, m);
+    if (n == 0) return 0;
+    const int A = board_size * board_size;
+    k_records_writeback<<<(unsigned)((n + 3) / 4), 128, 0, (cudaStream_t)stream>>>((unsigned char *)ring, rec_stride(A), capacity,
+                                                                                   first, n, A, policy, value);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+}
+
+// New n-step value targets from the re-searched root values, with re-analysis arithmetic (reanalysis.reanalyse ->
+// compute_n_step_returns on float32 rewards, workers.py:291-292): each reward term a float32 product, summed in float32
+// in order, the bootstrap a float32 product, one float32 add.  (Self-play's k_traj_pack sums the rewards in float64.)
+// A record reads its own header and the search_value of the record n_steps later in the same game, which is live and
+// already rewritten: games sit whole and in move order in the ring, and the stretch covers whole games.
+__global__ void __launch_bounds__(256)
+k_records_retarget(unsigned char *ring, size_t stride, int64_t capacity, int64_t first, int64_t n, const double *dpow, int n_steps)
+{
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const int64_t p = (first + k) % capacity;
+    RecHeader *h = reinterpret_cast<RecHeader *>(ring + (size_t)p * stride);
+    const int t = h->t, T = h->length, winner = h->winner;
+    float acc = 0.0f;
+    for (int i = 0; i < n_steps && t + i < T; ++i) acc = __fadd_rn(acc, __fmul_rn((float)dpow[i], rec_final_reward(t + i, T, winner)));
+    float boot = 0.0f;
+    if ((int64_t)t + n_steps < T) {
+        const RecHeader *hb = reinterpret_cast<const RecHeader *>(ring + (size_t)((p + n_steps) % capacity) * stride);
+        boot = __fmul_rn((float)hb->search_value, (float)dpow[n_steps]);
+    }
+    h->value_target = __fadd_rn(acc, boot);
+}
+
+extern "C" int gmz_records_retarget(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *discount_pow,
+                                    int n_steps, gmz_stream stream)
+{
+    const char *name = "gmz_records_retarget";
+    if (!ring || !discount_pow) return rc_fail2(name, "null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return rc_fail2(name, m);
+    if (n_steps < 0) return rc_fail2(name, "n_steps must be >= 0");
+    if (n == 0) return 0;
+    const int A = board_size * board_size;
+    k_records_retarget<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>((unsigned char *)ring, rec_stride(A), capacity,
+                                                                                     first, n, discount_pow, n_steps);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
 }

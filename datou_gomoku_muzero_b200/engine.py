@@ -104,6 +104,14 @@ class SearchEngine:
         check(self.lib.gmz_set_roots(self.handle, _ptr(b), _ptr(pl), _ptr(lm), _ptr(mc), self._stream()), "gmz_set_roots")
         self.launches += 1
 
+    def set_roots_from_records(self, ring, capacity, first, n):
+        """Roots from `n` <= G packed move records of a ring (uint8 device tensor [capacity, stride]): game k takes the
+        record at ring position (first + k) % capacity -- its board, and from its header the side to move, last move and
+        move count; games n..G-1 become inactive.  Nothing is copied to or from the host."""
+        check(self.lib.gmz_set_roots_from_records(self.handle, _ptr(ring), int(capacity), int(first), int(n), self._stream()),
+              "gmz_set_roots_from_records")
+        self.launches += 1
+
     def reset_games(self, mask=None):
         m = None if mask is None else self._dev(mask, torch.uint8).reshape(self.G)
         check(self.lib.gmz_games_reset(self.handle, _ptr(m), self._stream()), "gmz_games_reset")

@@ -158,19 +158,25 @@ class _GumbelEngineMCTS(MCTS):
         for k in keys:
             b["d_" + k].copy_(b["h_" + k], non_blocking=True)
         eng.set_roots(b["d_boards"], b["d_players"], b["d_last"], b["d_mc"])
-        if b["evaluator"] == "e0":
-            eng.search_e0(b["d_gumbel"], b["eval_seed"], b["logit_div"])
-        else:
-            ev = b["evaluator"]
-            lg, v = ev(eng.root_obs())
-            eng.root_expand(lg, v, b["d_gumbel"])
-            for _ in range(eng.S - 1):
-                lg, v = ev(eng.select())
-                eng.expand_backup(lg, v)
+        search_roots(eng, b["d_gumbel"], b["evaluator"], b["eval_seed"], b["logit_div"])
         pol, val, act, _ = eng.finalize(want_visits=False)
         b["o_policy"].copy_(pol, non_blocking=True)
         b["o_value"].copy_(val, non_blocking=True)
         b["o_action"].copy_(act, non_blocking=True)
+
+
+def search_roots(eng, gumbel, evaluator="e0", eval_seed=0, logit_div=16):
+    """One search of every root loaded in `eng`, enqueued on the current stream (follow with eng.finalize): "e0" runs the
+    fused kernel (either engine mode); a callable f(obs) -> (logits, values) drives the stepwise kernels (AlphaZero
+    mode)."""
+    if isinstance(evaluator, str) and evaluator == "e0":
+        eng.search_e0(gumbel, eval_seed, logit_div)
+        return
+    lg, v = evaluator(eng.root_obs())
+    eng.root_expand(lg, v, gumbel)
+    for _ in range(eng.S - 1):
+        lg, v = evaluator(eng.select())
+        eng.expand_backup(lg, v)
 
 
 class PipelinedBatchSearch:

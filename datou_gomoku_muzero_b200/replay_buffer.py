@@ -165,6 +165,7 @@ class DeviceReplayBuffer:
                           augmentation while gathering (loss.py:37-51)
     update_priorities  = replay_buffer.py:98-103 on device tensors (td_errors float32, as the loss returns them)
     rewrite_targets    = the re-analysis write-back (db_manager.py:189-214) for records in the ring
+    reanalyse(engines) = Surge re-analysis (workers.py:243-305) of the records in the ring, in place, on the device
     """
 
     def __init__(self, capacity, board_size, device=None, unroll_steps=None):
@@ -233,6 +234,86 @@ class DeviceReplayBuffer:
             raise ValueError("ring position out of range")
         self.ring[pos, 64:64 + 8 * self.A] = pol.view(torch.uint8).reshape(pos.numel(), 8 * self.A)      # gmz_move_record: policy f64[A]
         self.ring[pos, 36:40] = val.view(torch.uint8).reshape(pos.numel(), 4)                             # header: value_target f32
+
+    def reanalyse(self, engines, first=None, count=None, evaluator="e0", eval_seed=0, logit_div=16, noise_seed=0):
+        """Surge re-analysis (workers.py:243-305) of the records in the ring, in place: every position is searched again
+        with the latest evaluator, its policy and root search value are replaced, and the n-step value targets of the
+        stretch are recomputed from the new root values (re-analysis arithmetic: float32 rewards, workers.py:291-292).
+        Observations, boards, actions, rewards and the PER tree are left as they are.
+
+        Which records: by default every live record, oldest first.  An explicit stretch (`first` = a ring position,
+        `count` records; either may be omitted: from the oldest live record / up to the newest) is widened to whole
+        games, as far as those games are still live -- the reference re-analyses whole GameRecords.  A stretch that
+        reaches outside the live records raises ValueError.  Returns the widened (first, count).
+
+        engines: SearchEngines of the buffer's board size.  The stretch goes through them G records per batch, batches
+        alternating between the engines, each on a stream of its own; the caller's current stream waits for all of them
+        and then runs the target recomputation, so later add_packed / batch / sample calls see the new bytes.  Loading the
+        roots overwrites an engine's games: do not pass the engine that is running self-play.
+        evaluator: "e0" (the fixed evaluator, either engine mode; eval_seed / logit_div as SearchEngine.search_e0) or a
+        callable f(obs f32 [G,3,N,N]) -> (logits, values) on AlphaZero-mode engines.  Noise is drawn on the device: record
+        k of the widened stretch uses Gumbel counters k*A .. k*A + A-1 of `noise_seed`, as reanalyse_positions gives its
+        position k.  Policies and values never go to the host; the only host read is the two boundary headers of an
+        explicit stretch."""
+        from .mcts import search_roots
+        engines = list(engines)
+        e0 = isinstance(evaluator, str)
+        if e0 and evaluator != "e0":
+            raise ValueError(f"unknown evaluator {evaluator!r}")
+        if not engines:
+            raise ValueError("reanalyse needs at least one engine")
+        for e in engines:
+            if e.N != self.N:
+                raise ValueError(f"engine board size {e.N} differs from the buffer's {self.N}")
+            if e.device != self.device:
+                raise ValueError(f"engine on {e.device}, buffer on {self.device}")
+            if not e0 and e.mode != "AlphaZero":
+                raise ValueError("a network evaluator needs AlphaZero-mode engines")
+        cap, live = self.capacity, self.sum_tree.count
+        oldest = self.sum_tree.write_ptr if live == cap else 0
+        if first is not None and not 0 <= int(first) < cap:
+            raise ValueError(f"first={first} is not a ring position (capacity {cap})")
+        rel = 0 if first is None else (int(first) - oldest) % cap          # offset from the oldest live record
+        n = live - rel if count is None else int(count)
+        if (first is not None and rel >= live) or n < 0 or rel + n > live:
+            raise ValueError(f"stretch first={first}, count={count} reaches outside the {live} live records")
+        if n > 0 and (first is not None or count is not None):
+            ends = torch.tensor([(oldest + rel) % cap, (oldest + rel + n - 1) % cap], device=self.device)
+            h = self.ring[ends, :12].cpu().numpy().view(np.int32)          # header: game_seq, t, length
+            end = rel + n + int(h[1, 2]) - 1 - int(h[1, 1])
+            rel = max(0, rel - int(h[0, 1]))                               # a cut oldest game: its live suffix
+            if end > live:
+                raise RuntimeError("ring records do not hold whole games")
+            n = end - rel
+        start = (oldest + rel) % cap
+        if n == 0:
+            return start, 0
+        cur = torch.cuda.current_stream(self.device)
+        streams = [torch.cuda.Stream(device=self.device) for _ in engines]
+        gumbel = [torch.empty((e.G, self.A), dtype=torch.float64, device=self.device) for e in engines]
+        for s in streams:
+            s.wait_stream(cur)
+        s0 = b = 0
+        while s0 < n:
+            i = b % len(engines)
+            e = engines[i]
+            k = min(e.G, n - s0)
+            pos = (start + s0) % cap
+            with torch.cuda.stream(streams[i]):
+                e.set_roots_from_records(self.ring, cap, pos, k)
+                e.fill_gumbel(gumbel[i], noise_seed, s0 * self.A)
+                search_roots(e, gumbel[i], evaluator, eval_seed, logit_div)
+                pol, val, _, _ = e.finalize(want_visits=False)
+                check(self.lib.gmz_records_writeback(_ptr(self.ring), cap, self.N, pos, k, _ptr(pol), _ptr(val), e._stream()),
+                      "gmz_records_writeback")
+            s0 += k
+            b += 1
+        for s in streams:
+            cur.wait_stream(s)
+        dpow = torch.tensor([config.DISCOUNT ** i for i in range(config.N_STEPS + 1)], dtype=torch.float64, device=self.device)
+        check(self.lib.gmz_records_retarget(_ptr(self.ring), cap, self.N, start, n, _ptr(dpow), int(config.N_STEPS),
+                                            self.sum_tree._stream()), "gmz_records_retarget")
+        return start, n
 
     def update_priorities(self, tree_indices, td_errors):
         if not config.ENABLE_PER:

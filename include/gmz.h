@@ -276,6 +276,23 @@ int gmz_records_batch(const void *ring, int64_t capacity, int board_size, const 
  * additionally has bit 1.  n_records = 0 is a no-op. */
 int gmz_records_tactics(const void *records, int64_t n_records, int board_size, int n_in_row, uint8_t *out_flags,
                         gmz_stream stream);
+/* Re-analysis of a stretch of the ring in place (workers.py:243-305).  A stretch is (first, n): record k sits at ring
+ * position (first + k) % capacity, 0 <= first < capacity, 0 <= n <= capacity; n = 0 is a no-op.
+ * gmz_set_roots_from_records: the engine's roots straight from records, n <= G.  Game k < n takes record k's board
+ *   (before the move), and its header's to_move (not move parity), last_move and move_count -- what gmz_set_roots does
+ *   with those fields; games n..G-1 become inactive (full-board padding, as reanalyse_positions pads).
+ * gmz_records_writeback: policy f64 [n,A] row k and value f64 [n] entry k (gmz_finalize's outputs) replace record k's
+ *   policy and header search_value; nothing else is written.
+ * gmz_records_retarget: record k's value_target from its own header (t, length, winner) and the search_value of the
+ *   record n_steps later in the same game, with re-analysis arithmetic (float32 rewards, workers.py:291-292): reward
+ *   terms (float)discount_pow[i] * r in float32, summed in float32 for i = 0..n_steps-1, plus the float32 bootstrap
+ *   (float)search_value * (float)discount_pow[n_steps].  The stretch must hold whole live games (their later moves are
+ *   read).  discount_pow f64 [n_steps+1] = discount**i as the host computes them. */
+int gmz_set_roots_from_records(gmz_engine *e, const void *ring, int64_t capacity, int64_t first, int64_t n, gmz_stream stream);
+int gmz_records_writeback(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *policy,
+                          const double *value, gmz_stream stream);
+int gmz_records_retarget(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *discount_pow,
+                         int n_steps, gmz_stream stream);
 
 /* ---- tactics classifier (find_winning_moves_rebuilt, workers.py:49-123) ---- */
 /* boards int8 [B,A], players int8 [B] (the side to move) -> out_cls int8 [B,A]: per empty cell
