@@ -73,6 +73,8 @@ SIGNATURES = {
     "gmz_set_roots_from_records": (C.c_int, [_P, _P, C.c_int64, C.c_int64, C.c_int64, _P]),
     "gmz_records_writeback": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_int64, _P, _P, _P]),
     "gmz_records_retarget": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_int64, _P, C.c_int, _P]),
+    "gmz_records_compact": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int64, C.c_int64, _P, _P, _P, _P]),
+    "gmz_records_expand": (C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, C.c_int64, _P]),
     "gmz_tactics_classify": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gmz_per_update": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int, _P]),
     "gmz_per_add": (C.c_int, [_P, C.c_int64, C.c_int64, _P, C.c_int, _P, _P]),

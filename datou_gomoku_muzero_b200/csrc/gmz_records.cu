@@ -83,6 +83,27 @@ __device__ __forceinline__ void rec_apply(u64 &P, u64 &M, int colour, int a, int
     if (lane == (a >> 6)) { const u64 bit = 1ull << (a & 63); if (colour > 0) { P |= bit; M &= ~bit; } else { M |= bit; P &= ~bit; } }
 }
 
+// A record's observation planes (game.py:12-17) and board (before the move) from the position's bitboards: P / M hold
+// the stones of +1 / -1, 64 cells per lane; the own plane is P if colour (the side to move) > 0, else M; the third plane
+// marks `last` (-1 or any value outside [0, A): no cell).  Called by the whole warp: every lane takes part in the shuffles.
+__device__ __forceinline__ void rec_write_position(unsigned char *rec, int A, u64 P, u64 M, int colour, int last, int lane)
+{
+    float *obs = reinterpret_cast<float *>(rec + 64 + (size_t)8 * A);
+    int8_t *brd = reinterpret_cast<int8_t *>(rec + 64 + (size_t)20 * A);
+    const u64 own = colour > 0 ? P : M, opp = colour > 0 ? M : P;
+    for (int c0 = 0; c0 < A; c0 += 32) {
+        const int c = c0 + lane, cw = min(c, A - 1) >> 6;
+        const u64 ow = __shfl_sync(GMZ_FULL, own, cw), pw = __shfl_sync(GMZ_FULL, opp, cw);
+        const u64 bp = __shfl_sync(GMZ_FULL, P, cw), bm = __shfl_sync(GMZ_FULL, M, cw);
+        if (c < A) {
+            obs[c] = (float)((ow >> (c & 63)) & 1ull);
+            obs[A + c] = (float)((pw >> (c & 63)) & 1ull);
+            obs[2 * A + c] = c == last ? 1.0f : 0.0f;
+            brd[c] = (int8_t)((int)((bp >> (c & 63)) & 1ull) - (int)((bm >> (c & 63)) & 1ull));
+        }
+    }
+}
+
 // One CTA per finished game, warp w emits moves w, w + 4, ... (each warp replays the game on its own bitboards).
 __global__ void __launch_bounds__(128)
 k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, const double *value, const int32_t *action,
@@ -103,22 +124,9 @@ k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, co
         for (; m < t; ++m) { const int a = acts[m]; rec_apply(P, M, colour, a, lane); colour = -colour; last = a; ++mc; }
         unsigned char *rec = out + (size_t)(move_offset[gi] + t) * stride;
         double *pol = reinterpret_cast<double *>(rec + 64);
-        float *obs = reinterpret_cast<float *>(rec + 64 + (size_t)8 * A);
-        int8_t *brd = reinterpret_cast<int8_t *>(rec + 64 + (size_t)20 * A);
         const double *psrc = policy + ((size_t)slot * max_moves + t) * A;
-        const u64 own = colour > 0 ? P : M, opp = colour > 0 ? M : P;
-        for (int c0 = 0; c0 < A; c0 += 32) {           // all 32 lanes take part in the shuffles
-            const int c = c0 + lane, cw = min(c, A - 1) >> 6;
-            const u64 ow = __shfl_sync(GMZ_FULL, own, cw), pw = __shfl_sync(GMZ_FULL, opp, cw);
-            const u64 bp = __shfl_sync(GMZ_FULL, P, cw), bm = __shfl_sync(GMZ_FULL, M, cw);
-            if (c < A) {
-                obs[c] = (float)((ow >> (c & 63)) & 1ull);
-                obs[A + c] = (float)((pw >> (c & 63)) & 1ull);
-                obs[2 * A + c] = c == last ? 1.0f : 0.0f;
-                brd[c] = (int8_t)((int)((bp >> (c & 63)) & 1ull) - (int)((bm >> (c & 63)) & 1ull));
-                pol[c] = psrc[c];
-            }
-        }
+        rec_write_position(rec, A, P, M, colour, last, lane);
+        for (int c = lane; c < A; c += 32) pol[c] = psrc[c];
         if (lane == 0) {
             // compute_n_step_returns (workers.py:144-152): Python-float reward sum, float32 bootstrap, float32 add
             double acc = 0.0;
@@ -305,6 +313,147 @@ extern "C" int gmz_records_retarget(void *ring, int64_t capacity, int board_size
     const int A = board_size * board_size;
     k_records_retarget<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>((unsigned char *)ring, rec_stride(A), capacity,
                                                                                      first, n, discount_pow, n_steps);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Checkpoint form of the ring (DeviceReplayBuffer.state_dict / load_state_dict).  Of a record only the header and the
+// policy carry information: the board follows from the previous record's board and action, the observation planes from
+// the board and the header.  A stretch is saved as headers u8 [n][64] + policies f64 [n][A], plus the board of the first
+// record of every segment (a run of records that starts at k = 0 or at a header t = 0: games sit whole and in move order
+// in the ring, only the oldest live game can be cut).
+
+// Saving: record k of the stretch (one warp per record) -> its header and policy bytes verbatim, and a flag byte:
+//   bit 0: the record starts a segment (k == 0 or t == 0),
+//   bit 1: the record is NOT rebuildable -- its board or observation planes differ from what k_records_expand writes:
+//          the board holds a value outside {-1, 0, 1}; the planes are not (board == own, board == -own, cell == last_move)
+//          as 0.0f / 1.0f bit patterns, own = to_move > 0 ? +1 : -1; or (no segment start) the board is not record k-1's
+//          board with record k-1's action played for record k-1's to_move (rec_apply: overwrite the cell, an action
+//          outside [0, A) changes nothing).
+// Each record is compared with its predecessor only, so the check needs no sequential replay.
+__global__ void __launch_bounds__(128)
+k_records_compact(const unsigned char *ring, size_t stride, int64_t capacity, int64_t first, int64_t n, int A,
+                  unsigned char *out_headers, double *out_policy, uint8_t *out_flags)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t k = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (k >= n) return;
+    const unsigned char *rec = ring + (size_t)((first + k) % capacity) * stride;
+    const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
+    if (lane < 16) reinterpret_cast<uint32_t *>(out_headers + (size_t)k * 64)[lane] = reinterpret_cast<const uint32_t *>(rec)[lane];
+    const double *pol = reinterpret_cast<const double *>(rec + 64);
+    double *dst = out_policy + (size_t)k * A;
+    for (int c = lane; c < A; c += 32) dst[c] = pol[c];
+
+    const bool start = k == 0 || h->t == 0;
+    const int own = h->to_move > 0 ? 1 : -1, last = h->last_move;
+    const uint32_t *obs = reinterpret_cast<const uint32_t *>(rec + 64 + (size_t)8 * A);
+    const int8_t *brd = reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * A);
+    const int8_t *pbrd = nullptr;
+    int pa = -1, pown = 0;
+    if (!start) {
+        const unsigned char *prv = ring + (size_t)((first + k - 1) % capacity) * stride;
+        const RecHeader *hp = reinterpret_cast<const RecHeader *>(prv);
+        pa = hp->action;
+        pown = hp->to_move > 0 ? 1 : -1;
+        pbrd = reinterpret_cast<const int8_t *>(prv + 64 + (size_t)20 * A);
+    }
+    const uint32_t one = 0x3f800000u;                   // 1.0f
+    bool bad = false;
+    for (int c = lane; c < A; c += 32) {
+        const int b = brd[c];
+        bad |= b < -1 || b > 1;
+        bad |= obs[c] != (b == own ? one : 0u);
+        bad |= obs[A + c] != (b == -own ? one : 0u);
+        bad |= obs[2 * A + c] != (c == last ? one : 0u);
+        if (pbrd) bad |= b != (c == pa ? pown : (int)pbrd[c]);
+    }
+    bad = __any_sync(GMZ_FULL, bad);
+    if (lane == 0) out_flags[k] = (uint8_t)((start ? 1 : 0) | (bad ? 2 : 0));
+}
+
+extern "C" int gmz_records_compact(const void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, void *out_headers,
+                                   double *out_policy, uint8_t *out_flags, gmz_stream stream)
+{
+    const char *name = "gmz_records_compact";
+    if (!ring || !out_headers || !out_policy || !out_flags) return rc_fail2(name, "null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return rc_fail2(name, m);
+    if (n == 0) return 0;
+    const int A = board_size * board_size;
+    k_records_compact<<<(unsigned)((n + 3) / 4), 128, 0, (cudaStream_t)stream>>>((const unsigned char *)ring, rec_stride(A), capacity,
+                                                                                 first, n, A, (unsigned char *)out_headers, out_policy,
+                                                                                 out_flags);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+}
+
+// Loading: one CTA per segment, segment s = records [seg_start[s], seg_start[s+1]) (the last one up to n), clamped to
+// [0, n).  Warp w replays the segment from its base board on its own bitboards, every record's action played for that
+// record's own header to_move (the exact inverse of the check above), and emits records w, w + 4, ...: record k >= skip
+// becomes a full record at ring position (first + k - skip) % capacity -- header and policy verbatim, board and
+// observation planes rebuilt (rec_write_position, as k_traj_pack writes them), tail padding zero.  Records below skip
+// are replayed but not written.  No memory is indexed by a header field, so any table contents stay in bounds.
+__global__ void __launch_bounds__(128)
+k_records_expand(const unsigned char *headers, const double *policy, int64_t n, const int64_t *seg_start, const int8_t *base_boards,
+                 int64_t n_seg, int64_t skip, int A, size_t stride, unsigned char *ring, int64_t capacity, int64_t first)
+{
+    const int64_t s = blockIdx.x;
+    const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
+    const int64_t lo = min(max(seg_start[s], (int64_t)0), n);
+    const int64_t hi = s + 1 < n_seg ? min(max(seg_start[s + 1], lo), n) : n;
+    if (lo >= hi) return;
+    const int8_t *bb = base_boards + (size_t)s * A;
+    u64 P = 0, M = 0;
+    for (int w = 0; w < (A + 63) / 64; ++w) {          // ballots pack 32 cells at a time (root_load, gmz_engine.cu)
+        u64 pw = 0, mw = 0;
+        for (int h = 0; h < 2; ++h) {
+            const int a = 64 * w + 32 * h + lane;
+            const int c = a < A ? (int)bb[a] : 0;
+            pw |= (u64)__ballot_sync(GMZ_FULL, c == 1) << (32 * h);
+            mw |= (u64)__ballot_sync(GMZ_FULL, c == -1) << (32 * h);
+        }
+        if (lane == w) { P = pw; M = mw; }
+    }
+    const size_t body = (size_t)64 + (size_t)21 * A;
+    int64_t m = lo;
+    for (int64_t k = lo + wi; k < hi; k += 4) {
+        for (; m < k; ++m) {
+            const RecHeader *hm = reinterpret_cast<const RecHeader *>(headers + (size_t)m * 64);
+            rec_apply(P, M, hm->to_move, hm->action, lane);
+        }
+        if (k < skip) continue;
+        const unsigned char *src = headers + (size_t)k * 64;
+        const RecHeader *hk = reinterpret_cast<const RecHeader *>(src);
+        unsigned char *rec = ring + (size_t)((first + k - skip) % capacity) * stride;
+        if (lane < 16) reinterpret_cast<uint32_t *>(rec)[lane] = reinterpret_cast<const uint32_t *>(src)[lane];
+        double *pol = reinterpret_cast<double *>(rec + 64);
+        const double *psrc = policy + (size_t)k * A;
+        for (int c = lane; c < A; c += 32) pol[c] = psrc[c];
+        rec_write_position(rec, A, P, M, hk->to_move, hk->last_move, lane);
+        for (size_t i = body + lane; i < stride; i += 32) rec[i] = 0;
+    }
+}
+
+extern "C" int gmz_records_expand(const void *headers, const double *policy, int64_t n, const int64_t *seg_start,
+                                  const int8_t *base_boards, int64_t n_seg, int64_t skip, int board_size, void *ring, int64_t capacity,
+                                  int64_t first, gmz_stream stream)
+{
+    const char *name = "gmz_records_expand";
+    if (!headers || !policy || !seg_start || !base_boards || !ring) return rc_fail2(name, "null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
+    if (capacity < 1) return rc_fail2(name, "capacity must be >= 1");
+    if (n < 0) return rc_fail2(name, "n must be >= 0");
+    if (skip < 0 || skip > n) return rc_fail2(name, "skip must be in 0..n");
+    if (n - skip > capacity) return rc_fail2(name, "n - skip exceeds the ring capacity");
+    if (first < 0 || first >= capacity) return rc_fail2(name, "first outside the ring [0, capacity)");
+    if (n > 0 && (n_seg < 1 || n_seg > n || n_seg > 0x7fffffff)) return rc_fail2(name, "n_seg must be in 1..n when n > 0");
+    if (n == 0) return 0;
+    const int A = board_size * board_size;
+    k_records_expand<<<(unsigned)n_seg, 128, 0, (cudaStream_t)stream>>>((const unsigned char *)headers, policy, n, seg_start, base_boards,
+                                                                        n_seg, skip, A, rec_stride(A), (unsigned char *)ring, capacity,
+                                                                        first);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
 }

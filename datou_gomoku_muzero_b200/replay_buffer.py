@@ -152,6 +152,68 @@ class InMemoryReplayBuffer:
         return self.sum_tree.count
 
 
+RING_STATE_FORMAT, RING_STATE_VERSION = "gmz_device_replay_ring", 1
+
+
+def validate_ring_state(sd, board_size):
+    """Host-side check of a DeviceReplayBuffer.state_dict() before anything of it goes to the device; raises ValueError
+    naming the first thing that does not fit.  Checks the tag and version, the board size, every shape and dtype, count
+    and write_ptr against the saved capacity, the tree length, the base boards' stone values and the header t chain:
+    segments start exactly at k = 0 and wherever t = 0, t grows by 1 and length stays put inside a segment, 0 <= t <
+    length, and every segment ends at its game's last move (games are appended whole)."""
+    if not isinstance(sd, dict):
+        raise ValueError("ring state must be a dict (DeviceReplayBuffer.state_dict())")
+    if sd.get("format") != RING_STATE_FORMAT or sd.get("version") != RING_STATE_VERSION:
+        raise ValueError(f"unknown ring state format {sd.get('format')!r} version {sd.get('version')!r} "
+                         f"(expected {RING_STATE_FORMAT!r} version {RING_STATE_VERSION})")
+    for key in ("board_size", "capacity", "count", "write_ptr"):
+        if not isinstance(sd.get(key), int) or isinstance(sd.get(key), bool):
+            raise ValueError(f"ring state {key} must be an int")
+    N, cap, n, wp = sd["board_size"], sd["capacity"], sd["count"], sd["write_ptr"]
+    if N != int(board_size):
+        raise ValueError(f"ring state board size {N} differs from the buffer's {int(board_size)}")
+    A = N * N
+    if cap < 1:
+        raise ValueError(f"ring state capacity {cap} must be >= 1")
+    if not 0 <= n <= cap:
+        raise ValueError(f"ring state count {n} outside 0..capacity ({cap})")
+    if not 0 <= wp < cap or (n < cap and wp != n):
+        raise ValueError(f"ring state write_ptr {wp} outside the saved ring (capacity {cap}, count {n})")
+
+    def tensor(key, dtype, shape):
+        t = sd.get(key)
+        if not torch.is_tensor(t) or t.device.type != "cpu" or t.dtype != dtype or tuple(t.shape) != shape:
+            got = f"{t.dtype} {tuple(t.shape)} on {t.device}" if torch.is_tensor(t) else type(t).__name__
+            raise ValueError(f"ring state {key} must be a CPU {dtype} tensor of shape {shape}, got {got}")
+        return t
+    seg = sd.get("seg_start")
+    n_seg = int(seg.shape[0]) if torch.is_tensor(seg) and seg.dim() == 1 else -1
+    headers = tensor("headers", torch.uint8, (n, 64))
+    tensor("policies", torch.float64, (n, A))
+    seg = tensor("seg_start", torch.int64, (max(n_seg, 0),))
+    base = tensor("base_boards", torch.int8, (max(n_seg, 0), A))
+    tensor("tree", torch.float64, (2 * cap - 1,))
+    tensor("max_priority", torch.float64, ())
+    if base.numel() and (base.min() < -1 or base.max() > 1):
+        raise ValueError("ring state base_boards hold a value outside {-1, 0, 1}")
+    h = headers.numpy().view(np.int32)                  # gmz_move_record: game_seq, t, length, ...
+    t, T = h[:, 1].astype(np.int64), h[:, 2].astype(np.int64)
+    k = np.arange(n)
+    starts = (k == 0) | (t == 0)
+    if not np.array_equal(seg.numpy(), np.flatnonzero(starts)):
+        raise ValueError("ring state seg_start does not match the header t chain (segments start at k = 0 and where t = 0)")
+    if n and not ((t >= 0) & (t < T)).all():
+        raise ValueError(f"ring state header t outside 0..length-1 at record {int(np.flatnonzero((t < 0) | (t >= T))[0])}")
+    inner = ~starts[1:]
+    broken = inner & ((t[1:] != t[:-1] + 1) | (T[1:] != T[:-1]))
+    if broken.any():
+        raise ValueError(f"ring state header t chain broken inside a segment at record {int(np.flatnonzero(broken)[0]) + 1}")
+    ends = np.append(starts[1:], True) if n else starts
+    if n and (t[ends] != T[ends] - 1).any():
+        raise ValueError("ring state holds a game cut before its last move")
+    return n_seg
+
+
 class DeviceReplayBuffer:
     """The reference's InMemoryReplayBuffer (replay_buffer.py:43-106) with tree AND data on the device.
 
@@ -166,6 +228,8 @@ class DeviceReplayBuffer:
     update_priorities  = replay_buffer.py:98-103 on device tensors (td_errors float32, as the loss returns them)
     rewrite_targets    = the re-analysis write-back (db_manager.py:189-214) for records in the ring
     reanalyse(engines) = Surge re-analysis (workers.py:243-305) of the records in the ring, in place, on the device
+    state_dict() / load_state_dict(sd) = checkpoint and restore of ring, tree, write_ptr, count and max_priority in a
+                          compact form (headers, policies, one board per segment), rebuilt on the device
     """
 
     def __init__(self, capacity, board_size, device=None, unroll_steps=None):
@@ -324,6 +388,73 @@ class DeviceReplayBuffer:
         pr = (td.abs() + np.float32(config.PER_EPSILON)).double()        # float32 arithmetic like the reference, then widened
         self.max_priority = torch.maximum(self.max_priority, pr.max())
         self.sum_tree.update_many(tree_indices, pr)
+
+    def state_dict(self):
+        """The buffer's state as a dict of CPU tensors, ints and strs, for torch.save next to the network (loads with
+        torch.load(weights_only=True)).  Records are kept in compact form, oldest first: headers u8 [count, 64] and
+        policies f64 [count, A] verbatim, plus seg_start int64 [n_seg] (the first record of each segment: the oldest live
+        record and every game start) and base_boards int8 [n_seg, A] (their boards).  Boards and observation planes of
+        the other records are rebuilt by load_state_dict.  tree, write_ptr, count and max_priority are saved verbatim.
+
+        Runs on the current stream after any pending add_packed / reanalyse / update_priorities and synchronises with
+        the host (the result is host memory).  Extra device memory: the compact size of the live records.  Raises
+        ValueError, leaving the buffer as it is, if a live record's board or observation planes are not what its
+        predecessor and header imply (gmz_records_compact bit 1: such a record cannot be rebuilt)."""
+        cap, n, wp, A, dev = self.capacity, self.sum_tree.count, self.sum_tree.write_ptr, self.A, self.device
+        oldest = wp if n == cap else 0
+        headers = torch.empty((n, 64), dtype=torch.uint8, device=dev)
+        policies = torch.empty((n, A), dtype=torch.float64, device=dev)
+        seg = torch.empty(0, dtype=torch.int64, device=dev)
+        if n > 0:
+            flags = torch.empty(n, dtype=torch.uint8, device=dev)
+            check(self.lib.gmz_records_compact(_ptr(self.ring), cap, self.N, oldest, n, _ptr(headers), _ptr(policies),
+                                               _ptr(flags), self.sum_tree._stream()), "gmz_records_compact")
+            bad = (flags & 2) != 0
+            n_bad, k_bad = (int(x) for x in torch.stack([bad.sum(), bad.int().argmax()]).cpu())
+            if n_bad:
+                raise ValueError(f"{n_bad} live ring records cannot be rebuilt from their predecessor and header (board or "
+                                 f"observation planes altered); the first is at ring position {(oldest + k_bad) % cap}")
+            seg = (flags & 1).nonzero().reshape(-1)
+        body = 64 + 20 * A
+        base = self.ring[(oldest + seg) % cap, body:body + A].view(torch.int8)
+        return {"format": RING_STATE_FORMAT, "version": RING_STATE_VERSION, "board_size": self.N, "capacity": cap,
+                "count": n, "write_ptr": wp, "headers": headers.cpu(), "policies": policies.cpu(), "seg_start": seg.cpu(),
+                "base_boards": base.cpu(), "tree": self.sum_tree.tree.cpu(), "max_priority": self.max_priority.cpu()}
+
+    def load_state_dict(self, sd):
+        """Restore a state_dict() (validated on the host first: validate_ring_state; ValueError before any device work).
+
+        Same capacity: the state bit for bit -- record k of the saved order at ring position (oldest + k) % capacity, tree,
+        write_ptr, count and max_priority verbatim (ring positions holding no live record are zeroed, as in a new buffer;
+        the tail padding of each record is zero).  Later sample / batch / add_packed / reanalyse calls behave as on the
+        saved buffer.
+        Different capacity: the newest min(count, capacity) records, oldest first, at positions 0.. (a cut may fall inside
+        the oldest kept game), write_ptr and count to match, and the tree rebuilt by SumTree.add_many from the kept
+        records' saved leaf priorities in order -- equal to sequential add()s of them, not bit-equal to the old internal
+        sums.  max_priority is kept.
+        Value targets are restored as saved, whatever config.N_STEPS / DISCOUNT say now."""
+        n_seg = validate_ring_state(sd, self.N)
+        cap, dev, st = self.capacity, self.device, self.sum_tree
+        scap, n, swp = sd["capacity"], sd["count"], sd["write_ptr"]
+        kept = min(n, cap)
+        skip = n - kept
+        if kept > 0:
+            headers, policies, seg, base = (sd[key].to(dev).contiguous() for key in ("headers", "policies", "seg_start", "base_boards"))
+            first = (swp if n == cap else 0) if scap == cap else 0
+            check(self.lib.gmz_records_expand(_ptr(headers), _ptr(policies), n, _ptr(seg), _ptr(base), n_seg, skip, self.N,
+                                              _ptr(self.ring), cap, first, st._stream()), "gmz_records_expand")
+        if kept < cap:
+            self.ring[kept:].zero_()
+        if scap == cap:
+            st.tree.copy_(sd["tree"])
+            st.write_ptr, st.count = swp, n
+        else:
+            soldest = swp if n == scap else 0
+            leaf = (soldest + torch.arange(skip, n, dtype=torch.int64)) % scap + (scap - 1)
+            st.tree.zero_()
+            st.write_ptr, st.count = 0, 0
+            st.add_many(sd["tree"][leaf])
+        self.max_priority = sd["max_priority"].to(dev)
 
     def __len__(self):
         return self.sum_tree.count

@@ -293,6 +293,24 @@ int gmz_records_writeback(void *ring, int64_t capacity, int board_size, int64_t 
                           const double *value, gmz_stream stream);
 int gmz_records_retarget(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *discount_pow,
                          int n_steps, gmz_stream stream);
+/* Checkpoint form of the ring: only a record's header and policy carry information -- its board follows from the previous
+ * record's board and action, its observation planes from the board and the header.  A SEGMENT is a run of consecutive
+ * records that starts at k = 0 or at a header t = 0 (games sit whole and in move order in the ring).
+ * gmz_records_compact: the stretch (first, n) -> out_headers u8 [n][64] and out_policy f64 [n][A], verbatim, and
+ *   out_flags u8 [n]: bit 0 = record k starts a segment; bit 1 = record k is NOT rebuildable by gmz_records_expand: its
+ *   board holds a value outside {-1, 0, 1}, its planes are not (board == own, board == -own, cell == last_move) as
+ *   0.0f / 1.0f with own = to_move > 0 ? +1 : -1, or (not a segment start) its board is not record k-1's board with record
+ *   k-1's action played for record k-1's to_move (an action outside [0, A) changes nothing).
+ * gmz_records_expand: n compact records (headers, policy as above), seg_start int64 [n_seg] (the k of each segment's
+ *   first record, 1 <= n_seg <= n when n > 0) and base_boards int8 [n_seg][A] (those records' boards) -> record k, for
+ *   every k >= skip (0 <= skip <= n, n - skip <= capacity), as a full record at ring position (first + k - skip) % capacity:
+ *   header and policy verbatim, board replayed from the segment's base board with every earlier record's action played
+ *   for that record's to_move, planes derived from it, tail padding zero.  Segments are clamped to [0, n).
+ * n = 0 is a no-op for both.  All pointers are device pointers. */
+int gmz_records_compact(const void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, void *out_headers,
+                        double *out_policy, uint8_t *out_flags, gmz_stream stream);
+int gmz_records_expand(const void *headers, const double *policy, int64_t n, const int64_t *seg_start, const int8_t *base_boards,
+                       int64_t n_seg, int64_t skip, int board_size, void *ring, int64_t capacity, int64_t first, gmz_stream stream);
 
 /* ---- tactics classifier (find_winning_moves_rebuilt, workers.py:49-123) ---- */
 /* boards int8 [B,A], players int8 [B] (the side to move) -> out_cls int8 [B,A]: per empty cell
