@@ -13,7 +13,7 @@ import torch
 import torch.nn.functional as F
 
 from ._lib import check
-from .network import GomokuNetEZ, _fold, _fold_heads, _support_scalar
+from .network import GomokuNetEZ, _fold, _fold_heads, _support_scalar, capture_stream
 
 _M64 = (1 << 64) - 1
 
@@ -45,6 +45,11 @@ class MuZeroDeviceSearch:
     initial_fn result.  A 4-D hidden state [G,C,N,N] is stored NHWC (one row = N*N cells x C channels), so
     the gathered batch is a channels_last tensor without a copy.
 
+    Pool layouts: by default game g owns rows g*nodes_per_game .. g*nodes_per_game + nodes_per_game - 1.  A search given
+    per-game budgets (`rows`, re-analysis) uses one compact arena instead: game g owns rows base[g] .. base[g] + rows[g] - 1,
+    base the exclusive prefix sum of `rows`; a node at or beyond its game's budget is not stored (skip slot) and is counted
+    in `overflow` (int64 device scalar).  `nodes_per_game` then caps the budget a game may ask for.
+
     One simulation step = gmz_select_mz -> gmz_hidden_gather -> recurrent_fn -> gmz_hidden_scatter ->
     gmz_expand_backup, all on the device.  If recurrent_fn has `embed` ([E] action-embedding vector) and
     `forward_fused(x)` (x = [G, C+E, N, N] channels_last: hidden state and one-hot action embedding already
@@ -61,6 +66,10 @@ class MuZeroDeviceSearch:
         self.use_graph, self.graph_warmup, self.graph = bool(graph), int(graph_warmup), None
         self.fused = hasattr(recurrent_fn, "forward_fused") and getattr(recurrent_fn, "embed", None) is not None
         self._root_slot = (torch.arange(engine.G, dtype=torch.int32, device=engine.device) * engine.S).contiguous()
+        self.arena = False                              # pool layout: g * nodes + node (False) or base[g] + node (True)
+        self._budget = torch.zeros(engine.G, dtype=torch.int32, device=engine.device)
+        self._base = torch.zeros(engine.G, dtype=torch.int32, device=engine.device)
+        self.overflow = torch.zeros((), dtype=torch.int64, device=engine.device)
 
     def set_recurrent_fn(self, recurrent_fn):
         """Swap the dynamics evaluator (e.g. after a model update that built a new FoldedRecurrentInference): the
@@ -86,12 +95,17 @@ class MuZeroDeviceSearch:
             return h.permute(0, 2, 3, 1).contiguous().reshape(h.shape[0], -1)
         return h.contiguous().reshape(h.shape[0], -1)
 
-    def _ensure_pool(self, hidden):
+    def _ensure_pool(self, hidden, arena_rows=None):
         e = self.e
         rows = self._rows(hidden)
-        shape = (e.G * self.nodes, rows.shape[1])
-        if self.pool is None or self.pool.shape != shape or self.pool.dtype != hidden.dtype:
+        arena = arena_rows is not None
+        shape = (int(arena_rows) if arena else e.G * self.nodes, rows.shape[1])
+        if arena and self.pool is not None and self.arena and self.pool.shape[0] >= shape[0]:
+            shape = tuple(self.pool.shape)              # the arena only grows
+        if self.pool is None or self.pool.shape != shape or self.pool.dtype != hidden.dtype or self.arena != arena:
+            self.pool = None                            # free the old pool first
             self.pool = torch.empty(shape, dtype=hidden.dtype, device=hidden.device)
+            self.arena = arena
             self.hshape = tuple(hidden.shape[1:])
             self.row_bytes = rows.shape[1] * hidden.element_size()
             if self.row_bytes % 4:
@@ -113,7 +127,8 @@ class MuZeroDeviceSearch:
 
     def _gather(self, slot, action):
         e = self.e
-        check(e.lib.gmz_hidden_gather(self.pool.data_ptr(), slot.data_ptr(), action.data_ptr(), e.G, e.S, self.nodes,
+        S, nodes = (1, 1) if self.arena else (e.S, self.nodes)         # arena: slots are already pool rows
+        check(e.lib.gmz_hidden_gather(self.pool.data_ptr(), slot.data_ptr(), action.data_ptr(), e.G, S, nodes,
                                       self.positions, self.pos_bytes,
                                       None if self.embed is None else self.embed.data_ptr(), self.embed_bytes,
                                       self.x.data_ptr(), e._stream()), "gmz_hidden_gather")
@@ -123,7 +138,8 @@ class MuZeroDeviceSearch:
         e = self.e
         if rows.dtype != self.pool.dtype or rows.shape[1] != self.pool.shape[1]:
             raise ValueError("recurrent_fn returned a hidden state of a different dtype / shape than initial_fn")
-        check(e.lib.gmz_hidden_scatter(self.pool.data_ptr(), slot.data_ptr(), e.G, e.S, self.nodes, self.row_bytes,
+        S, nodes = (1, 1) if self.arena else (e.S, self.nodes)
+        check(e.lib.gmz_hidden_scatter(self.pool.data_ptr(), slot.data_ptr(), e.G, S, nodes, self.row_bytes,
                                        rows.data_ptr(), e._stream()), "gmz_hidden_scatter")
         e.launches += 1
 
@@ -136,9 +152,21 @@ class MuZeroDeviceSearch:
             return self.x.view(e.G, n1, n2, C_ + E).permute(0, 3, 1, 2)           # channels_last [G, C+E, N, N]
         return self.x.view((e.G,) + self.hshape)
 
+    def _arena_row(self, slot, count=False):
+        """Engine slot g*S + node -> arena row base[g] + node, or -1 (skip) for node >= rows[g]; with `count`, such nodes
+        are added to `overflow`.  Device tensor ops only (captured with the step)."""
+        node = slot - self._root_slot
+        live = slot >= 0
+        ok = live & (node < self._budget)
+        if count:
+            self.overflow.add_((live & ~ok).sum())
+        return torch.where(ok, self._base + node, -1).to(torch.int32)
+
     def _step(self):
         e = self.e
         parent, action, child, depth = e.select_mz()
+        if self.arena:
+            parent, child = self._arena_row(parent), self._arena_row(child, count=True)
         self._gather(parent, action)
         if self.embed is not None:
             lg, v, r, h_out = self.recurrent_fn.forward_fused(self._x_view())
@@ -151,21 +179,40 @@ class MuZeroDeviceSearch:
         e = self.e
         n0 = e.launches
         self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
+        with torch.cuda.graph(self.graph, stream=capture_stream(e.device)):
             self._step()
         self._launches_per_step = e.launches - n0
         e.launches = n0                                   # capture launched nothing
 
-    @torch.no_grad()
-    def search(self, gumbel, max_steps=None):
-        """Runs one search for every game from the engine's current roots; call engine.finalize() after."""
+    def budget_table(self):
+        """Tree nodes a search can create, by the number of root survivors k = min(K, empty cells) = 0..K: the root plus
+        one node per recurrent evaluation (int64 numpy [K+1])."""
         e = self.e
+        return np.array([evals_per_search(e.S, e.K, k) + 1 for k in range(e.K + 1)], dtype=np.int64)
+
+    @torch.no_grad()
+    def search(self, gumbel, max_steps=None, rows=None, arena_rows=None):
+        """Runs one search for every game from the engine's current roots; call engine.finalize() after.
+
+        rows (int32 device tensor [G]) / arena_rows (host int >= rows.sum()): per-game node budgets in one compact arena of
+        at least `arena_rows` rows (grown, and the graph re-captured, only when that is more than the arena has).  The
+        search then runs exactly `max_steps` steps (the largest evaluation count of the batch) and reads nothing back to
+        the host; steps after a game has finished evaluate nothing for it."""
+        e = self.e
+        arena = rows is not None
         lg, v, h = self.initial_fn(e.root_obs())
-        self._scatter(self._root_slot, self._ensure_pool(h))
+        pool_rows = self._ensure_pool(h, arena_rows if arena else None)
+        root = self._root_slot
+        if arena:
+            self._budget.copy_(rows)
+            torch.cumsum(self._budget, 0, dtype=torch.int32, out=self._base)
+            self._base.sub_(self._budget)
+            root = self._arena_row(root, count=True)
+        self._scatter(root, pool_rows)
         e.root_expand(lg, v, gumbel)
-        steps, limit = 0, int(max_steps) if max_steps else e.S - 1      # at most S-1 evaluations (sim_count starts at 1)
+        steps, limit = 0, int(max_steps) if max_steps is not None and (arena or max_steps) else e.S - 1   # at most S-1 evaluations
         while steps < limit:
-            if steps + 2 > self.nodes:          # this step may create node id steps + 1
+            if not arena and steps + 2 > self.nodes:          # this step may create node id steps + 1
                 raise RuntimeError("hidden-state pool too small: pass a larger nodes_per_game")
             if self.use_graph and self.graph is None and steps >= self.graph_warmup:
                 self._capture()
@@ -176,7 +223,7 @@ class MuZeroDeviceSearch:
                 self._step()
             steps += 1
             self.evaluations += 1
-            if steps % 8 == 0 and steps < limit and int(e._mz_out[0].max().item()) < 0:   # every game is done
+            if not arena and steps % 8 == 0 and steps < limit and int(e._mz_out[0].max().item()) < 0:   # every game is done
                 self.evaluations -= 1           # the last step evaluated nothing
                 steps -= 1
                 break

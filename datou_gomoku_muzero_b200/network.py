@@ -16,6 +16,13 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 
+def capture_stream(device):
+    """The stream to capture a searcher's step graph on: the current one (the stream of the engine being driven), unless
+    that is the legacy default stream, which cannot be captured (torch.cuda.graph then uses its own side stream)."""
+    cur = torch.cuda.current_stream(device)
+    return None if cur == torch.cuda.default_stream(device) else cur
+
+
 def _c3(cin, cout):
     return nn.Conv2d(cin, cout, 3, padding=1, bias=False)
 
@@ -299,7 +306,7 @@ class NetworkSearch:
         n0 = e.launches
         torch.cuda.synchronize(e.device)
         self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
+        with torch.cuda.graph(self.graph, stream=capture_stream(e.device)):
             self._step()
         self._launches_per_step = e.launches - n0
         e.launches = n0                                # capturing launched nothing

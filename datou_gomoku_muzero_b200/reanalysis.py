@@ -26,7 +26,8 @@ def positions_of(game_record, board_size):
 
 def reanalyse(game_records, batch_search, board_size=None, gumbel_fn=None):
     """game_records: list of GameRecord.  batch_search: an `AlphaZeroMCTS.for_engine(...)`-style object
-    (search_batch over exactly G roots).  Returns, per game, (new_policies [T,A] float64,
+    (search_batch over exactly G roots; `MuZeroMCTS.for_engine(engine, (initial_fn, recurrent_fn))` re-analyses with the
+    learned dynamics, any evaluator of mcts.resolve_searchers works).  Returns, per game, (new_policies [T,A] float64,
     new_value_targets list[float], search_values float64 [T]) -- the first two are what
     `finish_reanalysis_for_game` is handed (workers.py:292-294).
     gumbel_fn(n, A) supplies the noise rows (default: np.random.gumbel like each reference search)."""
@@ -89,7 +90,10 @@ def reanalyse_positions(engines, boards, players, last_moves, move_counts, evalu
     """Re-search `n` stored positions (host arrays: boards int8 [n, A], players [n], last_moves [n], move_counts [n])
     with the latest evaluator -- the inner loop of the reference's re-analysis mode (workers.py:254-266) for any number of
     positions.  They stream through `len(engines)` engines in flight (PipelinedBatchSearch: pinned staging, H2D, search,
-    D2H), G positions per batch; the last batch is padded with inactive (full-board) roots.  Noise: `gumbel` float64
+    D2H), G positions per batch; the last batch is padded with inactive (full-board) roots.  evaluator: anything
+    mcts.resolve_searchers takes -- "e0", a callable, a GomokuNetEZ module, a pair (initial_fn, recurrent_fn) for
+    MuZero-mode engines (pass cls=MuZeroMCTS), or one already-built NetworkSearch / MuZeroDeviceSearch per engine; MuZero
+    searchers get per-game node budgets from the host boards, as DeviceReplayBuffer.reanalyse does.  Noise: `gumbel` float64
     [n, A] from the host, or drawn on the device from `noise_seed` (position i uses counters i*A .. i*A + A - 1).
     Returns (policies float64 [n, A], values float64 [n]); want_policies=False returns (None, values),
     "checksum" returns (sum of all policy entries, values) without materialising the [n, A] array."""

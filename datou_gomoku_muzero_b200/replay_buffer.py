@@ -139,6 +139,37 @@ class InMemoryReplayBuffer:
         indices = np.random.choice(self.sum_tree.count, batch_size, replace=False)
         return [self.data[i] for i in indices], indices, np.ones(batch_size, dtype=np.float32)
 
+    def _mz_budgets(self, start, n, batches, engines, searchers):
+        """Per-record node budgets of a re-analysis stretch for MuZeroDeviceSearch engines (others: 1), from each record's
+        empty-cell count on the device.  Returns (rows int32 device [n], per-batch arena rows incl. one per padding game,
+        per-batch step counts) -- the two lists from one device-to-host copy."""
+        from .muzero import MuZeroDeviceSearch
+        dev, A, m = self.device, self.A, len(engines)
+        K = max(e.K for e in engines)
+        table = np.ones((m, K + 1), np.int32)                 # [engine, k] -> rows; clamped to each engine's own K below
+        kmax = np.array([e.K for e in engines], np.int64)
+        for i, x in enumerate(searchers):
+            if isinstance(x, MuZeroDeviceSearch):
+                t = x.budget_table()
+                table[i] = t[np.minimum(np.arange(K + 1), engines[i].K)]
+        first = np.array([s0 for _, s0, _ in batches], np.int64)
+        host = torch.from_numpy(np.concatenate([first, kmax, table.reshape(-1).astype(np.int64)])).pin_memory()
+        dv = host.to(dev, non_blocking=True)
+        nb = len(batches)
+        d_first, d_kmax, d_table = dv[:nb], dv[nb:nb + m], dv[nb + m:].reshape(m, K + 1)
+        body = 64 + 20 * A                                    # gmz_move_record: board int8 [A]
+        idx = (start + torch.arange(n, device=dev)) % self.capacity
+        empty = (self.ring[idx, body:body + A] == 0).sum(1)
+        batch = torch.searchsorted(d_first, torch.arange(n, device=dev), right=True) - 1
+        eng = batch % m
+        rows = d_table[eng, torch.minimum(empty, d_kmax[eng])]
+        out = torch.zeros((2, nb), dtype=torch.int64, device=dev)
+        out[0].scatter_add_(0, batch, rows)
+        out[1].scatter_reduce_(0, batch, rows - 1, "amax")
+        total, steps = out.cpu().tolist()                     # the one host read
+        total = [t + engines[i].G - k for t, (i, _, k) in zip(total, batches)]
+        return rows.to(torch.int32), total, steps
+
     def update_priorities(self, tree_indices, td_errors):
         if not config.ENABLE_PER:
             return
@@ -314,15 +345,27 @@ class DeviceReplayBuffer:
         alternating between the engines, each on a stream of its own; the caller's current stream waits for all of them
         and then runs the target recomputation, so later add_packed / batch / sample calls see the new bytes.  Loading the
         roots overwrites an engine's games: do not pass the engine that is running self-play.
-        evaluator: "e0" (the fixed evaluator, either engine mode; eval_seed / logit_div as SearchEngine.search_e0) or a
-        callable f(obs f32 [G,3,N,N]) -> (logits, values) on AlphaZero-mode engines.  Noise is drawn on the device: record
-        k of the widened stretch uses Gumbel counters k*A .. k*A + A-1 of `noise_seed`, as reanalyse_positions gives its
-        position k.  Policies and values never go to the host; the only host read is the two boundary headers of an
-        explicit stretch."""
-        from .mcts import search_roots
+        evaluator: whatever SelfPlayEngine takes, resolved to one searcher per engine by mcts.resolve_searchers -- "e0"
+        (the fixed evaluator, either engine mode; eval_seed / logit_div as SearchEngine.search_e0); a callable
+        f(obs f32 [G,3,N,N]) -> (logits, values) (eager, AlphaZero mode); a GomokuNetEZ module (a bf16 NetworkSearch per
+        engine, AlphaZero mode); a pair (initial_fn, recurrent_fn) (a MuZeroDeviceSearch(graph=True) per engine, MuZero
+        mode); or a list of already-built NetworkSearch / MuZeroDeviceSearch objects, one bound to each engine, which keep
+        their captured graphs from call to call.  Anything else raises ValueError before any kernel is enqueued.
+        Noise is drawn on the device: record k of the widened stretch uses Gumbel counters k*A .. k*A + A-1 of
+        `noise_seed`, as reanalyse_positions gives its position k.
+
+        MuZero searchers keep hidden states in a compact arena: a record with k = min(K, empty cells) root survivors gets
+        the root plus muzero.evals_per_search(S, K, k) rows, so the arena holds what the batch can use, not G * S rows.
+        One device pass over the stretch counts the empty cells; one small read brings every batch's row total and step
+        count to the host before any search is enqueued (ValueError, nothing touched, if a searcher's nodes_per_game is
+        below a record's budget), and each batch then runs its exact step count without reading anything back.
+
+        Policies and values never go to the host; the only host reads are that budget read (MuZero searchers) and the two
+        boundary headers of an explicit stretch."""
+        from .mcts import check_budget, resolve_searchers, search_roots
+        from .muzero import MuZeroDeviceSearch
         engines = list(engines)
-        e0 = isinstance(evaluator, str)
-        if e0 and evaluator != "e0":
+        if isinstance(evaluator, str) and evaluator != "e0":
             raise ValueError(f"unknown evaluator {evaluator!r}")
         if not engines:
             raise ValueError("reanalyse needs at least one engine")
@@ -331,8 +374,7 @@ class DeviceReplayBuffer:
                 raise ValueError(f"engine board size {e.N} differs from the buffer's {self.N}")
             if e.device != self.device:
                 raise ValueError(f"engine on {e.device}, buffer on {self.device}")
-            if not e0 and e.mode != "AlphaZero":
-                raise ValueError("a network evaluator needs AlphaZero-mode engines")
+        searchers = resolve_searchers(engines, evaluator)
         cap, live = self.capacity, self.sum_tree.count
         oldest = self.sum_tree.write_ptr if live == cap else 0
         if first is not None and not 0 <= int(first) < cap:
@@ -352,32 +394,76 @@ class DeviceReplayBuffer:
         start = (oldest + rel) % cap
         if n == 0:
             return start, 0
+        batches, s0 = [], 0                                   # (engine, first record of the stretch, records)
+        while s0 < n:
+            i = len(batches) % len(engines)
+            batches.append((i, s0, min(engines[i].G, n - s0)))
+            s0 += batches[-1][2]
+        budgets = self._mz_budgets(start, n, batches, engines, searchers) \
+            if any(isinstance(x, MuZeroDeviceSearch) for x in searchers) else None
+        if budgets is not None:
+            rows, total, steps = budgets
+            for b, (i, _, _) in enumerate(batches):
+                if isinstance(searchers[i], MuZeroDeviceSearch):
+                    check_budget(searchers[i], steps[b] + 1)
+            arena = [max((total[b] for b, x in enumerate(batches) if x[0] == i), default=0) for i in range(len(engines))]
         cur = torch.cuda.current_stream(self.device)
         streams = [torch.cuda.Stream(device=self.device) for _ in engines]
         gumbel = [torch.empty((e.G, self.A), dtype=torch.float64, device=self.device) for e in engines]
         for s in streams:
             s.wait_stream(cur)
-        s0 = b = 0
-        while s0 < n:
-            i = b % len(engines)
+        for b, (i, s0, k) in enumerate(batches):
             e = engines[i]
-            k = min(e.G, n - s0)
             pos = (start + s0) % cap
             with torch.cuda.stream(streams[i]):
                 e.set_roots_from_records(self.ring, cap, pos, k)
                 e.fill_gumbel(gumbel[i], noise_seed, s0 * self.A)
-                search_roots(e, gumbel[i], evaluator, eval_seed, logit_div)
+                budget = None
+                if isinstance(searchers[i], MuZeroDeviceSearch):      # padding games: inactive roots, one row each
+                    budget = (rows[s0:s0 + k] if k == e.G else torch.cat((rows[s0:s0 + k], rows.new_ones(e.G - k))),
+                              arena[i], steps[b])
+                search_roots(e, gumbel[i], searchers[i], eval_seed, logit_div, budget)
                 pol, val, _, _ = e.finalize(want_visits=False)
                 check(self.lib.gmz_records_writeback(_ptr(self.ring), cap, self.N, pos, k, _ptr(pol), _ptr(val), e._stream()),
                       "gmz_records_writeback")
-            s0 += k
-            b += 1
         for s in streams:
             cur.wait_stream(s)
-        dpow = torch.tensor([config.DISCOUNT ** i for i in range(config.N_STEPS + 1)], dtype=torch.float64, device=self.device)
+        dpow = torch.tensor([config.DISCOUNT ** i for i in range(config.N_STEPS + 1)], dtype=torch.float64).pin_memory()
+        dpow = dpow.to(self.device, non_blocking=True)      # no host synchronisation
         check(self.lib.gmz_records_retarget(_ptr(self.ring), cap, self.N, start, n, _ptr(dpow), int(config.N_STEPS),
                                             self.sum_tree._stream()), "gmz_records_retarget")
         return start, n
+
+    def _mz_budgets(self, start, n, batches, engines, searchers):
+        """Per-record node budgets of a re-analysis stretch for MuZeroDeviceSearch engines (others: 1), from each record's
+        empty-cell count on the device.  Returns (rows int32 device [n], per-batch arena rows incl. one per padding game,
+        per-batch step counts) -- the two lists from one device-to-host copy."""
+        from .muzero import MuZeroDeviceSearch
+        dev, A, m = self.device, self.A, len(engines)
+        K = max(e.K for e in engines)
+        table = np.ones((m, K + 1), np.int32)                 # [engine, k] -> rows; clamped to each engine's own K below
+        kmax = np.array([e.K for e in engines], np.int64)
+        for i, x in enumerate(searchers):
+            if isinstance(x, MuZeroDeviceSearch):
+                t = x.budget_table()
+                table[i] = t[np.minimum(np.arange(K + 1), engines[i].K)]
+        first = np.array([s0 for _, s0, _ in batches], np.int64)
+        host = torch.from_numpy(np.concatenate([first, kmax, table.reshape(-1).astype(np.int64)])).pin_memory()
+        dv = host.to(dev, non_blocking=True)
+        nb = len(batches)
+        d_first, d_kmax, d_table = dv[:nb], dv[nb:nb + m], dv[nb + m:].reshape(m, K + 1)
+        body = 64 + 20 * A                                    # gmz_move_record: board int8 [A]
+        idx = (start + torch.arange(n, device=dev)) % self.capacity
+        empty = (self.ring[idx, body:body + A] == 0).sum(1)
+        batch = torch.searchsorted(d_first, torch.arange(n, device=dev), right=True) - 1
+        eng = batch % m
+        rows = d_table[eng, torch.minimum(empty, d_kmax[eng])]
+        out = torch.zeros((2, nb), dtype=torch.int64, device=dev)
+        out[0].scatter_add_(0, batch, rows)
+        out[1].scatter_reduce_(0, batch, rows - 1, "amax")
+        total, steps = out.cpu().tolist()                     # the one host read
+        total = [t + engines[i].G - k for t, (i, _, k) in zip(total, batches)]
+        return rows.to(torch.int32), total, steps
 
     def update_priorities(self, tree_indices, td_errors):
         if not config.ENABLE_PER:

@@ -16,7 +16,8 @@ class SelfPlayEngine:
     simulation step, select -> network -> expand/backup, bf16 NHWC observations written by the select); any callable
     `f(obs f32 [G,3,N,N]) -> (logits f32 [G,A], values f32/f64 [G])` run on the device (eager stepwise path); or --
     for an engine in MuZero mode -- a pair `(initial_fn, recurrent_fn)` / a `muzero.MuZeroDeviceSearch`
-    (learned dynamics in the tree, hidden states in the device pool; MuZeroMCTS.search, mcts.py:288-362)."""
+    (learned dynamics in the tree, hidden states in the device pool; MuZeroMCTS.search, mcts.py:288-362).  The evaluator
+    is resolved by mcts.resolve_searchers, as for re-analysis."""
 
     def __init__(self, engine: SearchEngine, evaluator="e0", seed=0, logit_div=16, noise_seed=0):
         self.e = engine
@@ -28,25 +29,12 @@ class SelfPlayEngine:
         self.moves_played = 0
         self.games_finished = 0
         self.done_mask = torch.zeros(G, dtype=torch.uint8, device=engine.device)
-        self.mz = self.ns = None
-        if not isinstance(evaluator, str) and engine.mode == "AlphaZero":
-            from .network import NetworkSearch
-            if isinstance(evaluator, NetworkSearch):
-                if evaluator.e is not engine:
-                    raise ValueError("the NetworkSearch drives a different engine")
-                self.ns = evaluator
-            elif isinstance(evaluator, torch.nn.Module):
-                self.ns = NetworkSearch(engine, evaluator)
-        elif isinstance(evaluator, str) and evaluator != "e0":
-            raise ValueError(f"unknown evaluator {evaluator!r}")
-        if not isinstance(evaluator, str) and engine.mode == "MuZero":
-            from .muzero import MuZeroDeviceSearch
-            if isinstance(evaluator, MuZeroDeviceSearch):
-                self.mz = evaluator
-            elif isinstance(evaluator, (tuple, list)) and len(evaluator) == 2:
-                self.mz = MuZeroDeviceSearch(engine, evaluator[0], evaluator[1])
-            else:
-                raise ValueError("a MuZero-mode engine needs evaluator='e0', (initial_fn, recurrent_fn) or a MuZeroDeviceSearch")
+        from .mcts import resolve_searchers
+        from .muzero import MuZeroDeviceSearch
+        from .network import NetworkSearch
+        searcher = resolve_searchers([engine], evaluator)[0]
+        self.ns = searcher if isinstance(searcher, NetworkSearch) else None
+        self.mz = searcher if isinstance(searcher, MuZeroDeviceSearch) else None
         self._e0 = isinstance(evaluator, str)
         engine.reset_games()
 
