@@ -9,7 +9,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libgmz.so")
-SOURCES = ["gmz_engine.cu", "gmz_per.cu", "gmz_slices.cu", "gmz_tactics.cu", "gmz_hidden.cu", "gmz_records.cu"]
+SOURCES = ["gmz_engine.cu", "gmz_per.cu", "gmz_tactics.cu", "gmz_hidden.cu", "gmz_records.cu"]
 # the persistent play kernel: one object per (MuZero mode, float32 accumulation), built in parallel
 PLAY_SOURCE = "gmz_play_inst.cu"
 PLAY_VARIANTS = [(0, 0), (0, 1), (1, 0), (1, 1)]

@@ -60,12 +60,8 @@ SIGNATURES = {
     "gmz_selfplay_step": (C.c_int, [_P, C.POINTER(GmzTraj), _P, _P, _P, C.c_int, _P, _P]),
     "gmz_play_counters": (C.c_int, [_P, _P, _P]),
     "gmz_select_counters": (C.c_int, [_P, _P, _P]),
-    "gmz_value_targets": (C.c_int, [C.POINTER(GmzTraj), _P, _P, _P, C.c_int, _P, C.c_int, _P, _P]),
     "gmz_hidden_gather": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P]),
     "gmz_hidden_scatter": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
-    "gmz_build_batch": (C.c_int, [C.POINTER(GmzTraj), C.c_int, _P, _P, _P, _P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),
-    "gmz_build_batch_aug": (C.c_int, [C.POINTER(GmzTraj), C.c_int, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int,
-                                      _P, _P, _P, _P, _P, _P]),
     "gmz_move_record_bytes": (C.c_size_t, [C.c_int]),
     "gmz_traj_pack": (C.c_int, [C.POINTER(GmzTraj), C.c_int, _P, C.c_int, _P, _P, C.c_int, _P, _P]),
     "gmz_records_batch": (C.c_int, [_P, C.c_int64, C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),

@@ -20,6 +20,7 @@ import torch
 from . import _lib
 from ._lib import check
 from .config import config
+from .trajectory import record_dtype
 
 
 def _ptr(t):
@@ -139,37 +140,6 @@ class InMemoryReplayBuffer:
         indices = np.random.choice(self.sum_tree.count, batch_size, replace=False)
         return [self.data[i] for i in indices], indices, np.ones(batch_size, dtype=np.float32)
 
-    def _mz_budgets(self, start, n, batches, engines, searchers):
-        """Per-record node budgets of a re-analysis stretch for MuZeroDeviceSearch engines (others: 1), from each record's
-        empty-cell count on the device.  Returns (rows int32 device [n], per-batch arena rows incl. one per padding game,
-        per-batch step counts) -- the two lists from one device-to-host copy."""
-        from .muzero import MuZeroDeviceSearch
-        dev, A, m = self.device, self.A, len(engines)
-        K = max(e.K for e in engines)
-        table = np.ones((m, K + 1), np.int32)                 # [engine, k] -> rows; clamped to each engine's own K below
-        kmax = np.array([e.K for e in engines], np.int64)
-        for i, x in enumerate(searchers):
-            if isinstance(x, MuZeroDeviceSearch):
-                t = x.budget_table()
-                table[i] = t[np.minimum(np.arange(K + 1), engines[i].K)]
-        first = np.array([s0 for _, s0, _ in batches], np.int64)
-        host = torch.from_numpy(np.concatenate([first, kmax, table.reshape(-1).astype(np.int64)])).pin_memory()
-        dv = host.to(dev, non_blocking=True)
-        nb = len(batches)
-        d_first, d_kmax, d_table = dv[:nb], dv[nb:nb + m], dv[nb + m:].reshape(m, K + 1)
-        body = 64 + 20 * A                                    # gmz_move_record: board int8 [A]
-        idx = (start + torch.arange(n, device=dev)) % self.capacity
-        empty = (self.ring[idx, body:body + A] == 0).sum(1)
-        batch = torch.searchsorted(d_first, torch.arange(n, device=dev), right=True) - 1
-        eng = batch % m
-        rows = d_table[eng, torch.minimum(empty, d_kmax[eng])]
-        out = torch.zeros((2, nb), dtype=torch.int64, device=dev)
-        out[0].scatter_add_(0, batch, rows)
-        out[1].scatter_reduce_(0, batch, rows - 1, "amax")
-        total, steps = out.cpu().tolist()                     # the one host read
-        total = [t + engines[i].G - k for t, (i, _, k) in zip(total, batches)]
-        return rows.to(torch.int32), total, steps
-
     def update_priorities(self, tree_indices, td_errors):
         if not config.ENABLE_PER:
             return
@@ -268,6 +238,8 @@ class DeviceReplayBuffer:
         self.capacity, self.N, self.A = int(capacity), int(board_size), int(board_size) ** 2
         self.device, self.lib = self.sum_tree.device, self.sum_tree.lib
         self.stride = int(self.lib.gmz_move_record_bytes(self.N))
+        # byte range of each record field within a ring row (policy, board, header scalars, ...)
+        self._field = {name: slice(off, off + dt.itemsize) for name, (dt, off) in record_dtype(self.N).fields.items()}
         self.ring = torch.zeros((self.capacity, self.stride), dtype=torch.uint8, device=self.device)
         self.max_priority = torch.ones((), dtype=torch.float64, device=self.device)
         self.unroll = int(config.NUM_UNROLL_STEPS if unroll_steps is None else unroll_steps)
@@ -327,8 +299,8 @@ class DeviceReplayBuffer:
             return
         if int(pos.min()) < 0 or int(pos.max()) >= self.capacity:
             raise ValueError("ring position out of range")
-        self.ring[pos, 64:64 + 8 * self.A] = pol.view(torch.uint8).reshape(pos.numel(), 8 * self.A)      # gmz_move_record: policy f64[A]
-        self.ring[pos, 36:40] = val.view(torch.uint8).reshape(pos.numel(), 4)                             # header: value_target f32
+        self.ring[pos, self._field["policy"]] = pol.view(torch.uint8).reshape(pos.numel(), 8 * self.A)
+        self.ring[pos, self._field["value_target"]] = val.view(torch.uint8).reshape(pos.numel(), 4)
 
     def reanalyse(self, engines, first=None, count=None, evaluator="e0", eval_seed=0, logit_div=16, noise_seed=0):
         """Surge re-analysis (workers.py:243-305) of the records in the ring, in place: every position is searched again
@@ -385,9 +357,10 @@ class DeviceReplayBuffer:
             raise ValueError(f"stretch first={first}, count={count} reaches outside the {live} live records")
         if n > 0 and (first is not None or count is not None):
             ends = torch.tensor([(oldest + rel) % cap, (oldest + rel + n - 1) % cap], device=self.device)
-            h = self.ring[ends, :12].cpu().numpy().view(np.int32)          # header: game_seq, t, length
-            end = rel + n + int(h[1, 2]) - 1 - int(h[1, 1])
-            rel = max(0, rel - int(h[0, 1]))                               # a cut oldest game: its live suffix
+            h = torch.cat([self.ring[ends, self._field["t"]], self.ring[ends, self._field["length"]]], 1)
+            h = h.cpu().numpy().view(np.int32)                             # (t, length) of both ends
+            end = rel + n + int(h[1, 1]) - 1 - int(h[1, 0])
+            rel = max(0, rel - int(h[0, 0]))                               # a cut oldest game: its live suffix
             if end > live:
                 raise RuntimeError("ring records do not hold whole games")
             n = end - rel
@@ -439,7 +412,7 @@ class DeviceReplayBuffer:
         empty-cell count on the device.  Returns (rows int32 device [n], per-batch arena rows incl. one per padding game,
         per-batch step counts) -- the two lists from one device-to-host copy."""
         from .muzero import MuZeroDeviceSearch
-        dev, A, m = self.device, self.A, len(engines)
+        dev, m = self.device, len(engines)
         K = max(e.K for e in engines)
         table = np.ones((m, K + 1), np.int32)                 # [engine, k] -> rows; clamped to each engine's own K below
         kmax = np.array([e.K for e in engines], np.int64)
@@ -452,9 +425,8 @@ class DeviceReplayBuffer:
         dv = host.to(dev, non_blocking=True)
         nb = len(batches)
         d_first, d_kmax, d_table = dv[:nb], dv[nb:nb + m], dv[nb + m:].reshape(m, K + 1)
-        body = 64 + 20 * A                                    # gmz_move_record: board int8 [A]
         idx = (start + torch.arange(n, device=dev)) % self.capacity
-        empty = (self.ring[idx, body:body + A] == 0).sum(1)
+        empty = (self.ring[idx, self._field["board"]] == 0).sum(1)
         batch = torch.searchsorted(d_first, torch.arange(n, device=dev), right=True) - 1
         eng = batch % m
         rows = d_table[eng, torch.minimum(empty, d_kmax[eng])]
@@ -501,8 +473,7 @@ class DeviceReplayBuffer:
                 raise ValueError(f"{n_bad} live ring records cannot be rebuilt from their predecessor and header (board or "
                                  f"observation planes altered); the first is at ring position {(oldest + k_bad) % cap}")
             seg = (flags & 1).nonzero().reshape(-1)
-        body = 64 + 20 * A
-        base = self.ring[(oldest + seg) % cap, body:body + A].view(torch.int8)
+        base = self.ring[(oldest + seg) % cap, self._field["board"]].view(torch.int8)
         return {"format": RING_STATE_FORMAT, "version": RING_STATE_VERSION, "board_size": self.N, "capacity": cap,
                 "count": n, "write_ptr": wp, "headers": headers.cpu(), "policies": policies.cpu(), "seg_start": seg.cpu(),
                 "base_boards": base.cpu(), "tree": self.sum_tree.tree.cpu(), "max_priority": self.max_priority.cpu()}

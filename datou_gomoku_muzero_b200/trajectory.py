@@ -109,13 +109,12 @@ class TrajectoryStore:
         check(e.lib.gmz_traj_init(e.handle, C.byref(self.c), e._stream()), "gmz_traj_init")
         e.launches += 1
 
-    def harvest(self, copy_policies=True, recycle=True, unpark=True):
-        """Finished games since the last harvest -> list of dicts (host arrays).  With `recycle` their
-        slots go back on the free stack and (with `unpark`) parked games restart -- pass unpark=False after
-        play(restart=False) to leave finished games finished; a DeviceSliceStore keeps the slots (the games stay
-        resident for sampling) and recycles them itself when it evicts.  A game that recorded more moves than the
-        store's `max_moves` (only possible with a user-supplied max_moves below the remaining plies) comes back with
-        `length` clamped to what was recorded and `truncated` = True."""
+    def harvest(self, copy_policies=True, unpark=True):
+        """Finished games since the last harvest -> list of dicts (host arrays).  Their slots go back on the free
+        stack and (with `unpark`) parked games restart -- pass unpark=False after play(restart=False) to leave
+        finished games finished.  A game that recorded more moves than the store's `max_moves` (only possible with a
+        user-supplied max_moves below the remaining plies) comes back with `length` clamped to what was recorded and
+        `truncated` = True."""
         e = self.e
         n = int(self.fin_count.item())
         if n == 0:
@@ -141,8 +140,7 @@ class TrajectoryStore:
                             start_move_count=int(si[i, 1]), start_last_move=int(si[i, 2]),
                             truncated=bool(full_len[i] > self.max_moves)))
         self.fin_count.zero_()
-        if recycle:
-            self.release(slots, unpark=unpark)
+        self.release(slots, unpark=unpark)
         return out
 
     def pack_finished(self, recycle=True):
@@ -189,79 +187,6 @@ class TrajectoryStore:
         if unpark:
             check(e.lib.gmz_selfplay_unpark(e.handle, C.byref(self.c), e._stream()), "gmz_selfplay_unpark")
             e.launches += 1
-
-
-class DeviceSliceStore:
-    """Replay data resident on the GPU: finished games stay in their trajectory slots, a training
-    sample is the pair (slot, t), and `batch()` builds the trainer tuple (obs, act, rew, pi, val) of
-    workers.py:430-433 with one kernel.  n-step value targets are computed on the device when a game
-    is ingested (workers.py:144-152, 205).  Oldest games are evicted (slots recycled) past `capacity_games`.
-    The sample index is a device tensor (`index`, int32 [n, 2]); `batch()` takes (slot, t) pairs as a sequence or as
-    a tensor.  (replay_buffer.DeviceReplayBuffer is the variant that also holds the PER tree and stores packed move
-    records instead of keeping trajectory slots resident.)"""
-
-    def __init__(self, traj: "TrajectoryStore", capacity_games=None):
-        self.traj, e = traj, traj.e
-        self.e = e
-        n = traj.n_slots
-        self.capacity_games = int(capacity_games) if capacity_games else max(1, n - e.G - 1)
-        self.targets = torch.zeros((n, traj.max_moves), dtype=torch.float32, device=e.device)
-        self.length = torch.zeros(n, dtype=torch.int32, device=e.device)
-        self.winner = torch.zeros(n, dtype=torch.int32, device=e.device)
-        self.resident = []          # slots in ingestion order
-        self.index = torch.zeros((0, 2), dtype=torch.int32, device=e.device)   # (slot, t) of every stored slice, in add() order
-
-    def ingest(self, finished):
-        """finished: records from TrajectoryStore.harvest(recycle=False).  Returns the new (slot, t) samples."""
-        if not finished:
-            return []
-        e = self.e
-        slots = torch.tensor([r["slot"] for r in finished], dtype=torch.int32, device=e.device)
-        lens = torch.tensor([r["length"] for r in finished], dtype=torch.int32, device=e.device)
-        wins = torch.tensor([r["winner"] for r in finished], dtype=torch.int32, device=e.device)
-        self.length[slots.long()] = lens
-        self.winner[slots.long()] = wins
-        dpow = torch.tensor([config.DISCOUNT ** i for i in range(config.N_STEPS + 1)], dtype=torch.float64, device=e.device)
-        check(e.lib.gmz_value_targets(C.byref(self.traj.c), slots.data_ptr(), lens.data_ptr(), wins.data_ptr(), len(finished),
-                                      dpow.data_ptr(), int(config.N_STEPS), self.targets.data_ptr(), e._stream()),
-              "gmz_value_targets")
-        e.launches += 1
-        hs = np.array([r["slot"] for r in finished], np.int32)
-        hl = np.minimum(np.array([r["length"] for r in finished], np.int64), self.traj.max_moves)
-        new = np.stack([np.repeat(hs, hl), (np.arange(int(hl.sum())) - np.repeat(np.cumsum(hl) - hl, hl)).astype(np.int32)], axis=1)
-        self.resident += hs.tolist()
-        self.index = torch.cat([self.index, torch.as_tensor(new, device=e.device)])
-        if len(self.resident) > self.capacity_games:
-            n_old = len(self.resident) - self.capacity_games
-            old, self.resident = self.resident[:n_old], self.resident[n_old:]
-            old_t = torch.tensor(old, dtype=torch.int32, device=e.device)
-            self.index = self.index[~torch.isin(self.index[:, 0], old_t)]          # one mask, no host loop
-            self.traj.release(old_t)
-        return [tuple(x) for x in new.tolist()]
-
-    def batch(self, samples, rot_k=0, flip=False):
-        """samples: sequence of (slot, t).  Returns device tensors (obs f32 [B,U+1,3,N,N], act i32 [B,U],
-        rew f32 [B,U], pi f64 [B,U+1,A], val f32 [B,U+1]).  rot_k / flip = the k and flip that
-        calculate_loss draws (loss.py:37-38); the D4 augmentation of loss.py:39-51 is then applied by the
-        gather itself (act comes back augmented; padded entries stay -1, so the reference's `act != -1` mask,
-        loss.py:85, can be taken from the returned tensor)."""
-        e = self.e
-        st = samples.to(device=e.device, dtype=torch.int32) if torch.is_tensor(samples) else torch.tensor(samples, dtype=torch.int32, device=e.device)
-        st = st.reshape(-1, 2)
-        B, U, N, A = int(st.shape[0]), int(config.NUM_UNROLL_STEPS), e.N, e.A
-        s_slot, s_t = st[:, 0].contiguous(), st[:, 1].contiguous()
-        obs = torch.empty((B, U + 1, 3, N, N), dtype=torch.float32, device=e.device)
-        act = torch.empty((B, U), dtype=torch.int32, device=e.device)
-        rew = torch.empty((B, U), dtype=torch.float32, device=e.device)
-        pi = torch.empty((B, U + 1, A), dtype=torch.float64, device=e.device)
-        val = torch.empty((B, U + 1), dtype=torch.float32, device=e.device)
-        check(e.lib.gmz_build_batch_aug(C.byref(self.traj.c), N, self.targets.data_ptr(), self.length.data_ptr(),
-                                        self.winner.data_ptr(), s_slot.data_ptr(), s_t.data_ptr(), B, U, int(rot_k) % 4,
-                                        1 if flip else 0, obs.data_ptr(), act.data_ptr(), rew.data_ptr(), pi.data_ptr(),
-                                        val.data_ptr(), e._stream()),
-              "gmz_build_batch_aug")
-        e.launches += 1
-        return obs, act, rew, pi, val
 
 
 def final_rewards(num_moves, winner):

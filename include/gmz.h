@@ -210,27 +210,6 @@ int gmz_hidden_scatter(void *pool, const int32_t *slot, int num_games, int sims_
  * = +-1, 0 (draw) or GMZ_WINNER_NONE. */
 int gmz_game_step(gmz_engine *e, const int32_t *actions, int32_t *out_winner, gmz_stream stream);
 
-/* ---- trajectory post-processing on the device (workers.py:144-152, 183-222, 430-433) ---- */
-/* n-step value targets of finished games: slots / lengths / winners int32 [n_games] (device),
- * discount_pow f64 [n_steps+1] = discount**i as the host computes them, out targets f32
- * [n_slots][max_moves].  Final rewards follow workers.py:183-187. */
-int gmz_value_targets(const gmz_traj *traj, const int32_t *slots, const int32_t *lengths, const int32_t *winners,
-                      int n_games, const double *discount_pow, int n_steps, float *targets, gmz_stream stream);
-/* A batch of TrainingSlices (data_structures.py:20-26) rebuilt from resident games: sample b is
- * (sample_slot[b], sample_t[b]).  Outputs: obs f32 [B,U+1,3,N,N], act i32 [B,U] (pad -1), rew f32
- * [B,U], pi f64 [B,U+1,A], val f32 [B,U+1] -- the tuple data_loader_worker stacks (workers.py:430-433). */
-int gmz_build_batch(const gmz_traj *traj, int board_size, const float *targets, const int32_t *len_by_slot,
-                    const int32_t *win_by_slot, const int32_t *sample_slot, const int32_t *sample_t, int batch,
-                    int unroll, float *obs, int32_t *act, float *rew, double *pi, float *val, gmz_stream stream);
-/* The same batch with the trainer's D4 augmentation (calculate_loss, loss.py:37-51) applied while
- * gathering: planes and policies rotated rot_k (0..3) quarter turns as torch.rot90 does, then
- * flipped left-right if `flip`; actions by the reference's own index formula (loss.py:46-51),
- * padded entries stay -1. */
-int gmz_build_batch_aug(const gmz_traj *traj, int board_size, const float *targets, const int32_t *len_by_slot,
-                        const int32_t *win_by_slot, const int32_t *sample_slot, const int32_t *sample_t, int batch,
-                        int unroll, int rot_k, int flip, float *obs, int32_t *act, float *rew, double *pi, float *val,
-                        gmz_stream stream);
-
 /* ---- packed move records: the device-side trajectory hand-off (workers.py:172-230, 399-433) ---- */
 /* One fixed-stride record per move of a finished game: everything the reference's self-play loop emits for
  * that move.  Layout (stride = gmz_move_record_bytes(board_size), a multiple of 16):
@@ -266,7 +245,10 @@ int gmz_traj_pack(const gmz_traj *traj, int board_size, const int32_t *fin, int 
 /* A training batch (workers.py:430-433) gathered from a RING of `capacity` records: sample b is the record at
  * ring position positions[b] (the reference's data index, replay_buffer.py:80) plus the next `unroll` records of
  * the same game, padded past its end like workers.py:208-222; rot_k / flip = the trainer's D4 augmentation
- * (loss.py:37-51).  Outputs as gmz_build_batch. */
+ * (loss.py:37-51): planes and policies turned rot_k (0..3) quarter turns as torch.rot90 does, then flipped
+ * left-right if `flip`; actions by the reference's own index formula (loss.py:46-51), padded entries stay -1.
+ * Outputs: obs f32 [B,U+1,3,N,N], act i32 [B,U] (padding -1), rew f32 [B,U], pi f64 [B,U+1,A], val f32 [B,U+1]
+ * -- the tuple data_loader_worker stacks (workers.py:430-433). */
 int gmz_records_batch(const void *ring, int64_t capacity, int board_size, const int64_t *positions, int batch, int unroll,
                       int rot_k, int flip, float *obs, int32_t *act, float *rew, double *pi, float *val, gmz_stream stream);
 /* Missed-win flags of n_records consecutive records (a packed block or a stretch of the ring), read in place: the

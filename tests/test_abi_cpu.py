@@ -116,9 +116,7 @@ def test_entry_points_reject_bad_arguments_without_crashing():
         ("gmz_fill_gumbel", (N, 8, 0, 0, N)), ("gmz_game_step", (N, N, N, N)),
         ("gmz_traj_init", (N, N, N)), ("gmz_selfplay_e0", (N, N, 0, 16, 0, 8, 1, N)),
         ("gmz_selfplay_unpark", (N, N, N)), ("gmz_selfplay_step", (N, N, N, N, N, 1, N, N)),
-        ("gmz_play_counters", (N, N, N)), ("gmz_select_counters", (N, N, N)), ("gmz_value_targets", (N, N, N, N, 3, N, 10, N, N)),
-        ("gmz_build_batch", (N, 9, N, N, N, N, N, 4, 5, N, N, N, N, N, N)),
-        ("gmz_build_batch_aug", (N, 9, N, N, N, N, N, 4, 5, 1, 1, N, N, N, N, N, N)),
+        ("gmz_play_counters", (N, N, N)), ("gmz_select_counters", (N, N, N)),
         ("gmz_hidden_gather", (N, N, N, 4, 20, 4, 36, 256, N, 0, N, N)), ("gmz_hidden_scatter", (N, N, 4, 20, 4, 9216, N, N)),
         ("gmz_tactics_classify", (N, N, 4, 9, 5, N, N)), ("gmz_per_update", (N, 8, N, N, 4, N)),
         ("gmz_per_add", (N, 8, 0, N, 4, N, N)), ("gmz_per_sample", (N, 8, 8, N, 4, 0.4, N, N, N, N)),

@@ -26,10 +26,12 @@ def _load_game(traj, slot, z, game=0):
 @pytest.mark.parametrize("name", NAMES)
 def test_pack_kernel_matches_reference_game_record(name):
     """Records written by gmz_traj_pack == observations / boards / policies / rewards / n-step value targets of the
-    GameRecord the reference's universal_worker produced, bit for bit (incl. the float32-valued games)."""
+    GameRecord the reference's universal_worker produced, bit for bit (incl. the float32-valued games), and the
+    trainer batches gathered from them in a DeviceReplayBuffer == the TrainingSlices it cut."""
     import torch
     from datou_gomoku_muzero_b200.config import config
     from datou_gomoku_muzero_b200.engine import SearchEngine
+    from datou_gomoku_muzero_b200.replay_buffer import DeviceReplayBuffer
     from datou_gomoku_muzero_b200.trajectory import TrajectoryStore
     z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
     N, U, n_steps = int(z["params"][0]), int(z["params"][5]), int(z["params"][6])
@@ -60,6 +62,13 @@ def test_pack_kernel_matches_reference_game_record(name):
         sl = pg.training_slices(1)
         assert np.array_equal(np.stack([s.observation for s in sl]), z["slice_obs"])
         assert np.array_equal(np.stack([s.value_history for s in sl]), z["slice_val"])
+        # the device ring's batches of both games == the TrainingSlices the reference cut, bit for bit, same dtypes
+        buf = DeviceReplayBuffer(pg.n_moves, N)
+        buf.add_packed(pg)
+        batch = [x.cpu().numpy() for x in buf.batch(torch.arange(pg.n_moves, device="cuda"))]
+        for part in (slice(0, T), slice(T, 2 * T)):
+            for got, key in zip(batch, ("slice_obs", "slice_act", "slice_rew", "slice_pi", "slice_val")):
+                assert got.dtype == z[key].dtype and np.array_equal(got[part], z[key]), key
     finally:
         config.DISCOUNT, config.N_STEPS, config.NUM_UNROLL_STEPS = saved
 

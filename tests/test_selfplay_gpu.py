@@ -107,70 +107,56 @@ def test_reanalysis_matches_oracle_per_position():
         off += T
 
 
-def test_device_slice_store_matches_reference_slices():
-    """Device-side n-step targets + batch assembly vs the TrainingSlices the reference's universal_worker
-    cut (tests/golden/selfplay_az_9_100.npz), and vs the host post-processing on kernel-played games."""
+def test_device_ring_batches_match_host_slices():
+    """Trainer batches gathered from the device replay ring (gmz_traj_pack -> DeviceReplayBuffer.batch) vs the host
+    post-processing (build_game_record + cut_training_slices) of the same kernel-played games: two engines play the
+    same seeded E0 self-play, one is harvested to the host, the other packed into a ring.  The persistent kernel's
+    finish order is not fixed, so games are paired by engine game index and action sequence."""
     import torch
-    from datou_gomoku_muzero_b200.config import config
     from datou_gomoku_muzero_b200.engine import SearchEngine
+    from datou_gomoku_muzero_b200.replay_buffer import DeviceReplayBuffer
     from datou_gomoku_muzero_b200.selfplay import SelfPlayEngine
-    from datou_gomoku_muzero_b200.trajectory import (DeviceSliceStore, TrajectoryStore, build_game_record,
-                                                     cut_training_slices)
-    z = np.load(os.path.join(GOLDEN_DIR, "selfplay_az_9_100.npz"))
-    N, nir, S, K, seed, U, n_steps, version = (int(x) for x in z["params"][:8])
-    A = N * N
-    saved = (config.DISCOUNT, config.N_STEPS, config.NUM_UNROLL_STEPS)
-    config.DISCOUNT, config.N_STEPS, config.NUM_UNROLL_STEPS = float(z["discount"]), n_steps, U
-    try:
-        eng = SearchEngine(4, board_size=N, num_simulations=8)
-        traj = TrajectoryStore(eng, extra_slots=8)
-        store = DeviceSliceStore(traj)
-        # plant the reference's game in a free slot, as if the kernel had just finished it
-        T, slot = len(z["actions"]), 6
-        traj.policy[slot, :T] = torch.from_numpy(z["policies"]).cuda()
-        traj.value[slot, :T] = torch.from_numpy(z["search_values"]).cuda()
-        traj.action[slot, :T] = torch.from_numpy(z["actions"]).cuda()
-        traj.start_board[slot].zero_()
-        traj.start_info[slot] = torch.tensor([1, 0, -1, 0], dtype=torch.int32).cuda()
-        new = store.ingest([dict(slot=slot, game=0, length=T, winner=int(z["winner"]))])
-        assert new == [(slot, t) for t in range(T)]
-        np.testing.assert_array_equal(store.targets[slot, :T].cpu().numpy(), z["values_targets"].astype(np.float32))
-        obs, act, rew, pi, val = (x.cpu().numpy() for x in store.batch(new))
-        assert np.array_equal(obs, z["slice_obs"]) and np.array_equal(act, z["slice_act"])
-        assert np.array_equal(rew, z["slice_rew"]) and np.array_equal(pi, z["slice_pi"]) and np.array_equal(val, z["slice_val"])
-        assert obs.dtype == z["slice_obs"].dtype and pi.dtype == np.float64 and act.dtype == np.int32
-        # games the kernel played itself: device batch == host build_game_record + cut_training_slices
-        eng2 = SearchEngine(12, board_size=6, num_simulations=20)
-        sp = SelfPlayEngine(eng2, "e0", seed=2, noise_seed=3)
-        traj2 = TrajectoryStore(eng2, extra_slots=24)
-        store2 = DeviceSliceStore(traj2)
-        fin = []
-        while len(fin) < 6:
-            sp.play(moves_per_game=5, traj=traj2)
-            fin += traj2.harvest(recycle=False)
-        samples = store2.ingest(fin)
-        obs, act, rew, pi, val = (x.cpu().numpy() for x in store2.batch(samples))
-        off = 0
-        for r in fin:
-            sl = cut_training_slices(build_game_record(r))
-            for s in sl:
-                assert np.array_equal(obs[off], s.observation) and np.array_equal(act[off], s.action_history)
-                assert np.array_equal(rew[off], s.reward_history) and np.array_equal(pi[off], s.policy_history)
-                assert np.array_equal(val[off], s.value_history)
-                off += 1
-        assert off == len(samples)
-    finally:
-        config.DISCOUNT, config.N_STEPS, config.NUM_UNROLL_STEPS = saved
+    from datou_gomoku_muzero_b200.trajectory import TrajectoryStore, build_game_record, cut_training_slices
+    N, G = 6, 12
+    sps, trajs = [], []
+    for _ in range(2):
+        eng = SearchEngine(G, board_size=N, num_simulations=20)
+        sps.append(SelfPlayEngine(eng, "e0", seed=2, noise_seed=3))
+        trajs.append(TrajectoryStore(eng, extra_slots=24))
+    buf = DeviceReplayBuffer(4096, N)
+    fin, at = [], {}                                   # at: (game, actions) -> ring position of the game's first move
+    for _ in range(40):
+        sps[0].play(moves_per_game=5, traj=trajs[0])
+        fin += trajs[0].harvest()
+        sps[1].play(moves_per_game=5, traj=trajs[1])
+        pg = trajs[1].pack_finished()
+        if pg is not None:
+            for i in range(len(pg)):
+                at[(int(pg.table[i][1]), tuple(pg.game(i)["action"].tolist()))] = buf.sum_tree.write_ptr + int(pg.offsets[i])
+            buf.add_packed(pg)
+        pairs = [(r, at[k]) for r in fin if (k := (r["game"], tuple(r["actions"].tolist()))) in at]
+        if len(pairs) >= 6:
+            break
+    assert len(pairs) >= 6 and len(buf) < buf.capacity          # the ring has not wrapped: positions are as recorded
+    for r, p0 in pairs:
+        sl = cut_training_slices(build_game_record(r))
+        obs, act, rew, pi, val = (x.cpu().numpy() for x in buf.batch(torch.arange(p0, p0 + len(sl), device="cuda")))
+        for t, s in enumerate(sl):
+            assert np.array_equal(obs[t], s.observation) and np.array_equal(act[t], s.action_history)
+            assert np.array_equal(rew[t], s.reward_history) and np.array_equal(pi[t], s.policy_history)
+            assert np.array_equal(val[t], s.value_history)
 
 
 def test_device_batch_d4_augmentation_matches_reference_loss_path():
-    """gmz_build_batch_aug vs what the reference's calculate_loss feeds its networks (loss.py:37-51,
+    """gmz_records_batch vs what the reference's calculate_loss feeds its networks (loss.py:37-51,
     captured in tests/golden/augment_kat.npz) for all 8 symmetries, and vs the numpy restatement."""
     import torch
     from datou_gomoku_muzero_b200.config import config
     from datou_gomoku_muzero_b200.engine import SearchEngine
-    from datou_gomoku_muzero_b200.trajectory import DeviceSliceStore, TrajectoryStore
+    from datou_gomoku_muzero_b200.replay_buffer import DeviceReplayBuffer
+    from datou_gomoku_muzero_b200.trajectory import TrajectoryStore
     from oracle import oracle
+    from test_records_gpu import _load_game
     z = np.load(os.path.join(GOLDEN_DIR, "selfplay_az_6_36.npz"))
     g = np.load(os.path.join(GOLDEN_DIR, "augment_kat.npz"))
     N, nir, S, K, seed, U, n_steps, version = (int(x) for x in z["params"][:8])
@@ -181,21 +167,19 @@ def test_device_batch_d4_augmentation_matches_reference_loss_path():
     try:
         eng = SearchEngine(4, board_size=N, num_simulations=8)
         traj = TrajectoryStore(eng, extra_slots=8)
-        store = DeviceSliceStore(traj)
-        T, slot = len(z["actions"]), 5
-        traj.policy[slot, :T] = torch.from_numpy(z["policies"]).cuda()
-        traj.value[slot, :T] = torch.from_numpy(z["search_values"]).cuda()
-        traj.action[slot, :T] = torch.from_numpy(z["actions"]).cuda()
-        traj.start_board[slot].zero_()
-        traj.start_info[slot] = torch.tensor([1, 0, -1, 0], dtype=torch.int32).cuda()
-        store.ingest([dict(slot=slot, game=0, length=T, winner=int(z["winner"]))])
-        samples = [(slot, t) for t in pick]
-        base = [x.cpu().numpy() for x in store.batch(samples)]
+        slot = 5
+        T = _load_game(traj, slot, z)
+        traj.fin_queue[0] = torch.tensor([slot, 0, T, int(z["winner"])], dtype=torch.int32).cuda()
+        traj.fin_count.fill_(1)
+        buf = DeviceReplayBuffer(T, N)
+        buf.add_packed(traj.pack_finished())
+        samples = torch.tensor(pick, device="cuda")                    # the game fills ring positions 0 .. T-1
+        base = [x.cpu().numpy() for x in buf.batch(samples)]
         assert np.array_equal(base[0], g["obs"]) and np.array_equal(base[1], g["act"]) and np.array_equal(base[3], g["pi"])
         valid = g["act"] != -1
         for k in range(4):
             for f in (0, 1):
-                obs, act, rew, pi, val = (x.cpu().numpy() for x in store.batch(samples, rot_k=k, flip=bool(f)))
+                obs, act, rew, pi, val = (x.cpu().numpy() for x in buf.batch(samples, rot_k=k, flip=bool(f)))
                 tag = f"k{k}f{f}"
                 assert np.array_equal(obs, g["obs_" + tag]), tag
                 assert np.array_equal(pi.astype(np.float32), g["pi_" + tag]), tag

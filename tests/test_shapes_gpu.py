@@ -381,33 +381,6 @@ def test_packed_records_and_ring_batches(N, nir):
                              [slices[int(p)] for p in pos])
 
 
-@pytest.mark.parametrize("N,nir", [(7, 4), (12, 5), (17, 5)])
-def test_device_slice_store_batches(N, nir):
-    """DeviceSliceStore (trajectory slots kept resident, gmz_value_targets, gmz_build_batch_aug) against the host
-    GameRecord / cut_training_slices of the same games, for all eight (rot_k, flip)."""
-    from datou_gomoku_muzero_b200.engine import SearchEngine
-    from datou_gomoku_muzero_b200.selfplay import SelfPlayEngine
-    from datou_gomoku_muzero_b200.trajectory import DeviceSliceStore, TrajectoryStore, build_game_record, cut_training_slices
-    G = 8
-    eng = SearchEngine(G, board_size=N, n_in_row=nir, num_simulations=8)
-    sp = SelfPlayEngine(eng, "e0", seed=2, noise_seed=9)
-    traj = TrajectoryStore(eng, extra_slots=24)
-    store = DeviceSliceStore(traj)
-    fin = []
-    for _ in range(30):
-        sp.play(moves_per_game=N * N // 4, traj=traj)
-        fin += traj.harvest(recycle=False)
-        if len(fin) >= 4:
-            break
-    fin = fin[:12]
-    samples = store.ingest(fin)
-    slices = [s for r in fin for s in cut_training_slices(build_game_record(r))]
-    assert len(samples) == len(slices) > 0
-    for k in range(4):
-        for flip in (False, True):
-            _check_augmented((N, k, flip), store.batch(samples, rot_k=k, flip=flip), k, flip, slices)
-
-
 @pytest.fixture
 def _per():
     from datou_gomoku_muzero_b200.config import config

@@ -1,5 +1,5 @@
-"""Small end-to-end run for compute-sanitizer: fused search, stepwise search, self-play with trajectories,
-slice store, PER, tactics -- tiny sizes."""
+"""Small end-to-end run for compute-sanitizer: fused search, stepwise search, self-play packed into the device
+replay ring, PER, tactics -- tiny sizes."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -7,7 +7,7 @@ import numpy as np, torch
 from datou_gomoku_muzero_b200.config import config
 from datou_gomoku_muzero_b200.engine import SearchEngine
 from datou_gomoku_muzero_b200.selfplay import SelfPlayEngine
-from datou_gomoku_muzero_b200.trajectory import TrajectoryStore, DeviceSliceStore
+from datou_gomoku_muzero_b200.trajectory import TrajectoryStore
 from datou_gomoku_muzero_b200 import replay_buffer as rb
 from datou_gomoku_muzero_b200.tactics import classify_boards
 for N, S, G in ((6, 24, 10), (15, 40, 9), (19, 20, 5)):
@@ -17,15 +17,6 @@ for N, S, G in ((6, 24, 10), (15, 40, 9), (19, 20, 5)):
     gum = torch.empty((G, A), dtype=torch.float64, device="cuda"); eng.fill_gumbel(gum, 1, 0)
     eng.search_e0(gum, 3, 16, trace=True); eng.finalize()
     eng.search_stepwise_e0(gum, 3, 16); eng.finalize()
-    sp = SelfPlayEngine(eng, "e0", seed=1, noise_seed=2)
-    traj = TrajectoryStore(eng, extra_slots=8)
-    store = DeviceSliceStore(traj)
-    fin = []
-    for _ in range(3):
-        sp.play(moves_per_game=6, traj=traj); fin += traj.harvest(recycle=False)
-    samples = store.ingest(fin)
-    if samples:
-        store.batch(samples[:7])
     # packed records -> device replay ring + PER tree -> batch (float32 accumulation, dense logits)
     e32 = SearchEngine(G, board_size=N, num_simulations=S, accum_dtype="float32")
     sp32 = SelfPlayEngine(e32, "e0", seed=5, logit_div=0, noise_seed=6)
