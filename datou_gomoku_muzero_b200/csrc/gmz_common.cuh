@@ -156,22 +156,26 @@ __device__ __forceinline__ float warp_sum_f32(float v)
     for (int o = 16; o > 0; o >>= 1) v = __fadd_rn(v, __shfl_xor_sync(GMZ_FULL, v, o));
     return v;
 }
-// Sum of non-negative terms (each <= ~400, at least one == 1 up to rounding) in 2^-23 fixed point: ONE integer
-// REDUX instead of a five-step shuffle tree.  Absolute error <= 32 * 2^-24 on a sum >= 1 (certified select only).
+// Sum of non-negative terms (lane total <= ~400, at least one == 1 up to rounding) in 2^-23 fixed point: ONE integer
+// REDUX instead of a five-step shuffle tree (the largest legal total, 392 * 2^23, stays below 2^32).  Error: <= 2^-24
+// per lane from the fixed point, plus one float32 rounding of the integer total (exact for totals below 2), i.e.
+// <= 33 * 2^-24 relative on a sum >= 1 (certified select only; tests/test_numerics_gpu.py).
 __device__ __forceinline__ float warp_sum_fx(float v)
 {
     const unsigned q = __float2uint_rn(__fmul_rn(v, 8388608.0f));
     return __fmul_rn((float)__reduce_add_sync(GMZ_FULL, q), 1.1920928955078125e-07f);
 }
-// 1/x for x in the float range, to ~1.5e-14: float reciprocal + one Newton step (the certified select
-// path only needs ~1e-9; the exact path keeps the correctly rounded division).
+// 1/x for x in the float range, to <= 4e-14 relative (1.4e-14 measured on a B200): float reciprocal + one Newton
+// step (the certified select path only needs ~1e-9; the exact path keeps the correctly rounded division).
 __device__ __forceinline__ float rcp_approx(float x)
 {
     float r;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
-// exp(x) for x <= 0 to ~2^-22 relative: one multiply and MUFU.EX2 (results below 2^-126 flush to 0)
+// exp(x) for x <= 0: one multiply and MUFU.EX2 (results below 2^-126 flush to +0).  Relative error <= 2^-22 + 1.3e-7 |x|
+// for x = (float)d: the float32 roundings of d and of d * log2(e) each move the exponent by up to 2^-24 |d|, so the
+// error grows with |d| (bound ~1.2e-5 at d = -87.4, measured 7.5e-6 on a B200); only near 0 is it ex2.approx's ~2^-22.
 __device__ __forceinline__ float exp_approx(float x)
 {
     float r;
@@ -180,7 +184,7 @@ __device__ __forceinline__ float exp_approx(float x)
 }
 __device__ __forceinline__ double rcp_newton(double x)
 {
-    const double r = (double)rcp_approx((float)x);           // ~2^-23; one Newton step squares it: ~1.5e-14 relative,
+    const double r = (double)rcp_approx((float)x);           // ~1.5 * 2^-23; one Newton step squares it: <= 4e-14 relative,
     return fma(r, fma(-x, r, 1.0), r);                       // nine orders below what the certificate tolerates
 }
 // xor-butterfly sum: a+b == b+a exactly, so every lane ends with the same bits

@@ -168,10 +168,12 @@ __device__ __forceinline__ void game_reset(const Params &p, GState *s, int lane)
 }
 
 // Gumbel(0,1) noise from a counter-based splitmix64 stream: -log(-log(u)), u in (0,1) with 53 bits.
+// (z >> 11) + 0.5 rounds to even once z >> 11 >= 2^52, so z >> 11 = 2^53 - 1 would give u = 1 and +inf noise:
+// that draw is clamped to 1 - 2^-53, a value no other draw produces.
 __device__ __forceinline__ double gumbel_at(u64 seed_mixed, u64 counter)
 {
     const u64 z = mix64(seed_mixed + counter * E0_GOLD);
-    const double u = ((double)(z >> 11) + 0.5) * (1.0 / 9007199254740992.0);
+    const double u = fmin(((double)(z >> 11) + 0.5) * (1.0 / 9007199254740992.0), 1.0 - 1.0 / 9007199254740992.0);
     return -log(-log(u));
 }
 

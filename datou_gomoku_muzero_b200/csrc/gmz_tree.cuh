@@ -531,8 +531,9 @@ constexpr int kFastMaxVisited = 31;   // visited children (slots 1..31) + the be
 // of this node in the parent's block (slot 0 = not mirrored: root children, children past the 31st).
 struct PathReg { int node, mir, n; double W, R; };
 __device__ __forceinline__ char *blk_of(const Params &p, size_t ni) { return p.nBlk + ni * (size_t)kBlkBytes; }
-constexpr double kCertEps = 4.5e-5;   // > 6x the error bound of a probability on this path (float32 exp / summary ~3e-6,
-                                      //  fixed-point softmax denominator ~2e-6, fixed-point summary sum U ~2e-6)
+constexpr double kCertEps = 4.5e-5;   // > 2x the error bound of a probability on this path, ~1.8e-5: float32 exp at
+                                      // |d| <= 87.4 ~1.2e-5 (grows with |d|), softmax denominator with U's share ~6e-6,
+                                      // rcp_approx + two float32 roundings ~2e-7 (tests/test_numerics_gpu.py budget)
 
 // ub / lub / U / "ambiguous" for the candidate set `cand` (bit i = this lane's action i).  Ambiguous:
 // two different unvisited logits closer than 1e-6 -- float64 rounding of logit + sigma could merge
@@ -562,7 +563,7 @@ __device__ __forceinline__ void unvisited_summary(const float *lg, unsigned cand
         if (WITH_U) u = __fadd_rn(u, exp_approx(d));
         am |= (d < 0.0f) && (d > -1e-6f);
     }
-    U = WITH_U ? warp_sum_fx(u) : 0.0f;              // <= 8 terms per lane, each <= 1: one fixed-point REDUX (error <= 2e-6 of U >= 1)
+    U = WITH_U ? warp_sum_fx(u) : 0.0f;              // <= 12 terms per lane (NC = 3), each <= 1: one fixed-point REDUX (error <= 2e-6 of U >= 1)
     amb = __any_sync(GMZ_FULL, am);
 }
 

@@ -54,5 +54,5 @@ def test_dump_outputs_are_reproducible_and_match_the_oracle(tmp_path):
     o = oracle.selfplay_game(cfg, gum.cpu().numpy())
     assert o["T"] == T + 1                                   # a game needs at least 9 plies: it is still going
     assert int(a["action"][0]) == int(o["actions"][T - 1]) and a["value"][0] == o["values"][T - 1]
-    np.testing.assert_allclose(a["policy"][0], o["policies"][T - 1], rtol=1e-5, atol=1e-12)
+    np.testing.assert_allclose(a["policy"][0], o["policies"][T - 1], rtol=1e-12, atol=1e-15)
     assert np.array_equal(a["board"][0], o["boards"][T].reshape(-1).astype(np.float32)) and a["winner"][0] == 2

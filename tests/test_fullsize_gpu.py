@@ -52,7 +52,7 @@ def test_full_size_search_properties_and_oracle_subset():
     g_host = gum.cpu().numpy()
     opol, oval, oact, ovis = oracle.search_batch(cfg, boards[sub], players[sub], last[sub], mc[sub], g_host[sub])
     assert np.array_equal(vis[sub], ovis) and np.array_equal(act[sub], oact) and np.array_equal(val[sub], oval)
-    np.testing.assert_allclose(pol[sub], opol, rtol=1e-5, atol=1e-12)
+    np.testing.assert_allclose(pol[sub], opol, rtol=1e-12, atol=1e-15)
     # --- the stepwise kernels (external-evaluator path) give the same bits as the fused kernel
     eng.search_stepwise_e0(gum, seed)
     pol3, val3, act3, vis3 = (t.cpu().numpy() for t in eng.finalize())
@@ -93,7 +93,7 @@ def test_full_size_selfplay_bookkeeping():
 def test_full_size_games_move_for_move_against_the_oracle(div, accum):
     """The bench configuration itself -- 15x15, 400 simulations, the persistent multi-move launch with in-kernel
     restart -- compared MOVE FOR MOVE with the CPU oracle's game loop: every move, root value and the winner of the
-    first finished games, policies within 1e-5 (quantised float64 and dense-logit float32-accumulation evaluators)."""
+    first finished games, policies within 1e-12 relative (quantised float64 and dense-logit float32-accumulation evaluators)."""
     import torch
     from datou_gomoku_muzero_b200.engine import SearchEngine
     from datou_gomoku_muzero_b200.selfplay import SelfPlayEngine
@@ -125,6 +125,6 @@ def test_full_size_games_move_for_move_against_the_oracle(div, accum):
         assert o["T"] == T and o["winner"] == r["winner"], (g, o["T"], T)
         assert np.array_equal(o["actions"], r["actions"]), g
         assert np.array_equal(o["values"], r["values"]), g
-        np.testing.assert_allclose(r["policies"], o["policies"], rtol=1e-5, atol=1e-12)
+        np.testing.assert_allclose(r["policies"], o["policies"], rtol=1e-12, atol=1e-15)
         checked += 1
     assert checked >= 8

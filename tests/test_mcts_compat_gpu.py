@@ -57,8 +57,8 @@ def test_search_game_reproduces_reference(cfg, mode, N):
         assert isinstance(policy, np.ndarray) and policy.dtype == np.float64 and policy.shape == (N * N,)
         assert isinstance(action, int) and action == c["action"], tag
         assert isinstance(value, (float, np.floating))
-        np.testing.assert_allclose(value, c["value"], rtol=1e-5, atol=1e-12, err_msg=tag)
-        np.testing.assert_allclose(policy, c["policy"], rtol=1e-5, atol=1e-12, err_msg=tag)
+        np.testing.assert_allclose(value, c["value"], rtol=1e-12, atol=1e-15, err_msg=tag)
+        np.testing.assert_allclose(policy, c["policy"], rtol=1e-12, atol=1e-15, err_msg=tag)
         assert q.n_initial == c["n_initial"] and q.n_recurrent == c["n_recurrent"], tag   # same request pattern
 
 
@@ -128,7 +128,7 @@ def test_search_batch_host_api():
     cfgo = oracle.make_config(board_size=N, num_simulations=S, eval_seed=seed)
     opol, oval, oact, _ = oracle.search_batch(cfgo, boards, players, last, mc, gum)
     assert np.array_equal(act, oact) and np.array_equal(val, oval)
-    np.testing.assert_allclose(pol, opol, rtol=1e-5, atol=1e-12)
+    np.testing.assert_allclose(pol, opol, rtol=1e-12, atol=1e-15)
 
 
 def test_pipelined_batch_search_matches_oracle():
@@ -157,7 +157,7 @@ def test_pipelined_batch_search_matches_oracle():
             pol, val, act = (x.copy() for x in pipe.result(tickets[b - 1]))
             opol, oval, oact, _ = oracle.search_batch(cfgo, *batches[b - 1])
             assert np.array_equal(act, oact) and np.array_equal(val, oval), b
-            np.testing.assert_allclose(pol, opol, rtol=1e-5, atol=1e-12)
+            np.testing.assert_allclose(pol, opol, rtol=1e-12, atol=1e-15)
     pol, val, act = pipe.result(tickets[-1])
     opol, oval, oact, _ = oracle.search_batch(cfgo, *batches[-1])
     assert np.array_equal(act, oact) and np.array_equal(val, oval)

@@ -98,7 +98,7 @@ def test_network_driven_search_replayed_through_the_oracle(accum):
             r = oracle.search(cfg, boards[g], players[g], last[g], mc[g], gum_h[g])
             assert np.array_equal(vis[g], r["visits"]), (accum, g)
             assert act[g] == r["action"] and val[g] == r["value"], (accum, g)
-            np.testing.assert_allclose(pol[g], r["policy"], rtol=1e-5, atol=1e-12)
+            np.testing.assert_allclose(pol[g], r["policy"], rtol=1e-12, atol=1e-15)
     finally:
         oracle.set_eval_callback(None)
 

@@ -1,7 +1,7 @@
 """GPU parity: the CUDA engine (through the C ABI) against (a) the golden vectors produced by
 the imported reference and (b) the CPU oracle on seeded random inputs.  Bar: visit counts,
-chosen moves, per-simulation leaf traces and terminal flags bit-exact; values / policies within
-1e-5 relative (north_star); in practice values are bit-exact and policies agree to ~1e-15."""
+chosen moves, per-simulation leaf traces, terminal flags and root values bit-exact; policies within
+1e-12 relative + 1e-15 absolute, a few ulp of float64 (a float32 improved policy would fail)."""
 import os
 
 import numpy as np
@@ -11,7 +11,7 @@ from _golden_util import GOLDEN_DIR, load_search_cases
 
 pytestmark = pytest.mark.gpu
 
-RTOL = 1e-5   # north_star tolerance for Q / value targets
+RTOL, ATOL = 1e-12, 1e-15   # policies: the oracle's own tolerance against the reference goldens
 
 
 def _engine(c, G=1, mode=None):
@@ -30,9 +30,9 @@ def _check(c, pol, val, act, vis, ta, td, tag):
         n = len(c["leaf_actions"])
         assert np.array_equal(ta[:n], c["leaf_actions"]), f"{tag}: leaf action trace"
         assert np.array_equal(td[:n], c["leaf_depths"]), f"{tag}: leaf depth trace"
-    np.testing.assert_allclose(val, c["value"], rtol=RTOL, atol=1e-12, err_msg=tag)
+    np.testing.assert_allclose(val, c["value"], rtol=RTOL, atol=ATOL, err_msg=tag)
     assert float(val) == c["value"], f"{tag}: root value bits"        # float64 / float32 accumulation is bit-exact
-    np.testing.assert_allclose(pol, c["policy"], rtol=RTOL, atol=1e-12, err_msg=tag)
+    np.testing.assert_allclose(pol, c["policy"], rtol=RTOL, atol=ATOL, err_msg=tag)
 
 
 @pytest.mark.parametrize("N", [6, 9, 15, 19])
@@ -192,8 +192,8 @@ def test_random_positions_match_oracle(N, S, G, div, accum):
     assert act[0] == -1 and pol[0].sum() == 0 and val[0] == 0.0      # sentinel (mcts.py:214-215)
     assert np.array_equal(vis, ovis)
     assert np.array_equal(act, oact)
-    np.testing.assert_allclose(val, oval, rtol=RTOL, atol=1e-12)
-    np.testing.assert_allclose(pol, opol, rtol=RTOL, atol=1e-12)
+    np.testing.assert_allclose(val, oval, rtol=RTOL, atol=ATOL)
+    np.testing.assert_allclose(pol, opol, rtol=RTOL, atol=ATOL)
     assert np.array_equal(val, oval), "value accumulation should be bit-exact"
     # the roots must come back unchanged (search() must not mutate the game)
     b2, p2, l2, m2 = (t.cpu().numpy() for t in eng.get_roots())
@@ -249,7 +249,7 @@ def test_muzero_device_search_matches_oracle(N, S, G):
     opol, oval, oact, ovis = oracle.search_batch(cfg, boards, players, last, mc, gumbel)
     assert np.array_equal(vis, ovis) and np.array_equal(act, oact)
     assert np.array_equal(val, oval)
-    np.testing.assert_allclose(pol, opol, rtol=RTOL, atol=1e-12)
+    np.testing.assert_allclose(pol, opol, rtol=RTOL, atol=ATOL)
     assert evals_per_search(S, 16, 16) == {100: 33, 400: 100, 50: 22}[S]      # SURVEY App. A.6 batch schedule
 
 
@@ -306,7 +306,7 @@ def test_muzero_fused_search_matches_oracle(N, S, G, div, accum):
                              accum_dtype=int(accum == "float32"))
     opol, oval, oact, ovis = oracle.search_batch(cfg, boards, players, last, mc, gumbel)
     assert np.array_equal(vis, ovis) and np.array_equal(act, oact) and np.array_equal(val, oval)
-    np.testing.assert_allclose(pol, opol, rtol=RTOL, atol=1e-12)
+    np.testing.assert_allclose(pol, opol, rtol=RTOL, atol=ATOL)
     r = oracle.search(cfg, boards[1], players[1], last[1], mc[1], gumbel[1], trace=True)
     n = r["n_evals"]
     assert np.array_equal(ta[1].cpu().numpy()[:n], r["leaf_actions"]) and np.array_equal(td[1].cpu().numpy()[:n], r["leaf_depths"])

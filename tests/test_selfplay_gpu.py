@@ -48,7 +48,7 @@ def test_selfplay_games_match_oracle(N, S, G, mode):
         assert o["T"] == r["length"], (g, o["T"], r["length"])
         assert np.array_equal(o["actions"], r["actions"]) and o["winner"] == r["winner"], g
         assert np.array_equal(o["values"], r["values"]), g
-        np.testing.assert_allclose(r["policies"], o["policies"], rtol=1e-5, atol=1e-12)
+        np.testing.assert_allclose(r["policies"], o["policies"], rtol=1e-12, atol=1e-15)
         checked += 1
     assert checked >= 8
 
@@ -93,7 +93,7 @@ def test_reanalysis_matches_oracle_per_position():
         b, pl, lm, mc = positions_of(gr, N)
         T = len(gr.actions)
         opol, oval, oact, _ = oracle.search_batch(cfg, b, pl, lm, mc, allnoise[off:off + T])
-        np.testing.assert_allclose(pol, opol, rtol=1e-5, atol=1e-12)
+        np.testing.assert_allclose(pol, opol, rtol=1e-12, atol=1e-15)
         assert np.array_equal(vals, oval)                       # the re-searched root values, bit for bit
         assert len(targets) == T and all(isinstance(t, float) for t in targets)
         # the new value targets: workers.py:291-292 restated (float32 rewards there, unlike self-play: float32 sums)
