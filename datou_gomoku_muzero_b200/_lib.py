@@ -29,6 +29,12 @@ class GmzTraj(C.Structure):
                 ("fin_queue", C.c_void_p), ("fin_count", C.c_void_p)]
 
 
+class GmzMatch(C.Structure):
+    _fields_ = [("n_openings", C.c_int32), ("reserved", C.c_int32), ("open_boards", C.c_void_p), ("open_players", C.c_void_p),
+                ("open_last", C.c_void_p), ("open_mc", C.c_void_p), ("cursor", C.c_void_p), ("slot_ticket", C.c_void_p),
+                ("slot_ply", C.c_void_p), ("results", C.c_void_p), ("moves", C.c_void_p), ("finished", C.c_void_p)]
+
+
 class GmzError(RuntimeError):
     pass
 
@@ -62,6 +68,9 @@ SIGNATURES = {
     "gmz_select_counters": (C.c_int, [_P, _P, _P]),
     "gmz_hidden_gather": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P]),
     "gmz_hidden_scatter": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "gmz_match_start": (C.c_int, [_P, _P, C.POINTER(GmzMatch), _P]),
+    "gmz_match_noise": (C.c_int, [_P, _P, C.POINTER(GmzMatch), C.c_uint64, _P, _P, _P]),
+    "gmz_match_step": (C.c_int, [_P, _P, C.POINTER(GmzMatch), _P, _P, _P]),
     "gmz_move_record_bytes": (C.c_size_t, [C.c_int]),
     "gmz_traj_pack": (C.c_int, [C.POINTER(GmzTraj), C.c_int, _P, C.c_int, _P, _P, C.c_int, _P, _P]),
     "gmz_records_batch": (C.c_int, [_P, C.c_int64, C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),

@@ -210,6 +210,40 @@ int gmz_hidden_scatter(void *pool, const int32_t *slot, int num_games, int sims_
  * = +-1, 0 (draw) or GMZ_WINNER_NONE. */
 int gmz_game_step(gmz_engine *e, const int32_t *actions, int32_t *out_winner, gmz_stream stream);
 
+/* ---- matches: two engines play each other (player A = engine a, player B = engine b) ---------------- */
+/* Caller-owned match state; every pointer is a device pointer.  Opening o is played twice: ticket 2o with A moving first,
+ * ticket 2o+1 with B moving first; the first mover takes the opening's side to move.  Slot g of engine a always holds a
+ * game A is to move in, slot g of engine b one B is to move in; after every ply the two games of slot g change engines.
+ * A slot whose incoming game ended (or that had none) takes the next opening of its owner's queue (engine a: A-first
+ * tickets, engine b: B-first tickets) or, once that queue is empty, the inactive full-board root.
+ * Gumbel noise of ply k of opening o = gmz_fill_gumbel(seed, offset = (o*A + k)*A) for both games of the pair. */
+typedef struct gmz_match {
+    int32_t n_openings;          /* O >= 1 */
+    int32_t reserved;
+    const int8_t *open_boards;   /* [O][A]    {-1,0,+1} */
+    const int8_t *open_players;  /* [O]       side to move, +-1 */
+    const int32_t *open_last;    /* [O]       last move, -1 = None */
+    const int32_t *open_mc;      /* [O]       move count */
+    int32_t *cursor;             /* [2]       next opening of the A-first / B-first queue (zeroed by gmz_match_start) */
+    int32_t *slot_ticket;        /* [2][G]    ticket in slot g of engine a (row 0) / b (row 1), -1 = idle */
+    int32_t *slot_ply;           /* [2][G]    plies played so far in that game */
+    int32_t *results;            /* [2O][4]   winner colour (+-1, 0 draw, GMZ_WINNER_NONE while unfinished), length,
+                                  *           first mover (0 = A, 1 = B), A's colour; written when the ticket is dealt */
+    int32_t *moves;              /* [2O][A]   actions by ply, -1 past the end; set to -1 when the ticket is dealt */
+    int32_t *finished;           /* [1]       games finished (zeroed by gmz_match_start) */
+} gmz_match;
+/* Clear the cursors and the finished counter and fill every slot of both engines from the two queues. */
+int gmz_match_start(gmz_engine *a, gmz_engine *b, const gmz_match *m, gmz_stream stream);
+/* gumbel_a / gumbel_b f64 [G,A]: the noise of the game in each slot of engine a / b (zeros for idle slots). */
+int gmz_match_noise(gmz_engine *a, gmz_engine *b, const gmz_match *m, uint64_t seed, double *gumbel_a, double *gumbel_b,
+                    gmz_stream stream);
+/* After gmz_finalize on both engines: play action_a int32 [G] on engine a's roots and action_b on engine b's
+ * (do_move + get_game_ended), log the moves, write the result rows of finished games, count them, swap the games of
+ * every slot between the engines and refill the slots whose incoming game ended.  A live game whose action is outside
+ * [0, A) ends with winner GMZ_WINNER_NONE (counted as finished). */
+int gmz_match_step(gmz_engine *a, gmz_engine *b, const gmz_match *m, const int32_t *action_a, const int32_t *action_b,
+                   gmz_stream stream);
+
 /* ---- packed move records: the device-side trajectory hand-off (workers.py:172-230, 399-433) ---- */
 /* One fixed-stride record per move of a finished game: everything the reference's self-play loop emits for
  * that move.  Layout (stride = gmz_move_record_bytes(board_size), a multiple of 16):
