@@ -209,7 +209,7 @@ class Arena:
 
     def __init__(self, engine_a, engine_b, evaluator_a="e0", evaluator_b="e0", *, eval_seed_a=0, eval_seed_b=0,
                  logit_div_a=16, logit_div_b=16, seed=0, check_every=4):
-        from .mcts import check_budget, resolve_searchers
+        from .mcts import resolve_searchers
         from .muzero import MuZeroDeviceSearch
         if engine_a is engine_b:
             raise ValueError("the two players need two different engines")
@@ -217,20 +217,16 @@ class Arena:
                         ("n_in_row", lambda e: e.cfg.n_in_row), ("device", lambda e: e.device)):
             if f(engine_a) != f(engine_b):
                 raise ValueError(f"the engines differ in {what}: {f(engine_a)} vs {f(engine_b)}")
-        for ev, div in ((evaluator_a, logit_div_a), (evaluator_b, logit_div_b)):
-            if isinstance(ev, str) and ev == "e0" and (div < 0 or div & (div - 1)):
-                raise ValueError("an 'e0' player needs logit_div 0 (dense) or a power of two")
         self.engines = (engine_a, engine_b)
-        self.searchers = (resolve_searchers([engine_a], evaluator_a)[0], resolve_searchers([engine_b], evaluator_b)[0])
-        self.eval_seeds = (int(eval_seed_a), int(eval_seed_b))
-        self.logit_divs = (int(logit_div_a), int(logit_div_b))
+        self.searchers = (resolve_searchers([engine_a], evaluator_a, eval_seed_a, logit_div_a)[0],
+                          resolve_searchers([engine_b], evaluator_b, eval_seed_b, logit_div_b)[0])
         self.seed, self.check_every = int(seed), max(1, int(check_every))
         G, A, dev = engine_a.G, engine_a.A, engine_a.device
         self.budgets = []
         for s in self.searchers:             # learned dynamics: every game gets the largest budget any root can need
             if isinstance(s, MuZeroDeviceSearch):
                 most = int(s.budget_table().max())
-                check_budget(s, most)
+                s.check_budget(most)
                 rows = torch.full((G,), most, dtype=torch.int32, device=dev)
                 self.budgets.append((rows, G * most, most - 1))
             else:
@@ -271,7 +267,6 @@ class Arena:
         overlap), both decisions, then gmz_match_step on the current stream.  Nothing is read back to the host."""
         if self._buf is None:
             raise RuntimeError("start() the match first")
-        from .mcts import search_roots
         a, b = self.engines
         cur = self._cur()
         st = C.c_void_p(cur.cuda_stream)
@@ -280,7 +275,7 @@ class Arena:
         for i, eng in enumerate(self.engines):
             self.streams[i].wait_stream(cur)
             with torch.cuda.stream(self.streams[i]):
-                search_roots(eng, self.gumbel[i], self.searchers[i], self.eval_seeds[i], self.logit_divs[i], self.budgets[i])
+                self.searchers[i].search(self.gumbel[i], self.budgets[i])
                 eng.finalize(want_visits=False)
         for s in self.streams:
             cur.wait_stream(s)

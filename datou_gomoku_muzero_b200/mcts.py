@@ -107,12 +107,12 @@ class _GumbelEngineMCTS(MCTS):
     def for_engine(cls, engine, evaluator="e0", eval_seed=0, logit_div=16):
         """Batched searches on `engine` with any evaluator `resolve_searchers` accepts (resolved once, here)."""
         import torch
-        searcher = resolve_searchers([engine], evaluator)[0]
+        searcher = resolve_searchers([engine], evaluator, eval_seed, logit_div)[0]
         self = cls(0, None, None)
         G, A = engine.G, engine.A
         pin = dict(pin_memory=True)
         self._batch = dict(
-            engine=engine, evaluator=searcher, eval_seed=int(eval_seed), logit_div=int(logit_div),
+            engine=engine, searcher=searcher,
             h_rows=torch.empty(G, dtype=torch.int32, **pin), d_rows=torch.empty(G, dtype=torch.int32, device=engine.device),
             h_boards=torch.empty((G, A), dtype=torch.int8, **pin), h_players=torch.empty(G, dtype=torch.int8, **pin),
             h_last=torch.empty(G, dtype=torch.int32, **pin), h_mc=torch.empty(G, dtype=torch.int32, **pin),
@@ -159,46 +159,80 @@ class _GumbelEngineMCTS(MCTS):
         else:
             eng.fill_gumbel(b["d_gumbel"], int(device_noise[0]), int(device_noise[1]))
         from .muzero import MuZeroDeviceSearch
-        budget = None
-        if isinstance(b["evaluator"], MuZeroDeviceSearch):      # per-game node budgets from the host boards
-            rows = host_budgets(b["evaluator"], b["h_boards"].numpy())
+        searcher, budget = b["searcher"], None
+        if isinstance(searcher, MuZeroDeviceSearch):      # per-game node budgets from the host boards
+            rows = searcher.host_budgets(b["h_boards"].numpy())
             b["h_rows"].numpy()[...] = rows
             keys += ("rows",)
             budget = (b["d_rows"], int(rows.sum()), int(rows.max()) - 1)
         for k in keys:
             b["d_" + k].copy_(b["h_" + k], non_blocking=True)
         eng.set_roots(b["d_boards"], b["d_players"], b["d_last"], b["d_mc"])
-        search_roots(eng, b["d_gumbel"], b["evaluator"], b["eval_seed"], b["logit_div"], budget)
+        searcher.search(b["d_gumbel"], budget)
         pol, val, act, _ = eng.finalize(want_visits=False)
         b["o_policy"].copy_(pol, non_blocking=True)
         b["o_value"].copy_(val, non_blocking=True)
         b["o_action"].copy_(act, non_blocking=True)
 
 
-def resolve_searchers(engines, evaluator):
+class E0Search:
+    """The fixed evaluator E0 in the fused search kernel (either engine mode): evaluator seed `seed`, logits divided by
+    `logit_div` (0 = dense logits, else a power of two).  A searcher as resolve_searchers describes."""
+
+    def __init__(self, engine, seed=0, logit_div=16):
+        seed, logit_div = int(seed), int(logit_div)
+        if logit_div < 0 or logit_div & (logit_div - 1):
+            raise ValueError("an 'e0' evaluator needs logit_div 0 (dense) or a power of two")
+        self.e, self.seed, self.logit_div = engine, seed, logit_div
+
+    def search(self, gumbel, budget=None):
+        self.e.search_e0(gumbel, self.seed, self.logit_div)
+
+
+class StepwiseSearch:
+    """An eager evaluator fn(obs f32 [G,3,N,N]) -> (logits f32 [G,A], values [G]) driving the stepwise kernels (AlphaZero
+    mode): root_obs -> fn -> root_expand, then S - 1 rounds of select -> fn -> expand_backup.  A searcher as
+    resolve_searchers describes."""
+
+    def __init__(self, engine, fn):
+        self.e, self.fn = engine, fn
+
+    def search(self, gumbel, budget=None):
+        e = self.e
+        lg, v = self.fn(e.root_obs())
+        e.root_expand(lg, v, gumbel)
+        for _ in range(e.S - 1):
+            lg, v = self.fn(e.select())
+            e.expand_backup(lg, v)
+
+
+def resolve_searchers(engines, evaluator, eval_seed=0, logit_div=16):
     """One searcher per engine for `evaluator`, checked before anything is enqueued (ValueError otherwise):
-      "e0"                              -> "e0": the fixed evaluator in the fused kernel (either engine mode);
+      "e0"                              -> an E0Search(engine, eval_seed, logit_div) per engine (either engine mode);
       callable f(obs f32 [G,3,N,N]) -> (logits f32 [G,A], values [G])
-                                        -> itself: eager select -> f -> expand_backup loop (AlphaZero mode);
+                                        -> a StepwiseSearch per engine: eager select -> f -> expand_backup (AlphaZero);
       torch.nn.Module (GomokuNetEZ)     -> a network.NetworkSearch per engine, bf16, one CUDA graph per step (AlphaZero);
       (initial_fn, recurrent_fn)        -> a muzero.MuZeroDeviceSearch(graph=True) per engine (MuZero mode);
-      [searcher, ...]                   -> already-built NetworkSearch / MuZeroDeviceSearch objects, one bound to each
-                                           engine in order (reused across calls: no re-capture, update_weights swaps
-                                           weights in place).
-    A lone NetworkSearch / MuZeroDeviceSearch stands for a one-element list."""
+      [searcher, ...]                   -> already-built searchers of those four types, one bound to each engine in
+                                           order (reused across calls: no re-capture, update_weights swaps weights in
+                                           place).
+    A lone searcher stands for a one-element list.  Every searcher `s` has `s.e`, the engine it drives, and
+    `s.search(gumbel, budget=None)`, which enqueues one search of every root loaded in that engine on the current stream
+    (follow with engine.finalize()); `budget` = (rows int32 device [G], arena rows, steps) gives a MuZeroDeviceSearch
+    per-game node budgets in its compact arena and its exact step count, and is unused by the others."""
     import torch
     from .muzero import MuZeroDeviceSearch
     from .network import NetworkSearch
     engines = list(engines)
-    built = (NetworkSearch, MuZeroDeviceSearch)
+    built = (E0Search, StepwiseSearch, NetworkSearch, MuZeroDeviceSearch)
     if isinstance(evaluator, built):
         evaluator = [evaluator]
     if isinstance(evaluator, (tuple, list)) and evaluator and all(isinstance(x, built) for x in evaluator):
         if len(evaluator) != len(engines):
             raise ValueError(f"{len(evaluator)} searchers for {len(engines)} engines: pass one per engine")
         for s, e in zip(evaluator, engines):
-            kind = "MuZero" if isinstance(s, MuZeroDeviceSearch) else "AlphaZero"
-            if e.mode != kind:
+            kind = "MuZero" if isinstance(s, MuZeroDeviceSearch) else None if isinstance(s, E0Search) else "AlphaZero"
+            if kind is not None and e.mode != kind:
                 raise ValueError(f"a {type(s).__name__} needs a {kind}-mode engine, not a {e.mode}-mode one")
             if s.e is not e:
                 raise ValueError(f"the {type(s).__name__} drives a different engine")
@@ -206,7 +240,7 @@ def resolve_searchers(engines, evaluator):
     if isinstance(evaluator, str):
         if evaluator != "e0":
             raise ValueError(f"unknown evaluator {evaluator!r}")
-        return ["e0"] * len(engines)
+        return [E0Search(e, eval_seed, logit_div) for e in engines]
     pair = isinstance(evaluator, (tuple, list)) and len(evaluator) == 2 and all(callable(f) for f in evaluator)
     module = isinstance(evaluator, torch.nn.Module)
     for e in engines:
@@ -219,49 +253,12 @@ def resolve_searchers(engines, evaluator):
         return [MuZeroDeviceSearch(e, evaluator[0], evaluator[1], graph=True) for e in engines]
     if module:
         return [NetworkSearch(e, evaluator) for e in engines]
-    return [evaluator] * len(engines)
+    return [StepwiseSearch(e, evaluator) for e in engines]
 
 
 def host_budgets(mz, boards):
-    """Per-game node budgets (int32 [G]) of a MuZeroDeviceSearch for roots given as host boards int8 [G, A]: the root
-    plus one node per recurrent evaluation, for k = min(K, empty cells) root survivors."""
-    k = np.minimum((np.asarray(boards) == 0).sum(axis=1), mz.e.K)
-    rows = mz.budget_table()[k].astype(np.int32)
-    check_budget(mz, int(rows.max()))
-    return rows
-
-
-def check_budget(mz, most_rows):
-    if most_rows > mz.nodes:
-        raise ValueError(f"the MuZeroDeviceSearch holds {mz.nodes} tree nodes per game (nodes_per_game); a root here needs "
-                         f"{most_rows}")
-
-
-def search_roots(eng, gumbel, evaluator="e0", eval_seed=0, logit_div=16, budget=None):
-    """One search of every root loaded in `eng`, enqueued on the current stream (follow with eng.finalize).  `evaluator`
-    is one engine's entry of `resolve_searchers`: "e0" runs the fused kernel (either engine mode); a NetworkSearch or
-    MuZeroDeviceSearch runs its graph-captured steps; a callable f(obs) -> (logits, values) drives the stepwise kernels
-    (AlphaZero mode).  A MuZeroDeviceSearch takes `budget` = (rows int32 device [G], arena rows, steps): per-game node
-    budgets in its compact arena and the exact number of steps, so the search reads nothing back to the host."""
-    from .muzero import MuZeroDeviceSearch
-    from .network import NetworkSearch
-    if isinstance(evaluator, str) and evaluator == "e0":
-        eng.search_e0(gumbel, eval_seed, logit_div)
-        return
-    if isinstance(evaluator, NetworkSearch):
-        evaluator.search(gumbel)
-        return
-    if isinstance(evaluator, MuZeroDeviceSearch):
-        if budget is None:
-            evaluator.search(gumbel)
-        else:
-            evaluator.search(gumbel, max_steps=budget[2], rows=budget[0], arena_rows=budget[1])
-        return
-    lg, v = evaluator(eng.root_obs())
-    eng.root_expand(lg, v, gumbel)
-    for _ in range(eng.S - 1):
-        lg, v = evaluator(eng.select())
-        eng.expand_backup(lg, v)
+    """mz.host_budgets(boards) for a MuZeroDeviceSearch `mz`, under the name callers of this module import."""
+    return mz.host_budgets(boards)
 
 
 class PipelinedBatchSearch:
@@ -277,8 +274,8 @@ class PipelinedBatchSearch:
     def __init__(self, engines, cls=None, evaluator="e0", eval_seed=0, logit_div=16):
         import torch
         cls = cls or AlphaZeroMCTS
-        searchers = resolve_searchers(engines, evaluator)
-        self.lanes = [cls.for_engine(e, s, eval_seed, logit_div) for e, s in zip(engines, searchers)]
+        searchers = resolve_searchers(engines, evaluator, eval_seed, logit_div)
+        self.lanes = [cls.for_engine(e, s) for e, s in zip(engines, searchers)]
         self.streams = [torch.cuda.Stream(device=e.device) for e in engines]
         for e, s in zip(engines, self.streams):      # work already enqueued on the engines (e.g. a ring re-analysis) comes first
             s.wait_stream(torch.cuda.current_stream(e.device))

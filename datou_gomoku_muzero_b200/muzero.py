@@ -13,7 +13,7 @@ import torch
 import torch.nn.functional as F
 
 from ._lib import check
-from .network import GomokuNetEZ, _fold, _fold_heads, _support_scalar, capture_stream
+from .network import GomokuNetEZ, GraphStepSearch, _fold, _fold_heads, _support_scalar
 
 _M64 = (1 << 64) - 1
 
@@ -38,7 +38,7 @@ def evals_per_search(num_simulations, num_top_actions, n_survivors):
     return evals
 
 
-class MuZeroDeviceSearch:
+class MuZeroDeviceSearch(GraphStepSearch):
     """initial_fn(obs f32 [G,3,N,N]) -> (logits f32 [G,A], values [G], hidden [G, ...])
     recurrent_fn(hidden [G, ...], actions int64 [G]) -> (logits, values, rewards [G], next_hidden [G, ...])
     Hidden rows may be any dtype / shape (4-byte multiples); the pool is allocated from the first
@@ -46,8 +46,8 @@ class MuZeroDeviceSearch:
     the gathered batch is a channels_last tensor without a copy.
 
     Pool layouts: by default game g owns rows g*nodes_per_game .. g*nodes_per_game + nodes_per_game - 1.  A search given
-    per-game budgets (`rows`, re-analysis) uses one compact arena instead: game g owns rows base[g] .. base[g] + rows[g] - 1,
-    base the exclusive prefix sum of `rows`; a node at or beyond its game's budget is not stored (skip slot) and is counted
+    per-game budgets (`budget`, re-analysis) uses one compact arena instead: game g owns rows base[g] .. base[g] + rows[g] - 1,
+    base the exclusive prefix sum of the budgets; a node at or beyond its game's budget is not stored (skip slot) and is counted
     in `overflow` (int64 device scalar).  `nodes_per_game` then caps the budget a game may ask for.
 
     One simulation step = gmz_select_mz -> gmz_hidden_gather -> recurrent_fn -> gmz_hidden_scatter ->
@@ -59,11 +59,11 @@ class MuZeroDeviceSearch:
     def __init__(self, engine, initial_fn, recurrent_fn, nodes_per_game=None, graph=False, graph_warmup=3):
         if engine.mode != "MuZero":
             raise ValueError("MuZeroDeviceSearch needs an engine created with mode='MuZero'")
-        self.e, self.initial_fn, self.recurrent_fn = engine, initial_fn, recurrent_fn
+        super().__init__(engine, graph, graph_warmup)
+        self.initial_fn, self.recurrent_fn = initial_fn, recurrent_fn
         self.nodes = int(nodes_per_game) if nodes_per_game else engine.S
         self.pool = None
         self.evaluations = 0
-        self.use_graph, self.graph_warmup, self.graph = bool(graph), int(graph_warmup), None
         self.fused = hasattr(recurrent_fn, "forward_fused") and getattr(recurrent_fn, "embed", None) is not None
         self._root_slot = (torch.arange(engine.G, dtype=torch.int32, device=engine.device) * engine.S).contiguous()
         self.arena = False                              # pool layout: g * nodes + node (False) or base[g] + node (True)
@@ -175,30 +175,38 @@ class MuZeroDeviceSearch:
         self._scatter(child, self._rows(h_out))
         e.expand_backup(lg, v, r)
 
-    def _capture(self):
-        e = self.e
-        n0 = e.launches
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph, stream=capture_stream(e.device)):
-            self._step()
-        self._launches_per_step = e.launches - n0
-        e.launches = n0                                   # capture launched nothing
-
     def budget_table(self):
         """Tree nodes a search can create, by the number of root survivors k = min(K, empty cells) = 0..K: the root plus
         one node per recurrent evaluation (int64 numpy [K+1])."""
         e = self.e
         return np.array([evals_per_search(e.S, e.K, k) + 1 for k in range(e.K + 1)], dtype=np.int64)
 
+    def host_budgets(self, boards):
+        """Per-game node budgets (int32 [G]) for roots given as host boards int8 [G, A]: the root plus one node per
+        recurrent evaluation, for k = min(K, empty cells) root survivors (ValueError if one exceeds nodes_per_game)."""
+        k = np.minimum((np.asarray(boards) == 0).sum(axis=1), self.e.K)
+        rows = self.budget_table()[k].astype(np.int32)
+        self.check_budget(int(rows.max()))
+        return rows
+
+    def check_budget(self, most_rows):
+        if most_rows > self.nodes:
+            raise ValueError(f"the MuZeroDeviceSearch holds {self.nodes} tree nodes per game (nodes_per_game); a root here "
+                             f"needs {most_rows}")
+
     @torch.no_grad()
-    def search(self, gumbel, max_steps=None, rows=None, arena_rows=None):
+    def search(self, gumbel, budget=None, max_steps=None):
         """Runs one search for every game from the engine's current roots; call engine.finalize() after.
 
-        rows (int32 device tensor [G]) / arena_rows (host int >= rows.sum()): per-game node budgets in one compact arena of
-        at least `arena_rows` rows (grown, and the graph re-captured, only when that is more than the arena has).  The
-        search then runs exactly `max_steps` steps (the largest evaluation count of the batch) and reads nothing back to
-        the host; steps after a game has finished evaluate nothing for it."""
+        budget = (rows, arena_rows, steps): rows (int32 device tensor [G]) / arena_rows (host int >= rows.sum()) are per-game
+        node budgets in one compact arena of at least `arena_rows` rows (grown, and the graph re-captured, only when that is
+        more than the arena has).  The search then runs exactly `steps` steps (the largest evaluation count of the batch)
+        and reads nothing back to the host; steps after a game has finished evaluate nothing for it.  Without a budget,
+        `max_steps` (if given and non-zero) caps the number of steps."""
         e = self.e
+        rows, arena_rows = None, None
+        if budget is not None:
+            rows, arena_rows, max_steps = budget
         arena = rows is not None
         lg, v, h = self.initial_fn(e.root_obs())
         pool_rows = self._ensure_pool(h, arena_rows if arena else None)
@@ -214,13 +222,7 @@ class MuZeroDeviceSearch:
         while steps < limit:
             if not arena and steps + 2 > self.nodes:          # this step may create node id steps + 1
                 raise RuntimeError("hidden-state pool too small: pass a larger nodes_per_game")
-            if self.use_graph and self.graph is None and steps >= self.graph_warmup:
-                self._capture()
-            if self.graph is not None:
-                self.graph.replay()
-                e.launches += self._launches_per_step
-            else:
-                self._step()
+            self._advance(steps)
             steps += 1
             self.evaluations += 1
             if not arena and steps % 8 == 0 and steps < limit and int(e._mz_out[0].max().item()) < 0:   # every game is done

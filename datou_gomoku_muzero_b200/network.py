@@ -23,6 +23,38 @@ def capture_stream(device):
     return None if cur == torch.cuda.default_stream(device) else cur
 
 
+class GraphStepSearch:
+    """Base of the searchers that replay one simulation step as a CUDA graph (NetworkSearch, MuZeroDeviceSearch).  The
+    subclass's `_step()` enqueues one step on engine `e`; `_advance(i)`, for step i of a search, runs it eagerly for the
+    first `graph_warmup` steps, then captures it once on capture_stream and replays the graph from then on.  The engine's
+    launch counter counts a replay as the launches of one eager step and the capture as none.  `graph = None` drops the
+    graph, which is captured again at the next step past the warm-up."""
+
+    sync_before_capture = False
+
+    def __init__(self, engine, graph, graph_warmup):
+        self.e = engine
+        self.use_graph, self.graph_warmup, self.graph = bool(graph), int(graph_warmup), None
+        self._launches_per_step = 0
+
+    def _advance(self, i):
+        e = self.e
+        if self.use_graph and self.graph is None and i >= self.graph_warmup:
+            n0 = e.launches
+            if self.sync_before_capture:
+                torch.cuda.synchronize(e.device)
+            self.graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(self.graph, stream=capture_stream(e.device)):
+                self._step()
+            self._launches_per_step = e.launches - n0
+            e.launches = n0                                # capturing launched nothing
+        if self.graph is not None:
+            self.graph.replay()
+            e.launches += self._launches_per_step
+        else:
+            self._step()
+
+
 def _c3(cin, cout):
     return nn.Conv2d(cin, cout, 3, padding=1, bias=False)
 
@@ -275,7 +307,7 @@ class DeviceEvaluator:
         return self.logits, self.values
 
 
-class NetworkSearch:
+class NetworkSearch(GraphStepSearch):
     """AlphaZeroMCTS.search (mcts.py:197-280) for the engine's G games with a NETWORK evaluator, one CUDA graph per
     simulation step: { gmz_select -> folded network -> gmz_expand_backup } -- the reference's per-simulation round trip
     (mcts.py:253 -> workers.py:339-355: pickle, queue, H2D, forward, D2H, queue, unpickle) collapsed into one graph
@@ -283,14 +315,14 @@ class NetworkSearch:
     bf16 NHWC, the network's input format.  Create the engine with accum_dtype="float32": the network returns float32
     values, and that is the dtype the reference's tree then accumulates in (SURVEY App. A.7)."""
 
+    sync_before_capture = True
+
     def __init__(self, engine, net, dtype=torch.bfloat16, graph=True, graph_warmup=2):
         if engine.mode != "AlphaZero":
             raise ValueError("NetworkSearch drives an AlphaZero-mode engine (MuZero mode: muzero.MuZeroDeviceSearch)")
-        self.e = engine
+        super().__init__(engine, graph, graph_warmup)
         self.obs = engine.obs_buffer_bf16() if dtype == torch.bfloat16 else engine.leaf_obs
         self.ev = DeviceEvaluator(net, self.obs, dtype=dtype, graph=False)
-        self.use_graph, self.graph_warmup, self.graph = bool(graph), int(graph_warmup), None
-        self._launches_per_step = 0
 
     def update_weights(self, state_dict):
         self.ev.update_weights(state_dict)           # in place: a captured graph keeps replaying against the same buffers
@@ -301,32 +333,16 @@ class NetworkSearch:
         self.ev._forward()
         e.expand_backup(self.ev.logits, self.ev.values)
 
-    def _capture(self):
-        e = self.e
-        n0 = e.launches
-        torch.cuda.synchronize(e.device)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph, stream=capture_stream(e.device)):
-            self._step()
-        self._launches_per_step = e.launches - n0
-        e.launches = n0                                # capturing launched nothing
-
     @torch.no_grad()
-    def search(self, gumbel, num_simulations=None):
-        """One search for every game from the engine's current roots; follow with engine.finalize()."""
+    def search(self, gumbel, budget=None, num_simulations=None):
+        """One search for every game from the engine's current roots, `num_simulations` (default S) simulations; follow
+        with engine.finalize().  `budget` is unused (node budgets are a MuZeroDeviceSearch matter).  Returns the number
+        of simulation steps after the root's."""
         e = self.e
         e.root_obs(self.obs)
         self.ev._forward()
         e.root_expand(self.ev.logits, self.ev.values, gumbel)
         steps = (e.S if num_simulations is None else int(num_simulations)) - 1
-        done = 0
-        while done < steps:
-            if self.use_graph and self.graph is None and done >= self.graph_warmup:
-                self._capture()
-            if self.graph is not None:
-                self.graph.replay()
-                e.launches += self._launches_per_step
-            else:
-                self._step()
-            done += 1
-        return done
+        for i in range(steps):
+            self._advance(i)
+        return max(steps, 0)

@@ -92,7 +92,7 @@ def reanalyse_positions(engines, boards, players, last_moves, move_counts, evalu
     positions.  They stream through `len(engines)` engines in flight (PipelinedBatchSearch: pinned staging, H2D, search,
     D2H), G positions per batch; the last batch is padded with inactive (full-board) roots.  evaluator: anything
     mcts.resolve_searchers takes -- "e0", a callable, a GomokuNetEZ module, a pair (initial_fn, recurrent_fn) for
-    MuZero-mode engines (pass cls=MuZeroMCTS), or one already-built NetworkSearch / MuZeroDeviceSearch per engine; MuZero
+    MuZero-mode engines (pass cls=MuZeroMCTS), or one already-built searcher per engine; MuZero
     searchers get per-game node budgets from the host boards, as DeviceReplayBuffer.reanalyse does.  Noise: `gumbel` float64
     [n, A] from the host, or drawn on the device from `noise_seed` (position i uses counters i*A .. i*A + A - 1).
     Returns (policies float64 [n, A], values float64 [n]); want_policies=False returns (None, values),

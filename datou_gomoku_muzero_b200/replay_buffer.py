@@ -321,8 +321,9 @@ class DeviceReplayBuffer:
         (the fixed evaluator, either engine mode; eval_seed / logit_div as SearchEngine.search_e0); a callable
         f(obs f32 [G,3,N,N]) -> (logits, values) (eager, AlphaZero mode); a GomokuNetEZ module (a bf16 NetworkSearch per
         engine, AlphaZero mode); a pair (initial_fn, recurrent_fn) (a MuZeroDeviceSearch(graph=True) per engine, MuZero
-        mode); or a list of already-built NetworkSearch / MuZeroDeviceSearch objects, one bound to each engine, which keep
-        their captured graphs from call to call.  Anything else raises ValueError before any kernel is enqueued.
+        mode); or a list of already-built searchers of those kinds (mcts.E0Search, mcts.StepwiseSearch, NetworkSearch,
+        MuZeroDeviceSearch), one bound to each engine, which keep their captured graphs from call to call.  Anything else
+        raises ValueError before any kernel is enqueued.
         Noise is drawn on the device: record k of the widened stretch uses Gumbel counters k*A .. k*A + A-1 of
         `noise_seed`, as reanalyse_positions gives its position k.
 
@@ -334,11 +335,9 @@ class DeviceReplayBuffer:
 
         Policies and values never go to the host; the only host reads are that budget read (MuZero searchers) and the two
         boundary headers of an explicit stretch."""
-        from .mcts import check_budget, resolve_searchers, search_roots
+        from .mcts import resolve_searchers
         from .muzero import MuZeroDeviceSearch
         engines = list(engines)
-        if isinstance(evaluator, str) and evaluator != "e0":
-            raise ValueError(f"unknown evaluator {evaluator!r}")
         if not engines:
             raise ValueError("reanalyse needs at least one engine")
         for e in engines:
@@ -346,7 +345,7 @@ class DeviceReplayBuffer:
                 raise ValueError(f"engine board size {e.N} differs from the buffer's {self.N}")
             if e.device != self.device:
                 raise ValueError(f"engine on {e.device}, buffer on {self.device}")
-        searchers = resolve_searchers(engines, evaluator)
+        searchers = resolve_searchers(engines, evaluator, eval_seed, logit_div)
         cap, live = self.capacity, self.sum_tree.count
         oldest = self.sum_tree.write_ptr if live == cap else 0
         if first is not None and not 0 <= int(first) < cap:
@@ -378,7 +377,7 @@ class DeviceReplayBuffer:
             rows, total, steps = budgets
             for b, (i, _, _) in enumerate(batches):
                 if isinstance(searchers[i], MuZeroDeviceSearch):
-                    check_budget(searchers[i], steps[b] + 1)
+                    searchers[i].check_budget(steps[b] + 1)
             arena = [max((total[b] for b, x in enumerate(batches) if x[0] == i), default=0) for i in range(len(engines))]
         cur = torch.cuda.current_stream(self.device)
         streams = [torch.cuda.Stream(device=self.device) for _ in engines]
@@ -395,7 +394,7 @@ class DeviceReplayBuffer:
                 if isinstance(searchers[i], MuZeroDeviceSearch):      # padding games: inactive roots, one row each
                     budget = (rows[s0:s0 + k] if k == e.G else torch.cat((rows[s0:s0 + k], rows.new_ones(e.G - k))),
                               arena[i], steps[b])
-                search_roots(e, gumbel[i], searchers[i], eval_seed, logit_div, budget)
+                searchers[i].search(gumbel[i], budget)
                 pol, val, _, _ = e.finalize(want_visits=False)
                 check(self.lib.gmz_records_writeback(_ptr(self.ring), cap, self.N, pos, k, _ptr(pol), _ptr(val), e._stream()),
                       "gmz_records_writeback")

@@ -8,6 +8,7 @@ import numpy as np
 import torch
 
 from .engine import SearchEngine
+from .mcts import E0Search, resolve_searchers
 
 
 class SelfPlayEngine:
@@ -17,25 +18,18 @@ class SelfPlayEngine:
     `f(obs f32 [G,3,N,N]) -> (logits f32 [G,A], values f32/f64 [G])` run on the device (eager stepwise path); or --
     for an engine in MuZero mode -- a pair `(initial_fn, recurrent_fn)` / a `muzero.MuZeroDeviceSearch`
     (learned dynamics in the tree, hidden states in the device pool; MuZeroMCTS.search, mcts.py:288-362).  The evaluator
-    is resolved by mcts.resolve_searchers, as for re-analysis."""
+    is resolved by mcts.resolve_searchers, as for re-analysis, into `self.searcher`; seed / logit_div configure "e0"."""
 
     def __init__(self, engine: SearchEngine, evaluator="e0", seed=0, logit_div=16, noise_seed=0):
         self.e = engine
-        self.evaluator = evaluator
-        self.seed, self.logit_div, self.noise_seed = int(seed), int(logit_div), int(noise_seed)
+        self.searcher = resolve_searchers([engine], evaluator, seed, logit_div)[0]
+        self.noise_seed = int(noise_seed)
         G, A = engine.G, engine.A
         self.gumbel = torch.empty((G, A), dtype=torch.float64, device=engine.device)
         self.noise_counter = 0
         self.moves_played = 0
         self.games_finished = 0
         self.done_mask = torch.zeros(G, dtype=torch.uint8, device=engine.device)
-        from .mcts import resolve_searchers
-        from .muzero import MuZeroDeviceSearch
-        from .network import NetworkSearch
-        searcher = resolve_searchers([engine], evaluator)[0]
-        self.ns = searcher if isinstance(searcher, NetworkSearch) else None
-        self.mz = searcher if isinstance(searcher, MuZeroDeviceSearch) else None
-        self._e0 = isinstance(evaluator, str)
         engine.reset_games()
 
     def search(self, gumbel=None):
@@ -45,20 +39,7 @@ class SelfPlayEngine:
             e.fill_gumbel(self.gumbel, self.noise_seed, self.noise_counter)
             self.noise_counter += self.gumbel.numel()
             gumbel = self.gumbel
-        if self._e0:
-            e.search_e0(gumbel, self.seed, self.logit_div)
-        elif self.ns is not None:
-            self.ns.search(gumbel)
-        elif self.mz is not None:
-            self.mz.search(gumbel)
-        else:
-            obs = e.root_obs()
-            lg, v = self.evaluator(obs)
-            e.root_expand(lg, v, gumbel)
-            for _ in range(e.S - 1):
-                obs = e.select()
-                lg, v = self.evaluator(obs)
-                e.expand_backup(lg, v)
+        self.searcher.search(gumbel)
         return e.finalize(want_visits=False)
 
     def step(self, restart=True, traj=None):
@@ -83,10 +64,11 @@ class SelfPlayEngine:
         run of any length never parks a game."""
         e = self.e
         total = int(moves_per_game)
+        e0 = self.searcher if isinstance(self.searcher, E0Search) else None
 
         def advance(n):
-            if self._e0:
-                e.selfplay_e0(e.G * n, self.seed, self.logit_div, self.noise_seed, traj, restart)
+            if e0 is not None:
+                e.selfplay_e0(e.G * n, e0.seed, e0.logit_div, self.noise_seed, traj, restart)
                 self.moves_played += e.G * n
             else:
                 for _ in range(n):
@@ -95,7 +77,7 @@ class SelfPlayEngine:
         if sink is None or traj is None:
             advance(total)
             return
-        if chunk is None and not self._e0:
+        if chunk is None and e0 is None:
             chunk = 1              # lock-step games finish in bursts and a move costs S network batches: pack after every move
         if chunk is None:          # a game ends about every A/3 moves at the earliest in practice; spare slots absorb the finishes
             spare = max(1, traj.n_slots - e.G)

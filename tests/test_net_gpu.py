@@ -214,7 +214,7 @@ def test_bf16_network_against_fp32_network_at_8x128():
     assert rep["bf16"]["move_agreement"] > 0.5 and rep["bf16"]["mean_visit_l1"] < 0.35, rep
 
 
-def test_selfplay_with_the_network_play_equals_stepping():
+def test_selfplay_with_the_network_searcher_play_equals_stepping():
     """SelfPlayEngine with a GomokuNetEZ evaluator (the production path of universal_worker, workers.py:129-241):
     play(sink=...) -- lock-step network searches cut into chunks, finished games packed on the device and handed
     to the sink -- produces exactly the games a plain loop of step() calls does, every game is a legal finished
@@ -232,7 +232,7 @@ def test_selfplay_with_the_network_play_equals_stepping():
     def run(chunked):
         e = SearchEngine(G, board_size=N, num_simulations=S, n_in_row=4, accum_dtype="float32")
         sp = SelfPlayEngine(e, net if chunked else NetworkSearch(e, net), noise_seed=77)
-        assert sp.ns is not None
+        assert isinstance(sp.searcher, NetworkSearch)
         traj = TrajectoryStore(e, extra_slots=8 * G)
         got = []
         if chunked:

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from datou_gomoku_muzero_b200.mcts import host_budgets, resolve_searchers
+from datou_gomoku_muzero_b200.mcts import E0Search, StepwiseSearch, resolve_searchers
 from datou_gomoku_muzero_b200.muzero import MuZeroDeviceSearch, evals_per_search
 
 
@@ -24,15 +24,24 @@ def _ev(obs):
     ("MuZero", torch.nn.Linear(1, 1)),               # a module is an AlphaZero evaluator (NetworkSearch)
     ("AlphaZero", "e1"), ("MuZero", "e1"),
     ("AlphaZero", 3), ("AlphaZero", []), ("MuZero", [_ev]),
+    ("AlphaZero", "e0"),                             # with logit_div=12: the fused kernels take 0 or a power of two
 ])
 def test_resolver_refuses(mode, evaluator):
     with pytest.raises(ValueError):
-        resolve_searchers([_eng(mode), _eng(mode)], evaluator)
+        resolve_searchers([_eng(mode), _eng(mode)], evaluator, logit_div=12)
 
 
-def test_resolver_keeps_e0_and_callables():
-    assert resolve_searchers([_eng("MuZero"), _eng("AlphaZero")], "e0") == ["e0", "e0"]
-    assert resolve_searchers([_eng("AlphaZero")] * 3, _ev) == [_ev] * 3
+def test_resolver_wraps_e0_and_callables_in_searchers():
+    engines = [_eng("MuZero"), _eng("AlphaZero")]
+    got = resolve_searchers(engines, "e0", eval_seed=7, logit_div=0)
+    assert len(got) == 2
+    for s, e in zip(got, engines):
+        assert isinstance(s, E0Search) and s.e is e and (s.seed, s.logit_div) == (7, 0)
+    engines = [_eng("AlphaZero") for _ in range(3)]
+    got = resolve_searchers(engines, _ev)
+    assert len(got) == 3
+    for s, e in zip(got, engines):
+        assert isinstance(s, StepwiseSearch) and s.e is e and s.fn is _ev
 
 
 def test_host_budgets_follow_the_evaluation_schedule():
@@ -42,11 +51,11 @@ def test_host_budgets_follow_the_evaluation_schedule():
     boards = rs.choice(np.array([-1, 0, 1], np.int8), size=(40, 36), p=[0.4, 0.2, 0.4])
     boards[0] = 1                                     # a full board: the inactive padding root
     boards[1] = 0
-    rows = host_budgets(mz, boards)
+    rows = mz.host_budgets(boards)
     k = np.minimum((boards == 0).sum(1), 16)
     assert rows.dtype == np.int32
     assert rows.tolist() == [evals_per_search(32, 16, int(x)) + 1 for x in k]
     assert rows[0] == 1 and rows[1] == evals_per_search(32, 16, 16) + 1
     mz.nodes = int(rows.max()) - 1
     with pytest.raises(ValueError):
-        host_budgets(mz, boards)
+        mz.host_budgets(boards)

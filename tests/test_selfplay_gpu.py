@@ -236,12 +236,12 @@ def test_stepwise_selfplay_with_external_evaluator_matches_persistent_kernel():
         assert np.array_equal(a["values"], b["values"]) and np.array_equal(a["policies"], b["policies"]), g
 
 
-def test_muzero_stepwise_selfplay_matches_persistent_kernel():
+def test_muzero_searcher_selfplay_matches_persistent_kernel():
     """MuZero mode: SelfPlayEngine with (initial_fn, recurrent_fn) = E0 as torch ops (hidden states through
     the device pool kernels) plays the same games as the persistent MuZero-mode kernel."""
     import torch
     from datou_gomoku_muzero_b200.engine import SearchEngine
-    from datou_gomoku_muzero_b200.muzero import TorchE0
+    from datou_gomoku_muzero_b200.muzero import MuZeroDeviceSearch, TorchE0
     from datou_gomoku_muzero_b200.selfplay import SelfPlayEngine
     from datou_gomoku_muzero_b200.trajectory import TrajectoryStore
     N, S, G, seed, nseed = 6, 40, 12, 9, 33
@@ -255,7 +255,7 @@ def test_muzero_stepwise_selfplay_matches_persistent_kernel():
     e2 = SearchEngine(G, board_size=N, num_simulations=S, mode="MuZero")
     e0 = TorchE0(N, seed=seed)
     sp2 = SelfPlayEngine(e2, (e0.initial, e0.recurrent), noise_seed=nseed)
-    assert sp2.mz is not None
+    assert isinstance(sp2.searcher, MuZeroDeviceSearch)
     t2 = TrajectoryStore(e2, extra_slots=64)
     counters = np.zeros(G, np.int64)
     fin2 = []
