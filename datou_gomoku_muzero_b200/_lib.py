@@ -35,6 +35,12 @@ class GmzMatch(C.Structure):
                 ("slot_ply", C.c_void_p), ("results", C.c_void_p), ("moves", C.c_void_p), ("finished", C.c_void_p)]
 
 
+class GmzTreeOut(C.Structure):
+    _fields_ = [(name, C.c_void_p) for name in (
+        "num_nodes", "sim_count", "root", "minmax", "halving", "topk_action", "topk_gumbel", "topk_logit", "topk_round",
+        "root_logits", "parent", "action", "depth", "visits", "value_sum", "reward", "prior_logit")]
+
+
 class GmzError(RuntimeError):
     pass
 
@@ -71,6 +77,7 @@ SIGNATURES = {
     "gmz_match_start": (C.c_int, [_P, _P, C.POINTER(GmzMatch), _P]),
     "gmz_match_noise": (C.c_int, [_P, _P, C.POINTER(GmzMatch), C.c_uint64, _P, _P, _P]),
     "gmz_match_step": (C.c_int, [_P, _P, C.POINTER(GmzMatch), _P, _P, _P]),
+    "gmz_tree_export": (C.c_int, [_P, C.POINTER(GmzTreeOut), _P]),
     "gmz_move_record_bytes": (C.c_size_t, [C.c_int]),
     "gmz_traj_pack": (C.c_int, [C.POINTER(GmzTraj), C.c_int, _P, C.c_int, _P, _P, C.c_int, _P, _P]),
     "gmz_records_batch": (C.c_int, [_P, C.c_int64, C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),

@@ -276,6 +276,13 @@ class SearchEngine:
             return torch.stack(tr_a, 1) if tr_a else None, torch.stack(tr_d, 1) if tr_d else None
         return None, None
 
+    # ------------------------------------------------------------------ inspection
+    def export_tree(self, out=None):
+        """Every game's current search tree, the root's Gumbel top-k and halving rounds, as device tensors
+        (searchtree.SearchTrees; one kernel on the current stream, no host read).  `out`: a previous export to refill."""
+        from .searchtree import export_tree
+        return export_tree(self, out)
+
     # ------------------------------------------------------------------ game step
     def game_step(self, actions):
         a = self._dev(actions, torch.int32).reshape(self.G)

@@ -45,6 +45,7 @@ class _GumbelEngineMCTS(MCTS):
         super().__init__(worker_id, request_queue, result_queue)
         self._engines = {}
         self._batch = None
+        self._last = None       # (engine, move) of the last search(game), for last_tree()
 
     # ------------------------------------------------------------------ queue protocol (mcts.py:73-85)
     def _remote_initial_inference(self, obs):
@@ -100,7 +101,17 @@ class _GumbelEngineMCTS(MCTS):
         value = val[0].cpu().numpy()[()]
         if eng.accum_dtype == "float32":
             value = np.float32(value)          # root.get_value() is an np.float32 in this mode (exact: it was computed in float32)
-        return pol[0].cpu().numpy(), value, int(act[0].item())
+        self._last = (eng, int(act[0].item()))
+        return pol[0].cpu().numpy(), value, self._last[1]
+
+    def last_tree(self):
+        """The tree of the last `search(game)` as host numpy arrays (searchtree.SearchTrees.game), its principal variation
+        starting with the move `search` returned: the expected line, every root move's visits / Q / prior and Gumbel
+        fate, every node's statistics.  None if that search returned the sentinel (or none ran)."""
+        if self._last is None:
+            return None
+        eng, action = self._last
+        return eng.export_tree().game(0, first=action)
 
     # ------------------------------------------------------------------ batched entry
     @classmethod
@@ -307,6 +318,7 @@ class AlphaZeroMCTS(_GumbelEngineMCTS):
 
     def search(self, game):
         self._drain()
+        self._last = None
         A = config.ACTION_SPACE_SIZE
         obs = game.get_board_state(game.current_player, game.last_move)
         try:
@@ -341,6 +353,7 @@ class MuZeroMCTS(_GumbelEngineMCTS):
 
     def search(self, game):
         self._drain()
+        self._last = None
         A = config.ACTION_SPACE_SIZE
         obs = game.get_board_state(game.current_player, game.last_move)
         try:

@@ -244,6 +244,36 @@ int gmz_match_noise(gmz_engine *a, gmz_engine *b, const gmz_match *m, uint64_t s
 int gmz_match_step(gmz_engine *a, gmz_engine *b, const gmz_match *m, const int32_t *action_a, const int32_t *action_b,
                    gmz_stream stream);
 
+/* ---- search inspection: what a search holds, for a UI or a whole-tree comparison ---------------------- */
+/* A game's tree is CURRENT while its sim_count > 0: from gmz_root_expand / gmz_search_e0 until its root changes
+ * (gmz_set_roots*, gmz_game_step, gmz_selfplay_*, gmz_match_*, gmz_games_reset set sim_count to 0).  A search in
+ * progress (between gmz_expand_backup calls) has a current, partial tree; a game without a current tree exports
+ * 0 nodes.  Node 0 is the root, node k the k-th node created: one per AlphaZero simulation / MuZero evaluation.
+ * Every pointer is a device pointer and may be NULL (that output is skipped).  Everything written is a stored value. */
+typedef struct gmz_tree_out {
+    /* per game */
+    int32_t *num_nodes;    /* [G]     nodes of the current tree, 0 if none */
+    int32_t *sim_count;    /* [G]     the search's sim_count as stored (mcts.py:228) */
+    int32_t *root;         /* [G][3]  to_move, last_move (-1 = None), move_count of the searched root */
+    double *minmax;        /* [G][2]  MinMaxStats (minimum, maximum) (utils.py:6-25); (+inf, -inf) without a tree */
+    int32_t *halving;      /* [G][3]  current_phase, len(selected_children_actions), length of the initial top-k */
+    int32_t *topk_action;  /* [G][K]  Gumbel top-k in halving order: survivors first, then the eliminated, -1 past n_init */
+    double *topk_gumbel;   /* [G][K]  their Gumbel noise (0 past n_init) */
+    float *topk_logit;     /* [G][K]  their root logit (0 past n_init) */
+    int32_t *topk_round;   /* [G][K]  halving round that eliminated the entry, current_phase for a survivor, -1 past n_init */
+    float *root_logits;    /* [G][A]  the root's logit row (NaN without a tree) */
+    /* per node, k < num_nodes; entries past num_nodes are -1 (int) / 0 (float) */
+    int32_t *parent;       /* [G][S]  parent node, -1 for the root */
+    int32_t *action;       /* [G][S]  action from the parent, -1 for the root */
+    int32_t *depth;        /* [G][S]  edges from the root */
+    int32_t *visits;       /* [G][S]  visit_count */
+    double *value_sum;     /* [G][S]  value_sum as stored (float32 accumulation: an exact float32 value) */
+    double *reward;        /* [G][S]  reward (0 in AlphaZero mode) */
+    float *prior_logit;    /* [G][S]  the parent's logit at `action`, NaN for the root */
+} gmz_tree_out;
+/* Read-only: writes nothing into the engine's workspace.  One warp per game, on `stream`. */
+int gmz_tree_export(gmz_engine *e, const gmz_tree_out *out, gmz_stream stream);
+
 /* ---- packed move records: the device-side trajectory hand-off (workers.py:172-230, 399-433) ---- */
 /* One fixed-stride record per move of a finished game: everything the reference's self-play loop emits for
  * that move.  Layout (stride = gmz_move_record_bytes(board_size), a multiple of 16):
