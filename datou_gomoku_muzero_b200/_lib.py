@@ -26,13 +26,18 @@ class GmzTraj(C.Structure):
     _fields_ = [("n_slots", C.c_int32), ("max_moves", C.c_int32), ("fin_cap", C.c_int32), ("reserved", C.c_int32),
                 ("policy", C.c_void_p), ("value", C.c_void_p), ("action", C.c_void_p), ("start_board", C.c_void_p),
                 ("start_info", C.c_void_p), ("free_slots", C.c_void_p), ("free_top", C.c_void_p),
-                ("fin_queue", C.c_void_p), ("fin_count", C.c_void_p)]
+                ("fin_queue", C.c_void_p), ("fin_count", C.c_void_p), ("start_opening", C.c_void_p)]
 
 
 class GmzMatch(C.Structure):
     _fields_ = [("n_openings", C.c_int32), ("reserved", C.c_int32), ("open_boards", C.c_void_p), ("open_players", C.c_void_p),
                 ("open_last", C.c_void_p), ("open_mc", C.c_void_p), ("cursor", C.c_void_p), ("slot_ticket", C.c_void_p),
                 ("slot_ply", C.c_void_p), ("results", C.c_void_p), ("moves", C.c_void_p), ("finished", C.c_void_p)]
+
+
+class GmzOpenings(C.Structure):
+    _fields_ = [("n_openings", C.c_int32), ("reserved", C.c_int32), ("boards", C.c_void_p), ("players", C.c_void_p),
+                ("last_moves", C.c_void_p), ("move_counts", C.c_void_p)]
 
 
 class GmzTreeOut(C.Structure):
@@ -70,6 +75,7 @@ SIGNATURES = {
     "gmz_selfplay_e0": (C.c_int, [_P, C.POINTER(GmzTraj), C.c_uint64, C.c_int, C.c_uint64, C.c_int64, C.c_int, _P]),
     "gmz_selfplay_unpark": (C.c_int, [_P, C.POINTER(GmzTraj), _P]),
     "gmz_selfplay_step": (C.c_int, [_P, C.POINTER(GmzTraj), _P, _P, _P, C.c_int, _P, _P]),
+    "gmz_set_openings": (C.c_int, [_P, C.POINTER(GmzOpenings), _P]),
     "gmz_play_counters": (C.c_int, [_P, _P, _P]),
     "gmz_select_counters": (C.c_int, [_P, _P, _P]),
     "gmz_hidden_gather": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P]),

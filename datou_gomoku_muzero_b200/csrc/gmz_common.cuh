@@ -52,7 +52,9 @@ struct __align__(128) GState {
     int traj_slot;            // trajectory slot this game records into
     int traj_len;             // moves recorded in the current game
     unsigned noise_ctr;       // searches done by this game (Gumbel noise counter)
-    char pad1[96];
+    unsigned deals;           // games dealt to this game index since the opening book was bound (gmz_set_openings)
+    int opening;              // book opening the current game was dealt, + 1; 0 = not dealt from a book
+    char pad1[88];
 };
 static_assert(sizeof(GState) == 1024, "GState must be 1 KiB");
 

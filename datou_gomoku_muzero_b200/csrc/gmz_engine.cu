@@ -79,12 +79,12 @@ k_set_roots_records(Params p, const unsigned char *ring, size_t stride, int64_t 
     root_load(p, g, lane, reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * p.A), h->to_move, h->last_move, h->move_count);
 }
 
-__global__ void __launch_bounds__(CTA_THREADS) k_games_reset(Params p, const uint8_t *mask)
+__global__ void __launch_bounds__(CTA_THREADS) k_games_reset(Params p, BookDev book, const uint8_t *mask)
 {
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
     if (g >= p.G) return;
     if (mask && !mask[g]) return;
-    game_reset(p, p.gs + g, lane);
+    game_deal(p, book, p.gs + g, g, lane);
 }
 
 __global__ void __launch_bounds__(CTA_THREADS)
@@ -312,7 +312,7 @@ __global__ void k_fill_gumbel(double *out, size_t n, u64 seed, u64 offset)
 // its own -- record (policy, value, action) in the game's trajectory slot, do_move, get_game_ended,
 // hand finished games to the host queue and restart them in a fresh slot (workers.py:172-189, 230).
 __global__ void __launch_bounds__(CTA_THREADS)
-k_selfplay_step(Params p, TrajDev t, int use_traj, int restart, const double *policy, const double *value,
+k_selfplay_step(Params p, TrajDev t, BookDev book, int use_traj, int restart, const double *policy, const double *value,
                 const int32_t *action, int32_t *out_winner)
 {
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
@@ -334,6 +334,7 @@ k_selfplay_step(Params p, TrajDev t, int use_traj, int restart, const double *po
             if (lane == 0) {
                 int32_t *si = t.start_info + (size_t)slot * 4;
                 si[0] = s->to_move; si[1] = s->move_count; si[2] = s->last_move; si[3] = g;
+                if (t.start_opening) t.start_opening[slot] = s->opening;
             }
         }
         if (tl < t.max_moves) {
@@ -362,13 +363,13 @@ k_selfplay_step(Params p, TrajDev t, int use_traj, int restart, const double *po
         }
         ok = __shfl_sync(GMZ_FULL, ok, 0); nslot = __shfl_sync(GMZ_FULL, nslot, 0);
         __syncwarp();
-        if (ok) { game_reset(p, s, lane); if (lane == 0 && use_traj) s->traj_slot = nslot; }
+        if (ok) { game_deal(p, book, s, g, lane); if (lane == 0 && use_traj) s->traj_slot = nslot; }
         else if (lane == 0) s->parked = use_traj ? 1 : 0;
     }
 }
 
 // parked games (finished, no free trajectory slot at the time): take a slot and restart
-__global__ void __launch_bounds__(CTA_THREADS) k_unpark(Params p, TrajDev t)
+__global__ void __launch_bounds__(CTA_THREADS) k_unpark(Params p, TrajDev t, BookDev book)
 {
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
     if (g >= p.G) return;
@@ -378,7 +379,7 @@ __global__ void __launch_bounds__(CTA_THREADS) k_unpark(Params p, TrajDev t)
     if (lane == 0) ok = traj_pop_slot(t, slot);
     ok = __shfl_sync(GMZ_FULL, ok, 0); slot = __shfl_sync(GMZ_FULL, slot, 0);
     if (!ok) return;
-    game_reset(p, s, lane);
+    game_deal(p, book, s, g, lane);
     if (lane == 0) s->traj_slot = slot;
 }
 // give every game its initial trajectory slot (slot g) and clear the play bookkeeping
@@ -556,7 +557,7 @@ extern "C" int gmz_set_roots_from_records(gmz_engine *e, const void *ring, int64
 extern "C" int gmz_games_reset(gmz_engine *e, const uint8_t *mask, gmz_stream stream)
 {
     LIVE(e, "gmz_games_reset");
-    k_games_reset<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, mask);
+    k_games_reset<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, e->book, mask);
     return check_launch("k_games_reset");
 }
 extern "C" int gmz_get_roots(gmz_engine *e, int8_t *boards, int8_t *players, int32_t *last_moves, int32_t *move_counts,
@@ -638,11 +639,17 @@ extern "C" int gmz_e0_eval_obs(const float *obs, int batch, int board_size, uint
         obs, batch, board_size, e0_spec((u64)seed, logit_div), logits, values);
     return check_launch("k_e0_eval_obs");
 }
+// Self-play takes the book variant once a book has ever been bound, so that games dealt from it keep their labels after
+// an unbind; a search-only launch deals nothing and always takes the default variant.
 static int launch_play(gmz_engine *e, const PlayArgs &a, cudaStream_t st)
 {
     const bool mz = e->p.mode == GMZ_MODE_MUZERO, f = e->p.f32acc != 0;
-    if (mz) return f ? gmz_launch_play_mz1_f1(e, a, st) : gmz_launch_play_mz1_f0(e, a, st);
-    return f ? gmz_launch_play_mz0_f1(e, a, st) : gmz_launch_play_mz0_f0(e, a, st);
+    if (a.do_step && e->book_ever) {
+        if (mz) return f ? gmz_launch_play_mz1_f1_b1(e, a, st) : gmz_launch_play_mz1_f0_b1(e, a, st);
+        return f ? gmz_launch_play_mz0_f1_b1(e, a, st) : gmz_launch_play_mz0_f0_b1(e, a, st);
+    }
+    if (mz) return f ? gmz_launch_play_mz1_f1_b0(e, a, st) : gmz_launch_play_mz1_f0_b0(e, a, st);
+    return f ? gmz_launch_play_mz0_f1_b0(e, a, st) : gmz_launch_play_mz0_f0_b0(e, a, st);
 }
 static TrajDev traj_dev(const gmz_traj *t)
 {
@@ -652,6 +659,7 @@ static TrajDev traj_dev(const gmz_traj *t)
     d.policy = t->policy; d.value = t->value; d.action = t->action;
     d.start_board = (u64 *)t->start_board; d.start_info = t->start_info;
     d.free_slots = t->free_slots; d.free_top = t->free_top; d.fin_queue = t->fin_queue; d.fin_count = t->fin_count;
+    d.start_opening = t->start_opening;
     return d;
 }
 static int check_traj(const gmz_engine *e, const gmz_traj *t)
@@ -695,7 +703,7 @@ extern "C" int gmz_selfplay_e0(gmz_engine *e, const gmz_traj *traj, uint64_t eva
     PlayArgs a; memset(&a, 0, sizeof(a));
     a.e0 = e0_spec((u64)eval_seed, logit_div); a.noise_seed = noise_seed;
     a.total_tickets = total_moves; a.do_step = 1; a.restart = restart ? 1 : 0; a.use_traj = traj ? 1 : 0;
-    a.traj = traj_dev(traj);
+    a.traj = traj_dev(traj); a.book = e->book;
     return launch_play(e, a, (cudaStream_t)stream);
 }
 extern "C" int gmz_selfplay_step(gmz_engine *e, const gmz_traj *traj, const double *policy, const double *value,
@@ -704,7 +712,7 @@ extern "C" int gmz_selfplay_step(gmz_engine *e, const gmz_traj *traj, const doub
     LIVE(e, "gmz_selfplay_step");
     if (!action) return fail("gmz_selfplay_step: null argument");
     if (traj && (check_traj(e, traj) || !policy || !value)) return traj && policy && value ? 1 : fail("gmz_selfplay_step: policy/value required with a trajectory store");
-    k_selfplay_step<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, traj_dev(traj), traj ? 1 : 0, restart ? 1 : 0, policy, value, action, out_winner);
+    k_selfplay_step<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, traj_dev(traj), e->book, traj ? 1 : 0, restart ? 1 : 0, policy, value, action, out_winner);
     return check_launch("k_selfplay_step");
 }
 extern "C" int gmz_selfplay_unpark(gmz_engine *e, const gmz_traj *traj, gmz_stream stream)
@@ -712,8 +720,25 @@ extern "C" int gmz_selfplay_unpark(gmz_engine *e, const gmz_traj *traj, gmz_stre
     LIVE(e, "gmz_selfplay_unpark");
     if (!traj) return fail("gmz_selfplay_unpark: null argument");
     if (check_traj(e, traj)) return 1;
-    k_unpark<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, traj_dev(traj));
+    k_unpark<<<GRID(e), 0, (cudaStream_t)stream>>>(e->p, traj_dev(traj), e->book);
     return check_launch("k_unpark");
+}
+extern "C" int gmz_set_openings(gmz_engine *e, const gmz_openings *book, gmz_stream stream)
+{
+    if (book && book->n_openings < 1) return fail("gmz_set_openings: n_openings must be >= 1");
+    if (book && (!book->boards || !book->players || !book->last_moves || !book->move_counts))
+        return fail("gmz_set_openings: null array");
+    LIVE(e, "gmz_set_openings");
+    // every game's deal counter k back to 0: one 4-byte field per 1 KiB GState
+    cudaError_t err = cudaMemset2DAsync(&e->p.gs->deals, sizeof(GState), 0, sizeof(unsigned), e->p.G, (cudaStream_t)stream);
+    if (err != cudaSuccess) return fail("gmz_set_openings: %s", cudaGetErrorString(err));
+    memset(&e->book, 0, sizeof(e->book));
+    if (book) {
+        e->book.n = book->n_openings; e->book.boards = book->boards; e->book.players = book->players;
+        e->book.last_moves = book->last_moves; e->book.move_counts = book->move_counts;
+        e->book_ever = 1;
+    }
+    return 0;
 }
 extern "C" int gmz_play_counters(gmz_engine *e, uint64_t *out2, gmz_stream stream)
 {

@@ -32,6 +32,38 @@ __device__ __forceinline__ void root_load(const Params &p, int g, int lane, cons
         s->move_count = move_count;
         s->active = nvalid > 0;
         s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
-        s->winner = GMZ_WINNER_NONE;
+        s->winner = GMZ_WINNER_NONE; s->opening = 0;
     }
+}
+
+// GomokuGame.reset() on a GState (game.py:8-11).
+__device__ __forceinline__ void game_reset(const Params &p, GState *s, int lane)
+{
+    if (lane < GMZ_WORDS) {
+        u64 v = 0;
+        const int lo = 64 * lane;
+        if (lo < p.A) v = (p.A - lo >= 64) ? ~0ull : ((1ull << (p.A - lo)) - 1ull);
+        s->p1[lane] = 0; s->m1[lane] = 0; s->valid[lane] = v;
+    }
+    if (lane == 0) {
+        s->to_move = 1; s->last_move = -1; s->move_count = 0; s->active = 1;
+        s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
+        s->winner = GMZ_WINNER_NONE; s->traj_len = 0; s->parked = 0;
+    }
+}
+
+// A new self-play game for game g: its k-th deal since the book was bound (k = s->deals) takes opening (k*G + g) mod O,
+// so the games of an index depend on g and k only, not on which warp or launch deals them.  Without a book: the empty
+// board, labelled "none".  Every lane takes part (root_load ballots).
+__device__ __forceinline__ void game_deal(const Params &p, const BookDev &b, GState *s, int g, int lane)
+{
+    const unsigned k = s->deals;
+    int label = 0;
+    if (b.n > 0) {
+        const int o = (int)(((u64)k * (u64)p.G + (u64)g) % (u64)b.n);
+        root_load(p, g, lane, b.boards + (size_t)o * p.A, b.players[o], b.last_moves[o], b.move_counts[o]);
+        label = o + 1;
+    } else game_reset(p, s, lane);
+    __syncwarp();
+    if (lane == 0) { s->traj_len = 0; s->parked = 0; s->deals = k + 1; s->opening = label; }
 }

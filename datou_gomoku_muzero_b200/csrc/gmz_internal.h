@@ -6,6 +6,15 @@
 #include "../../include/gmz.h"
 #include "gmz_common.cuh"
 
+// The opening book self-play deals from (gmz_openings in include/gmz.h); n == 0: no book, deals are empty boards.
+struct BookDev {
+    int n, pad;
+    const int8_t *boards;      // [n][A]
+    const int8_t *players;     // [n]
+    const int32_t *last_moves; // [n]
+    const int32_t *move_counts;// [n]
+};
+
 struct gmz_engine {
     unsigned magic;          // GMZ_ENGINE_MAGIC while alive (gmz_destroy is idempotent per handle value)
     gmz_config cfg;
@@ -14,6 +23,8 @@ struct gmz_engine {
     int device;              // CUDA device the engine was created on
     size_t bytes;
     void *workspace;
+    BookDev book;            // the bound opening book (n == 0: none)
+    int book_ever;           // a book has been bound at some point: self-play launches the play kernel's book variant
 };
 #define GMZ_ENGINE_MAGIC 0x474d5a32u
 
@@ -22,9 +33,14 @@ int gmz_fail(const char *fmt, const char *a = "");
 int gmz_check_launch(const char *what);
 extern "C" void gmz_set_error_(const char *msg);
 
-// ticketed persistent play kernel, one translation unit per (MuZero mode, float32 accumulation) pair
+// ticketed persistent play kernel, one translation unit per (MuZero mode, float32 accumulation, book variant): _b1 deals
+// from a.book and labels each recorded game with its opening
 struct PlayArgs;
-int gmz_launch_play_mz0_f0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz0_f1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz1_f0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz1_f1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz0_f0_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz0_f1_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz1_f0_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz1_f1_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz0_f0_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz0_f1_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz1_f0_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz1_f1_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);

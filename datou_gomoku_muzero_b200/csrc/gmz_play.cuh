@@ -9,6 +9,7 @@
 // game owns lives in global memory (GState + its node pool), so any warp on any SM can continue it.
 #pragma once
 #include "gmz_tree.cuh"
+#include "gmz_engine.cuh"
 
 // CPython set iteration order over the valid actions, to break ties of the final
 // max(visit_counts, key=visit_counts.get) the way the reference does (mcts.py:274-275).
@@ -151,22 +152,6 @@ __device__ __forceinline__ int game_do_move(const Params &p, GState *s, int a, i
     return wv;
 }
 
-// GomokuGame.reset() on a GState (game.py:8-11).
-__device__ __forceinline__ void game_reset(const Params &p, GState *s, int lane)
-{
-    if (lane < GMZ_WORDS) {
-        u64 v = 0;
-        const int lo = 64 * lane;
-        if (lo < p.A) v = (p.A - lo >= 64) ? ~0ull : ((1ull << (p.A - lo)) - 1ull);
-        s->p1[lane] = 0; s->m1[lane] = 0; s->valid[lane] = v;
-    }
-    if (lane == 0) {
-        s->to_move = 1; s->last_move = -1; s->move_count = 0; s->active = 1;
-        s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
-        s->winner = GMZ_WINNER_NONE; s->traj_len = 0; s->parked = 0;
-    }
-}
-
 // Gumbel(0,1) noise from a counter-based splitmix64 stream: -log(-log(u)), u in (0,1) with 53 bits.
 // (z >> 11) + 0.5 rounds to even once z >> 11 >= 2^52, so z >> 11 = 2^53 - 1 would give u = 1 and +inf noise:
 // that draw is clamped to 1 - 2^-53, a value no other draw produces.
@@ -189,6 +174,7 @@ struct TrajDev {
     int32_t *free_top;   // number of ids on the stack
     int32_t *fin_queue;  // [fin_cap][4] = slot, game, length, winner
     int32_t *fin_count;
+    int32_t *start_opening;   // [n_slots]  book opening + 1 of the game recorded in a slot, 0 = none (may be null)
 };
 
 struct PlayArgs {
@@ -202,6 +188,7 @@ struct PlayArgs {
     double *out_policy; double *out_value; int32_t *out_action; int32_t *out_visits;   // search-only outputs
     int32_t *trace_a, *trace_d;   // [G][S] leaf action / depth per evaluation (search-only, optional)
     TrajDev traj;
+    BookDev book;         // self-play deals (book variant of k_play_e0 only)
 };
 
 __device__ __forceinline__ bool traj_pop_slot(const TrajDev &t, int &slot)
@@ -253,9 +240,18 @@ __device__ __noinline__ u64 play_root(const Params &p, const PlayArgs &a, WG &w,
     return h;
 }
 
+// The book variant's deal (game_deal), out of line like play_root: a restart is rare next to the simulations, and its
+// code stays out of the simulation loop's instruction stream and registers.
+static __device__ __noinline__ void play_deal(const Params &p, const BookDev &b, GState *s, int g, int lane)
+{
+    game_deal(p, b, s, g, lane);
+}
+
 // One search (mcts.py:197-280) -- and in self-play mode one whole move (workers.py:168-189) --
-// per ticket, one game per warp, E0 inlined.
-template <int NC, bool MZ, bool F32>
+// per ticket, one game per warp, E0 inlined.  BOOK: self-play deals through play_deal from the bound opening book and
+// records each game's opening label; the launcher takes it once a book has ever been bound on the engine, and the
+// default variant (BOOK = false) is the kernel as it was before books existed.
+template <int NC, bool MZ, bool F32, bool BOOK>
 __global__ void __launch_bounds__(32 * GMZ_PLAY_WARPS, GMZ_PLAY_MIN_CTAS)
 k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
 {
@@ -308,7 +304,8 @@ k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
         int2 *path = p.path + (size_t)g * (p.S + 2);    // descent path past depth 31 (rare)
 
         if (a.do_step && s->winner != GMZ_WINNER_NONE) {   // finished earlier, could not restart then
-            game_reset(p, s, lane);
+            if constexpr (BOOK) play_deal(p, a.book, s, g, lane);
+            else game_reset(p, s, lane);
             __syncwarp();
         }
         WG &w = s_wg[wi];
@@ -379,6 +376,7 @@ k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
                     if (lane == 0) {
                         int32_t *si = a.traj.start_info + (size_t)slot * 4;
                         si[0] = w.to_move; si[1] = s->move_count; si[2] = w.last_move; si[3] = g;
+                        if constexpr (BOOK) { if (a.traj.start_opening) a.traj.start_opening[slot] = s->opening; }
                     }
                 }
                 if (tl < a.traj.max_moves) pol = a.traj.policy + ((size_t)slot * a.traj.max_moves + tl) * (size_t)p.A;
@@ -421,7 +419,8 @@ k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
                 nslot = __shfl_sync(GMZ_FULL, nslot, 0);
                 __syncwarp();
                 if (ok) {
-                    game_reset(p, s, lane);
+                    if constexpr (BOOK) play_deal(p, a.book, s, g, lane);
+                    else game_reset(p, s, lane);
                     if (lane == 0 && a.use_traj) s->traj_slot = nslot;
                 } else if (lane == 0) s->parked = a.use_traj ? 1 : 0;
             }

@@ -107,8 +107,8 @@ __device__ __forceinline__ void rec_write_position(unsigned char *rec, int A, u6
 // One CTA per finished game, warp w emits moves w, w + 4, ... (each warp replays the game on its own bitboards).
 __global__ void __launch_bounds__(128)
 k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, const double *value, const int32_t *action,
-            const u64 *start_board, const int32_t *start_info, const int32_t *fin, int n_games, const int64_t *move_offset,
-            const double *dpow, int n_steps, unsigned char *out)
+            const u64 *start_board, const int32_t *start_info, const int32_t *start_opening, const int32_t *fin, int n_games,
+            const int64_t *move_offset, const double *dpow, int n_steps, unsigned char *out)
 {
     const int gi = blockIdx.x, lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
     if (gi >= n_games) return;
@@ -139,7 +139,7 @@ k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, co
             h.reward = rec_final_reward(t, T, winner);
             h.value_target = b < T ? __fadd_rn((float)acc, __fmul_rn((float)vals[b], gn)) : (float)acc;
             h.search_value = vals[t];
-            h.game = game; h.slot = slot; h.pad0 = 0; h.pad1 = 0;
+            h.game = game; h.slot = slot; h.opening = start_opening ? start_opening[slot] : 0; h.pad1 = 0;
             *reinterpret_cast<RecHeader *>(rec) = h;
         }
     }
@@ -153,7 +153,7 @@ extern "C" int gmz_traj_pack(const gmz_traj *traj, int board_size, const int32_t
     if (board_size < 1 || board_size > GMZ_MAX_BOARD || n_steps < 0) return rc_fail("gmz_traj_pack: bad size");
     const int A = board_size * board_size;
     k_traj_pack<<<n_games, 128, 0, (cudaStream_t)stream>>>(board_size, A, rec_stride(A), traj->max_moves, traj->policy, traj->value,
-                                                           traj->action, (const u64 *)traj->start_board, traj->start_info, fin, n_games,
+                                                           traj->action, (const u64 *)traj->start_board, traj->start_info, traj->start_opening, fin, n_games,
                                                            move_offset, discount_pow, n_steps, (unsigned char *)out_records);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : rc_fail(cudaGetErrorString(e));

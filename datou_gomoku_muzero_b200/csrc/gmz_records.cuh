@@ -11,7 +11,7 @@ struct RecHeader {            // 64 bytes, see include/gmz.h gmz_move_record
     int32_t action, to_move, last_move, move_count;
     float reward, value_target;
     double search_value;
-    int32_t game, slot, pad0, pad1;
+    int32_t game, slot, opening, pad1;   // opening: book opening + 1, 0 = none
 };
 static_assert(sizeof(RecHeader) == 64, "record header must be 64 bytes");
 

@@ -16,7 +16,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import GMZ_ACCUM_F32, GMZ_ACCUM_F64, GMZ_BF16, GMZ_F32, GMZ_F64, GMZ_MODE_ALPHAZERO, GMZ_MODE_MUZERO, GmzConfig, check
+from ._lib import (GMZ_ACCUM_F32, GMZ_ACCUM_F64, GMZ_BF16, GMZ_F32, GMZ_F64, GMZ_MODE_ALPHAZERO, GMZ_MODE_MUZERO, GmzConfig,
+                   GmzOpenings, check)
 
 
 def _ptr(t):
@@ -75,6 +76,7 @@ class SearchEngine:
         self.leaf_action = torch.zeros(G, dtype=torch.int32, device=dev)
         self.leaf_depth = torch.zeros(G, dtype=torch.int32, device=dev)
         self.launches = 0   # kernels of ours launched through this engine
+        self._book = None   # device copies of the bound opening book
 
     # ------------------------------------------------------------------ plumbing
     def _stream(self):
@@ -116,6 +118,22 @@ class SearchEngine:
         m = None if mask is None else self._dev(mask, torch.uint8).reshape(self.G)
         check(self.lib.gmz_games_reset(self.handle, _ptr(m), self._stream()), "gmz_games_reset")
         self.launches += 1
+
+    def set_openings(self, openings):
+        """Bind an opening book (arena.Openings, or any 4-tuple of boards [O,A] or [O,N,N], players, last moves, move
+        counts) that every later self-play deal of this engine takes its position from: the k-th deal of game g since
+        this call takes opening (k*G + g) mod O.  None unbinds (deals are empty boards again).  Games in flight continue
+        unchanged.  The book is checked first (arena.check_openings, ValueError) and nothing is launched if it fails."""
+        if openings is None:
+            check(self.lib.gmz_set_openings(self.handle, None, self._stream()), "gmz_set_openings")
+            self._book = None
+            return
+        from .arena import check_openings
+        op = check_openings(openings, self.N, self.cfg.n_in_row)
+        book = [torch.from_numpy(x).to(self.device) for x in op]
+        c = GmzOpenings(op.boards.shape[0], 0, *(t.data_ptr() for t in book))
+        check(self.lib.gmz_set_openings(self.handle, C.byref(c), self._stream()), "gmz_set_openings")
+        self._book = book
 
     def get_roots(self):
         b = torch.empty((self.G, self.N, self.N), dtype=torch.int8, device=self.device)

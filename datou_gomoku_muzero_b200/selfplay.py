@@ -18,9 +18,13 @@ class SelfPlayEngine:
     `f(obs f32 [G,3,N,N]) -> (logits f32 [G,A], values f32/f64 [G])` run on the device (eager stepwise path); or --
     for an engine in MuZero mode -- a pair `(initial_fn, recurrent_fn)` / a `muzero.MuZeroDeviceSearch`
     (learned dynamics in the tree, hidden states in the device pool; MuZeroMCTS.search, mcts.py:288-362).  The evaluator
-    is resolved by mcts.resolve_searchers, as for re-analysis, into `self.searcher`; seed / logit_div configure "e0"."""
+    is resolved by mcts.resolve_searchers, as for re-analysis, into `self.searcher`; seed / logit_div configure "e0".
 
-    def __init__(self, engine: SearchEngine, evaluator="e0", seed=0, logit_div=16, noise_seed=0):
+    openings: an opening book (arena.Openings) bound to the engine before the games are first dealt
+    (SearchEngine.set_openings): game g starts on opening g mod O, and every later restart of game index g takes the
+    book's next opening for that index.  None: empty boards."""
+
+    def __init__(self, engine: SearchEngine, evaluator="e0", seed=0, logit_div=16, noise_seed=0, openings=None):
         self.e = engine
         self.searcher = resolve_searchers([engine], evaluator, seed, logit_div)[0]
         self.noise_seed = int(noise_seed)
@@ -30,6 +34,8 @@ class SelfPlayEngine:
         self.moves_played = 0
         self.games_finished = 0
         self.done_mask = torch.zeros(G, dtype=torch.uint8, device=engine.device)
+        if openings is not None:
+            engine.set_openings(openings)
         engine.reset_games()
 
     def search(self, gumbel=None):

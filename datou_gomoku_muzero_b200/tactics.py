@@ -122,19 +122,26 @@ class SelfPlayStats:
     SelfPlayStatus (workers.py:191-203, 235): games, moves, results, missed fives and missed wins.  Pass
     `add` to play() alongside the replay sink, `sink=lambda pg: (stats.add(pg), buf.add_packed(pg))`.
     Game / move / result counts come from the host-side game table; the missed counts stay in device counters, so
-    `add` never waits for the GPU.  `summary()` reads them back once."""
+    `add` never waits for the GPU.  `summary()` reads them back once.
 
-    def __init__(self, n_in_row=None, device=None):
+    n_openings = O > 0 also keeps, per opening of a self-play book (SearchEngine.set_openings), how often the side to
+    move at the opening won, drew and lost, from each game's first record on the device; `by_opening()` reads them.
+    Games without a label in [0, O) count in the totals only."""
+
+    def __init__(self, n_in_row=None, device=None, n_openings=0):
         if not torch.cuda.is_available():
             raise _lib.GmzError("SelfPlayStats needs a CUDA device (there is no CPU fallback)")
         self.n_in_row = n_in_row
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         self._missed = torch.zeros(2, dtype=torch.int64, device=self.device)      # missed fives, missed wins
+        self.n_openings = int(n_openings)
+        self._by_opening = torch.zeros((self.n_openings, 3), dtype=torch.int64, device=self.device)
         self.reset()
 
     def reset(self):
         self.games = self.moves = self.wins_black = self.wins_white = self.draws = 0
         self._missed.zero_()
+        self._by_opening.zero_()
 
     def add(self, packed):
         """Count the games of a trajectory.PackedGames whose records are on this device.  Launches one kernel and a
@@ -153,6 +160,19 @@ class SelfPlayStats:
             return
         fives, missed = _missed(record_flags(packed.records[:M], packed.N, self.n_in_row))
         self._missed += torch.stack([fives.sum(), missed.sum()])
+        if self.n_openings:
+            # first record of each game: winner (bytes 12..15), to_move (20..23), opening label + 1 (56..59)
+            first = torch.as_tensor(np.asarray(packed.offsets[:-1], np.int64), device=self.device)
+            hdr = packed.records[first, :64].contiguous().view(torch.int32)
+            winner, to_move, label = hdr[:, 3], hdr[:, 5], hdr[:, 14].to(torch.int64) - 1
+            outcome = torch.where(winner == 0, 1, torch.where(winner == to_move, 0, 2)).to(torch.int64)
+            ok = (label >= 0) & (label < self.n_openings)
+            self._by_opening.view(-1).index_add_(0, torch.where(ok, label * 3 + outcome, 0), ok.to(torch.int64))
+
+    def by_opening(self):
+        """int64 [n_openings, 3]: per opening, the games the side to move at the opening won, drew and lost (one device
+        -> host copy)."""
+        return self._by_opening.cpu().numpy()
 
     def summary(self):
         """dict of the counts plus avg_game_length and per-game rates (one device -> host copy)."""

@@ -23,9 +23,9 @@ def record_dtype(board_size):
     A = N * N
     stride = (64 + 21 * A + 15) // 16 * 16
     names = ["game_seq", "t", "length", "winner", "action", "to_move", "last_move", "move_count", "reward", "value_target",
-             "search_value", "game", "slot", "policy", "obs", "board"]
-    formats = ["<i4"] * 8 + ["<f4", "<f4", "<f8", "<i4", "<i4", ("<f8", (A,)), ("<f4", (3, N, N)), ("i1", (N, N))]
-    offsets = [0, 4, 8, 12, 16, 20, 24, 28, 32, 36, 40, 48, 52, 64, 64 + 8 * A, 64 + 20 * A]
+             "search_value", "game", "slot", "opening", "policy", "obs", "board"]
+    formats = ["<i4"] * 8 + ["<f4", "<f4", "<f8", "<i4", "<i4", "<i4", ("<f8", (A,)), ("<f4", (3, N, N)), ("i1", (N, N))]
+    offsets = [0, 4, 8, 12, 16, 20, 24, 28, 32, 36, 40, 48, 52, 56, 64, 64 + 8 * A, 64 + 20 * A]
     return np.dtype({"names": names, "formats": formats, "offsets": offsets, "itemsize": stride})
 
 
@@ -55,6 +55,17 @@ class PackedGames:
 
     def game(self, i):
         return self.host()[self.offsets[i]:self.offsets[i + 1]]
+
+    def openings(self):
+        """int32 [n_games]: the opening book index each game was dealt (SearchEngine.set_openings), -1 for none.  Reads
+        only the first record header of each game."""
+        first = self.offsets[:-1]
+        if self._host is None and torch.is_tensor(self.records) and self.records.is_cuda:
+            idx = torch.as_tensor(first, device=self.records.device)
+            lab = self.records[idx, 56:60].contiguous().view(torch.int32).reshape(-1).cpu().numpy()
+        else:
+            lab = self.host()["opening"][first]
+        return lab.astype(np.int32) - 1
 
     def game_record(self, i):
         """GameRecord of game i (data_structures.py:9-16): lists of per-move array views / Python scalars."""
@@ -103,9 +114,11 @@ class TrajectoryStore:
         self.free_top = torch.zeros(1, dtype=torch.int32, device=dev)
         self.fin_queue = torch.zeros((n, 4), dtype=torch.int32, device=dev)
         self.fin_count = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.start_opening = torch.zeros(n, dtype=torch.int32, device=dev)      # book label + 1 per slot, 0 = none
         p = lambda t: t.data_ptr()
         self.c = GmzTraj(n, T, n, 0, p(self.policy), p(self.value), p(self.action), p(self.start_board),
-                         p(self.start_info), p(self.free_slots), p(self.free_top), p(self.fin_queue), p(self.fin_count))
+                         p(self.start_info), p(self.free_slots), p(self.free_top), p(self.fin_queue), p(self.fin_count),
+                         p(self.start_opening))
         check(e.lib.gmz_traj_init(e.handle, C.byref(self.c), e._stream()), "gmz_traj_init")
         e.launches += 1
 
@@ -114,7 +127,7 @@ class TrajectoryStore:
         stack and (with `unpark`) parked games restart -- pass unpark=False after play(restart=False) to leave
         finished games finished.  A game that recorded more moves than the store's `max_moves` (only possible with a
         user-supplied max_moves below the remaining plies) comes back with `length` clamped to what was recorded and
-        `truncated` = True."""
+        `truncated` = True.  `opening` is the index of the book opening the game was dealt, -1 for none."""
         e = self.e
         n = int(self.fin_count.item())
         if n == 0:
@@ -129,6 +142,7 @@ class TrajectoryStore:
         pol = self.policy[slots, :Tmax].cpu().numpy() if copy_policies else None
         sb = self.start_board[slots].cpu().numpy().view(np.uint64)
         si = self.start_info[slots].cpu().numpy()
+        so = self.start_opening[slots].cpu().numpy()
         out = []
         for i in range(n):
             T = int(q[i, 2])
@@ -138,7 +152,7 @@ class TrajectoryStore:
                             values=val[i, :T].copy(), policies=None if pol is None else pol[i, :T].copy(),
                             start_board=board.reshape(e.N, e.N), start_player=int(si[i, 0]),
                             start_move_count=int(si[i, 1]), start_last_move=int(si[i, 2]),
-                            truncated=bool(full_len[i] > self.max_moves)))
+                            truncated=bool(full_len[i] > self.max_moves), opening=int(so[i]) - 1))
         self.fin_count.zero_()
         self.release(slots, unpark=unpark)
         return out

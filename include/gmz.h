@@ -85,7 +85,8 @@ int gmz_destroy(gmz_engine *e);
  * (search() sentinel, mcts.py:214-215). */
 int gmz_set_roots(gmz_engine *e, const int8_t *boards, const int8_t *players, const int32_t *last_moves,
                   const int32_t *move_counts, gmz_stream stream);
-/* GomokuGame.reset() (game.py:8-11) for every game with mask[g] != 0 (NULL = all). */
+/* GomokuGame.reset() (game.py:8-11) for every game with mask[g] != 0 (NULL = all); with an opening book bound, each of
+ * those games is dealt its next opening instead (gmz_set_openings). */
 int gmz_games_reset(gmz_engine *e, const uint8_t *mask, gmz_stream stream);
 /* GomokuGame.get_board_state at the roots (game.py:12-17): obs [G,3,N,N] float32 (GMZ_F32) or the same
  * planes as bfloat16 in NHWC order (GMZ_BF16). */
@@ -163,6 +164,8 @@ typedef struct gmz_traj {
     int32_t *free_top;     /* [1]                      ids on the stack */
     int32_t *fin_queue;    /* [fin_cap][4]             slot, game, length, winner */
     int32_t *fin_count;    /* [1] */
+    int32_t *start_opening; /* [n_slots]               opening book label of the game in the slot: index + 1, 0 = not
+                            *                          dealt from a book (gmz_set_openings).  May be NULL: label 0 */
 } gmz_traj;
 /* Slot g -> game g, remaining slots on the free stack, queues cleared. */
 int gmz_traj_init(gmz_engine *e, const gmz_traj *traj, gmz_stream stream);
@@ -174,6 +177,29 @@ int gmz_traj_init(gmz_engine *e, const gmz_traj *traj, gmz_stream stream);
 int gmz_selfplay_e0(gmz_engine *e, const gmz_traj *traj, uint64_t eval_seed, int logit_div, uint64_t noise_seed,
                     int64_t total_moves, int restart, gmz_stream stream);
 int gmz_selfplay_unpark(gmz_engine *e, const gmz_traj *traj, gmz_stream stream);
+/* Self-play from an opening book.  A DEAL is every place a finished or reset self-play game gets a new position: the
+ * restarts of gmz_selfplay_e0, gmz_selfplay_step and gmz_selfplay_unpark, and gmz_games_reset.  Without a book a deal is
+ * GomokuGame.reset() (empty board, +1 to move).  With a book of O openings bound, the k-th deal of game g since the bind
+ * takes opening (k*G + g) mod O -- a function of g and k only, so the games of an index do not depend on how moves are
+ * split into launches, on the persistent or stepwise path, or on the warp schedule.  The Gumbel noise is unchanged
+ * (the game's own search counter).  Each packed record of a game dealt from the book carries its label (index + 1) in
+ * gmz_move_record.opening, also when the game is played on after an unbind.  gmz_set_roots*, gmz_search_e0 and the
+ * match entry points never use the book.  Arrays as gmz_set_roots takes them: boards int8 [O][A] in {-1, 0, +1},
+ * players int8 [O] (+-1), last_moves int32 [O] (-1 = None), move_counts int32 [O]; every opening must hold an empty
+ * cell and not have ended (the library does not read them on the host; datou_gomoku_muzero_b200.arena.check_openings
+ * does). */
+typedef struct gmz_openings {
+    int32_t n_openings;          /* O >= 1 */
+    int32_t reserved;
+    const int8_t *boards;        /* device pointers */
+    const int8_t *players;
+    const int32_t *last_moves;
+    const int32_t *move_counts;
+} gmz_openings;
+/* Bind (book != NULL, n_openings >= 1) or unbind (NULL) the book that deals of engine e draw from; resets every game's
+ * deal counter k to 0 on `stream`.  Applies to deals enqueued after it; games in flight continue unchanged.  The arrays
+ * are caller-owned and must stay valid while bound and while launches using them run. */
+int gmz_set_openings(gmz_engine *e, const gmz_openings *book, gmz_stream stream);
 /* The same move bookkeeping for the stepwise path (any evaluator): after gmz_finalize, record
  * (policy f64 [G,A], value f64 [G], action int32 [G]) in each game's trajectory slot, do_move,
  * get_game_ended, queue finished games and restart them (workers.py:172-189, 230).  traj may be
@@ -297,7 +323,8 @@ typedef struct gmz_move_record {
     double search_value;  /* root value of the search for this move */
     int32_t game;         /* engine game index that played it */
     int32_t slot;         /* trajectory slot it was recorded in */
-    int32_t reserved[2];
+    int32_t opening;      /* opening book label: index + 1 of the opening the game was dealt, 0 = none (gmz_set_openings) */
+    int32_t reserved;
 } gmz_move_record;
 size_t gmz_move_record_bytes(int board_size);
 /* Expand n_games finished games into records.  fin int32 [n_games][4] = (slot, game, length, winner) rows of the
