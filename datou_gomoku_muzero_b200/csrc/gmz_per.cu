@@ -14,6 +14,8 @@
 #include "gmz_common.cuh"
 
 #define PER_MAX_CHUNK 2048
+// k_per_update's 32 warps own tree depths 0..31, so the deepest leaf may sit at depth 32: 2*capacity - 2 < 2^33 - 1.
+#define PER_MAX_CAPACITY (1ll << 32)
 
 extern "C" void gmz_set_error_(const char *msg);   // defined in gmz_engine.cu (feeds gmz_last_error)
 
@@ -21,16 +23,18 @@ __device__ __forceinline__ int node_depth(long long k) { return 63 - __clzll((un
 
 // One CTA of 1024 threads (32 warps).  Stage 1 (warp 0): leaf writes and `change` per update,
 // in batch order (a repeated leaf sees the previous write).  Stage 2 (warp d): depth-d ancestors.
+// An index outside [0, len) is an inactive lane in both stages: it writes nothing.
 __global__ void __launch_bounds__(1024)
-k_per_update(double *tree, const long long *tree_idx, const double *prio, int n)
+k_per_update(double *tree, long long len, const long long *tree_idx, const double *prio, int n)
 {
     extern __shared__ double s_change[];           // [n]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (warp == 0) {
         for (int base = 0; base < n; base += 32) {
             const int i = base + lane;
-            const bool act = i < n;
-            const long long key = act ? tree_idx[i] : -1 - lane;
+            const long long k = i < n ? tree_idx[i] : -1;
+            const bool act = k >= 0 && k < len;
+            const long long key = act ? k : -1 - lane;
             const double p = act ? prio[i] : 0.0;
             const unsigned grp = __match_any_sync(GMZ_FULL, key);
             const int leader = __ffs(grp) - 1;
@@ -60,8 +64,8 @@ k_per_update(double *tree, const long long *tree_idx, const double *prio, int n)
         const int i = base + lane;
         long long key = -1 - lane;
         double ch = 0.0;
-        if (i < n) {
-            const long long leaf = tree_idx[i];
+        const long long leaf = i < n ? tree_idx[i] : -1;
+        if (leaf >= 0 && leaf < len) {
             const int D = node_depth(leaf);
             if (D > d) { key = ((leaf + 1) >> (D - d)) - 1; ch = s_change[i]; }
         }
@@ -136,7 +140,7 @@ extern "C" int gmz_per_update(double *tree, int64_t capacity, const int64_t *tre
                               gmz_stream stream)
 {
     if (!tree || !tree_idx || !priorities) return per_fail("gmz_per_update: null argument");
-    if (capacity < 1) return per_fail("gmz_per_update: capacity out of range");
+    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return per_fail("gmz_per_update: capacity out of range (1 .. 2^32)");
     static bool attr_set = false;
     if (!attr_set) {
         cudaFuncSetAttribute(k_per_update, cudaFuncAttributeMaxDynamicSharedMemorySize, PER_MAX_CHUNK * (int)sizeof(double));
@@ -144,7 +148,8 @@ extern "C" int gmz_per_update(double *tree, int64_t capacity, const int64_t *tre
     }
     for (int off = 0; off < n; off += PER_MAX_CHUNK) {     // chunks run in stream order = batch order
         const int m = n - off < PER_MAX_CHUNK ? n - off : PER_MAX_CHUNK;
-        k_per_update<<<1, 1024, m * sizeof(double), (cudaStream_t)stream>>>(tree, (const long long *)tree_idx + off, priorities + off, m);
+        k_per_update<<<1, 1024, m * sizeof(double), (cudaStream_t)stream>>>(tree, 2 * capacity - 1, (const long long *)tree_idx + off,
+                                                                           priorities + off, m);
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return per_fail(cudaGetErrorString(e));
@@ -226,8 +231,9 @@ extern "C" int gmz_per_add(double *tree, int64_t capacity, int64_t write_ptr, co
                            int64_t *scratch_idx, gmz_stream stream)
 {
     if (!tree || !priorities || !scratch_idx) return per_fail("gmz_per_add: null argument");
+    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return per_fail("gmz_per_add: capacity out of range (1 .. 2^32)");
     if (n <= 0) return 0;
-    if (capacity < 1 || write_ptr < 0 || write_ptr >= capacity) return per_fail("gmz_per_add: bad capacity / write_ptr");
+    if (write_ptr < 0 || write_ptr >= capacity) return per_fail("gmz_per_add: write_ptr outside the ring");
     if (n >= 64 && (int64_t)n <= capacity && capacity >= 2) {     // bulk path: node-parallel, whole GPU
         double *change = reinterpret_cast<double *>(scratch_idx);  // the caller's int64 [n] scratch, reused as float64 [n]
         k_per_add_leaves<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(tree, capacity, write_ptr, priorities, n, change);
@@ -245,6 +251,7 @@ extern "C" int gmz_per_sample(const double *tree, int64_t capacity, int64_t coun
                               int64_t *out_tree_idx, double *out_priority, float *out_weights, gmz_stream stream)
 {
     if (!tree || !u01 || !out_tree_idx || !out_priority || !out_weights) return per_fail("gmz_per_sample: null argument");
+    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return per_fail("gmz_per_sample: capacity out of range (1 .. 2^32)");
     if (batch <= 0) return 0;
     k_per_sample<<<1, 1024, 0, (cudaStream_t)stream>>>(tree, capacity, count, u01, batch, beta,
                                                         (long long *)out_tree_idx, out_priority, out_weights);

@@ -49,7 +49,17 @@ class SumTree:
 
     # ---- device-tensor entry points (no host round trip)
     def update_many(self, tree_idx, priorities):
-        """Apply tree.update(idx_i, p_i) for i = 0..n-1 in order (replay_buffer.py:16-19)."""
+        """Apply tree.update(idx_i, p_i) for i = 0..n-1 in order (replay_buffer.py:16-19).
+
+        Indices in host memory (list, numpy, CPU tensor) are checked here: one outside the tree (0 .. 2*capacity-2)
+        raises IndexError and nothing is updated.  Indices on the device are not read back; the kernel skips any that
+        lies outside the tree."""
+        if not (torch.is_tensor(tree_idx) and tree_idx.is_cuda):
+            host = np.asarray(tree_idx, dtype=np.int64).reshape(-1)
+            bad = (host < 0) | (host >= 2 * self.capacity - 1)
+            if bad.any():
+                raise IndexError(f"tree index {int(host[bad][0])} outside the tree (0 .. {2 * self.capacity - 2})")
+            tree_idx = host
         idx, pr = self._dev(tree_idx, torch.int64), self._dev(priorities, torch.float64)
         check(self.lib.gmz_per_update(_ptr(self.tree), self.capacity, _ptr(idx), _ptr(pr), int(idx.numel()),
                                       self._stream()), "gmz_per_update")
@@ -146,8 +156,8 @@ class InMemoryReplayBuffer:
         priorities = np.abs(td_errors) + config.PER_EPSILON      # keeps td_errors' dtype (float32 from the loss)
         if len(priorities) == 0:
             return
-        self.max_priority = max(self.max_priority, priorities.max())
         self.sum_tree.update_many(np.asarray(tree_indices, dtype=np.int64), priorities.astype(np.float64))
+        self.max_priority = max(self.max_priority, priorities.max())      # after the index check: a refused call changes nothing
 
     def __len__(self):
         return self.sum_tree.count
@@ -443,8 +453,8 @@ class DeviceReplayBuffer:
         if td.numel() == 0:
             return
         pr = (td.abs() + np.float32(config.PER_EPSILON)).double()        # float32 arithmetic like the reference, then widened
-        self.max_priority = torch.maximum(self.max_priority, pr.max())
         self.sum_tree.update_many(tree_indices, pr)
+        self.max_priority = torch.maximum(self.max_priority, pr.max())
 
     def state_dict(self):
         """The buffer's state as a dict of CPU tensors, ints and strs, for torch.save next to the network (loads with

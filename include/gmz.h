@@ -393,9 +393,14 @@ int gmz_tactics_classify(const int8_t *boards, const int8_t *players, int batch,
                          int8_t *out_cls, gmz_stream stream);
 
 /* ---- prioritized replay: SumTree (replay_buffer.py:4-106) ------------------- */
-/* tree f64 [2*capacity-1] lives in caller memory.  Sequential reference
- * semantics are preserved bit for bit (each node receives its += in batch order). */
-/* update_priorities / add: tree_idx int64 [n], priorities f64 [n], applied in order. */
+/* tree f64 [2*capacity-1] lives in caller memory, 1 <= capacity <= 2^32 (all three calls refuse
+ * any other capacity before looking at n / batch).  Sequential reference semantics are preserved
+ * bit for bit (each node receives its += in batch order). */
+/* update_priorities / add: tree_idx int64 [n], priorities f64 [n], applied in order.  A tree_idx
+ * outside [0, 2*capacity-1) is skipped: it writes nothing, and the other updates apply as if it were
+ * absent.  Leaves are capacity-1 .. 2*capacity-2; an internal-node index is accepted, as the reference's
+ * SumTree.update accepts it (the node is overwritten and the change goes to its ancestors); the call is
+ * bit-exact with sequential updates as long as no index of it is an ancestor of another. */
 int gmz_per_update(double *tree, int64_t capacity, const int64_t *tree_idx, const double *priorities, int n,
                    gmz_stream stream);
 /* add(): n priorities written at ring positions write_ptr, write_ptr+1, ... (mod capacity), applied in
