@@ -28,7 +28,6 @@ int gmz_fail(const char *fmt, const char *a)
     snprintf(g_err, sizeof(g_err), fmt, a);
     return 1;
 }
-extern "C" void gmz_set_error_(const char *msg) { snprintf(g_err, sizeof(g_err), "%s", msg); }
 int gmz_check_launch(const char *what)
 {
     cudaError_t e = cudaGetLastError();
@@ -74,9 +73,9 @@ k_set_roots_records(Params p, const unsigned char *ring, size_t stride, int64_t 
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
     if (g >= p.G) return;
     if (g >= n) { root_load(p, g, lane, nullptr, 1, -1, 0); return; }
-    const unsigned char *rec = ring + (size_t)((first + g) % capacity) * stride;
-    const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
-    root_load(p, g, lane, reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * p.A), h->to_move, h->last_move, h->move_count);
+    const unsigned char *rec = rec_at(ring, stride, capacity, first, g);
+    const gmz_move_record *h = rec_header(rec);
+    root_load(p, g, lane, rec_board(rec, p.A), h->to_move, h->last_move, h->move_count);
 }
 
 __global__ void __launch_bounds__(CTA_THREADS) k_games_reset(Params p, BookDev book, const uint8_t *mask)

@@ -10,12 +10,9 @@
 // (chunks per row, games).  The action plane is the dynamics net's one-hot action embedding
 // (network.py:70-73: a 1x1 conv without bias of a one-hot plane == `embed` at the action's cell, zeros
 // elsewhere), written by the same pass so the concatenated input is never built by a separate kernel.
-#include <cuda_runtime.h>
 #include <stdint.h>
-#include "../../include/gmz.h"
 
-extern "C" void gmz_set_error_(const char *msg);   // defined in gmz_engine.cu (feeds gmz_last_error)
-static int hd_fail(const char *m) { gmz_set_error_(m); return 1; }
+#include "gmz_internal.h"
 
 namespace {
 
@@ -113,36 +110,34 @@ extern "C" int gmz_hidden_gather(const void *pool, const int32_t *slot, const in
                                  int sims_per_game, int nodes_per_game, int positions, int pos_bytes,
                                  const void *embed, int embed_bytes, void *x, gmz_stream stream)
 {
-    if (!pool || !slot || !x) return hd_fail("gmz_hidden_gather: null argument");
-    if (embed_bytes && (!embed || !action)) return hd_fail("gmz_hidden_gather: embed_bytes > 0 needs embed and action");
+    if (!pool || !slot || !x) return gmz_fail("gmz_hidden_gather: null argument");
+    if (embed_bytes && (!embed || !action)) return gmz_fail("gmz_hidden_gather: embed_bytes > 0 needs embed and action");
     if (num_games <= 0) return 0;
     if (sims_per_game < 1 || nodes_per_game < 1 || positions < 1 || pos_bytes < 4 || embed_bytes < 0)
-        return hd_fail("gmz_hidden_gather: sizes must be positive");
+        return gmz_fail("gmz_hidden_gather: sizes must be positive");
     const uintptr_t bits = (uintptr_t)pool | (uintptr_t)x | (uintptr_t)embed | (uintptr_t)pos_bytes | (uintptr_t)embed_bytes;
-    if (bits & 3) return hd_fail("gmz_hidden_gather: sizes and pointers must be multiples of 4 bytes");
+    if (bits & 3) return gmz_fail("gmz_hidden_gather: sizes and pointers must be multiples of 4 bytes");
     if ((long long)positions * (pos_bytes + embed_bytes) > (1ll << 30) || num_games > 65535)
-        return hd_fail("gmz_hidden_gather: row or batch too large");
+        return gmz_fail("gmz_hidden_gather: row or batch too large");
     cudaStream_t st = (cudaStream_t)stream;
     if (!(bits & 15)) launch_gather<uint4>(pool, slot, action, num_games, sims_per_game, nodes_per_game, positions, pos_bytes, embed, embed_bytes, x, st);
     else if (!(bits & 7)) launch_gather<uint2>(pool, slot, action, num_games, sims_per_game, nodes_per_game, positions, pos_bytes, embed, embed_bytes, x, st);
     else launch_gather<unsigned>(pool, slot, action, num_games, sims_per_game, nodes_per_game, positions, pos_bytes, embed, embed_bytes, x, st);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : hd_fail(cudaGetErrorString(e));
+    return gmz_check_launch("k_hidden_gather");
 }
 
 extern "C" int gmz_hidden_scatter(void *pool, const int32_t *slot, int num_games, int sims_per_game, int nodes_per_game,
                                   int row_bytes, const void *hidden, gmz_stream stream)
 {
-    if (!pool || !slot || !hidden) return hd_fail("gmz_hidden_scatter: null argument");
+    if (!pool || !slot || !hidden) return gmz_fail("gmz_hidden_scatter: null argument");
     if (num_games <= 0) return 0;
-    if (sims_per_game < 1 || nodes_per_game < 1 || row_bytes < 4) return hd_fail("gmz_hidden_scatter: sizes must be positive");
+    if (sims_per_game < 1 || nodes_per_game < 1 || row_bytes < 4) return gmz_fail("gmz_hidden_scatter: sizes must be positive");
     const uintptr_t bits = (uintptr_t)pool | (uintptr_t)hidden | (uintptr_t)row_bytes;
-    if (bits & 3) return hd_fail("gmz_hidden_scatter: row_bytes and pointers must be multiples of 4 bytes");
-    if (num_games > 65535) return hd_fail("gmz_hidden_scatter: batch too large");
+    if (bits & 3) return gmz_fail("gmz_hidden_scatter: row_bytes and pointers must be multiples of 4 bytes");
+    if (num_games > 65535) return gmz_fail("gmz_hidden_scatter: batch too large");
     cudaStream_t st = (cudaStream_t)stream;
     if (!(bits & 15)) launch_scatter<uint4>(pool, slot, num_games, sims_per_game, nodes_per_game, row_bytes, hidden, st);
     else if (!(bits & 7)) launch_scatter<uint2>(pool, slot, num_games, sims_per_game, nodes_per_game, row_bytes, hidden, st);
     else launch_scatter<unsigned>(pool, slot, num_games, sims_per_game, nodes_per_game, row_bytes, hidden, st);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : hd_fail(cudaGetErrorString(e));
+    return gmz_check_launch("k_hidden_scatter");
 }

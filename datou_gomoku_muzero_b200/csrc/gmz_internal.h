@@ -31,7 +31,6 @@ struct gmz_engine {
 // error text behind gmz_last_error() (thread-local, defined in gmz_engine.cu); both return 1
 int gmz_fail(const char *fmt, const char *a = "");
 int gmz_check_launch(const char *what);
-extern "C" void gmz_set_error_(const char *msg);
 
 // ticketed persistent play kernel, one translation unit per (MuZero mode, float32 accumulation, book variant): _b1 deals
 // from a.book and labels each recorded game with its opening

@@ -8,16 +8,12 @@
 // the group leader accumulate the group's changes in lane (= batch) order.
 #include <math.h>
 #include <stdint.h>
-#include <stdio.h>
 
-#include "../../include/gmz.h"
-#include "gmz_common.cuh"
+#include "gmz_internal.h"
 
 #define PER_MAX_CHUNK 2048
 // k_per_update's 32 warps own tree depths 0..31, so the deepest leaf may sit at depth 32: 2*capacity - 2 < 2^33 - 1.
 #define PER_MAX_CAPACITY (1ll << 32)
-
-extern "C" void gmz_set_error_(const char *msg);   // defined in gmz_engine.cu (feeds gmz_last_error)
 
 __device__ __forceinline__ int node_depth(long long k) { return 63 - __clzll((unsigned long long)(k + 1)); }
 
@@ -130,17 +126,11 @@ k_per_sample(const double *tree, long long capacity, long long count, const doub
         for (int i = threadIdx.x; i < B; i += blockDim.x) out_w[i] = __fdiv_rn(out_w[i], m);
 }
 
-static int per_fail(const char *msg)
-{
-    gmz_set_error_(msg);
-    return 1;
-}
-
 extern "C" int gmz_per_update(double *tree, int64_t capacity, const int64_t *tree_idx, const double *priorities, int n,
                               gmz_stream stream)
 {
-    if (!tree || !tree_idx || !priorities) return per_fail("gmz_per_update: null argument");
-    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return per_fail("gmz_per_update: capacity out of range (1 .. 2^32)");
+    if (!tree || !tree_idx || !priorities) return gmz_fail("gmz_per_update: null argument");
+    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return gmz_fail("gmz_per_update: capacity out of range (1 .. 2^32)");
     static bool attr_set = false;
     if (!attr_set) {
         cudaFuncSetAttribute(k_per_update, cudaFuncAttributeMaxDynamicSharedMemorySize, PER_MAX_CHUNK * (int)sizeof(double));
@@ -151,9 +141,7 @@ extern "C" int gmz_per_update(double *tree, int64_t capacity, const int64_t *tre
         k_per_update<<<1, 1024, m * sizeof(double), (cudaStream_t)stream>>>(tree, 2 * capacity - 1, (const long long *)tree_idx + off,
                                                                            priorities + off, m);
     }
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return per_fail(cudaGetErrorString(e));
-    return 0;
+    return gmz_check_launch("k_per_update");
 }
 
 // SumTree.add for a batch (replay_buffer.py:21-25): leaf i goes to ring position (write_ptr + i) % capacity.
@@ -230,32 +218,30 @@ __global__ void k_per_add_nodes(double *tree, long long capacity, long long writ
 extern "C" int gmz_per_add(double *tree, int64_t capacity, int64_t write_ptr, const double *priorities, int n,
                            int64_t *scratch_idx, gmz_stream stream)
 {
-    if (!tree || !priorities || !scratch_idx) return per_fail("gmz_per_add: null argument");
-    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return per_fail("gmz_per_add: capacity out of range (1 .. 2^32)");
+    if (!tree || !priorities || !scratch_idx) return gmz_fail("gmz_per_add: null argument");
+    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return gmz_fail("gmz_per_add: capacity out of range (1 .. 2^32)");
     if (n <= 0) return 0;
-    if (write_ptr < 0 || write_ptr >= capacity) return per_fail("gmz_per_add: write_ptr outside the ring");
+    if (write_ptr < 0 || write_ptr >= capacity) return gmz_fail("gmz_per_add: write_ptr outside the ring");
     if (n >= 64 && (int64_t)n <= capacity && capacity >= 2) {     // bulk path: node-parallel, whole GPU
         double *change = reinterpret_cast<double *>(scratch_idx);  // the caller's int64 [n] scratch, reused as float64 [n]
         k_per_add_leaves<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(tree, capacity, write_ptr, priorities, n, change);
+        if (gmz_check_launch("k_per_add_leaves")) return 1;
         const long long nodes = capacity - 1;
         k_per_add_nodes<<<(unsigned)((nodes + 127) / 128), 128, 0, (cudaStream_t)stream>>>(tree, capacity, write_ptr, n, change);
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return per_fail(cudaGetErrorString(e));
-        return 0;
+        return gmz_check_launch("k_per_add_nodes");
     }
     k_per_add_idx<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>((long long *)scratch_idx, capacity, write_ptr, n);
+    if (gmz_check_launch("k_per_add_idx")) return 1;
     return gmz_per_update(tree, capacity, scratch_idx, priorities, n, stream);
 }
 
 extern "C" int gmz_per_sample(const double *tree, int64_t capacity, int64_t count, const double *u01, int batch, double beta,
                               int64_t *out_tree_idx, double *out_priority, float *out_weights, gmz_stream stream)
 {
-    if (!tree || !u01 || !out_tree_idx || !out_priority || !out_weights) return per_fail("gmz_per_sample: null argument");
-    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return per_fail("gmz_per_sample: capacity out of range (1 .. 2^32)");
+    if (!tree || !u01 || !out_tree_idx || !out_priority || !out_weights) return gmz_fail("gmz_per_sample: null argument");
+    if (capacity < 1 || capacity > PER_MAX_CAPACITY) return gmz_fail("gmz_per_sample: capacity out of range (1 .. 2^32)");
     if (batch <= 0) return 0;
     k_per_sample<<<1, 1024, 0, (cudaStream_t)stream>>>(tree, capacity, count, u01, batch, beta,
                                                         (long long *)out_tree_idx, out_priority, out_weights);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return per_fail(cudaGetErrorString(e));
-    return 0;
+    return gmz_check_launch("k_per_sample");
 }

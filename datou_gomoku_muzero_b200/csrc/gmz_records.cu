@@ -10,15 +10,10 @@
 //     (workers.py:430-433) is gathered straight from the ring, D4 augmentation (loss.py:37-51) included.
 // Record layout (gmz_move_record_bytes): 64-byte header | policy f64[A] | obs f32[3A] | board i8[A] | pad to 16.
 #include <stdint.h>
-#include <stdio.h>
 
-#include "../../include/gmz.h"
-#include "gmz_common.cuh"
+#include "gmz_internal.h"
 #include "gmz_records.cuh"
 #include "gmz_tactics.cuh"
-
-extern "C" void gmz_set_error_(const char *msg);
-static int rc_fail(const char *m) { gmz_set_error_(m); return 1; }
 
 extern "C" size_t gmz_move_record_bytes(int board_size)
 {
@@ -37,9 +32,9 @@ k_records_tactics(const unsigned char *records, size_t stride, int N, int n_in_r
     __shared__ int8_t sb[GMZ_MAX_BOARD * GMZ_MAX_BOARD];
     const int A = N * N;
     const unsigned char *rec = records + (size_t)blockIdx.x * stride;
-    const int8_t *brd = reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * A);
+    const int8_t *brd = rec_board(rec, A);
     for (int i = threadIdx.x; i < A; i += blockDim.x) sb[i] = brd[i];
-    const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
+    const gmz_move_record *h = rec_header(rec);
     const int P = h->to_move >= 0 ? 1 : -1, action = h->action;
     __syncthreads();
     int any = 0, five = 0, played = 0;
@@ -58,18 +53,17 @@ k_records_tactics(const unsigned char *records, size_t stride, int N, int n_in_r
 extern "C" int gmz_records_tactics(const void *records, int64_t n_records, int board_size, int n_in_row, uint8_t *out_flags,
                                    gmz_stream stream)
 {
-    if (!records || !out_flags) return rc_fail("gmz_records_tactics: null argument");
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail("gmz_records_tactics: board_size out of range");
-    if (n_in_row < 1) return rc_fail("gmz_records_tactics: n_in_row must be >= 1");
-    if (n_records < 0 || n_records > 0x7fffffff) return rc_fail("gmz_records_tactics: n_records out of range");
+    if (!records || !out_flags) return gmz_fail("gmz_records_tactics: null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return gmz_fail("gmz_records_tactics: board_size out of range");
+    if (n_in_row < 1) return gmz_fail("gmz_records_tactics: n_in_row must be >= 1");
+    if (n_records < 0 || n_records > 0x7fffffff) return gmz_fail("gmz_records_tactics: n_records out of range");
     if (n_records == 0) return 0;
     const int A = board_size * board_size;
     int threads = ((A + 31) / 32) * 32;          // the block-size rule of gmz_tactics_classify
     if (threads > 512) threads = 512;
     k_records_tactics<<<(unsigned)n_records, threads, 0, (cudaStream_t)stream>>>((const unsigned char *)records, rec_stride(A),
                                                                                board_size, n_in_row, out_flags);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail(cudaGetErrorString(e));
+    return gmz_check_launch("k_records_tactics");
 }
 
 __device__ __forceinline__ float rec_final_reward(int i, int T, int winner)   // workers.py:183-187
@@ -88,8 +82,8 @@ __device__ __forceinline__ void rec_apply(u64 &P, u64 &M, int colour, int a, int
 // marks `last` (-1 or any value outside [0, A): no cell).  Called by the whole warp: every lane takes part in the shuffles.
 __device__ __forceinline__ void rec_write_position(unsigned char *rec, int A, u64 P, u64 M, int colour, int last, int lane)
 {
-    float *obs = reinterpret_cast<float *>(rec + 64 + (size_t)8 * A);
-    int8_t *brd = reinterpret_cast<int8_t *>(rec + 64 + (size_t)20 * A);
+    float *obs = rec_obs(rec, A);
+    int8_t *brd = rec_board(rec, A);
     const u64 own = colour > 0 ? P : M, opp = colour > 0 ? M : P;
     for (int c0 = 0; c0 < A; c0 += 32) {
         const int c = c0 + lane, cw = min(c, A - 1) >> 6;
@@ -123,7 +117,7 @@ k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, co
     for (int t = wi; t < T; t += 4) {
         for (; m < t; ++m) { const int a = acts[m]; rec_apply(P, M, colour, a, lane); colour = -colour; last = a; ++mc; }
         unsigned char *rec = out + (size_t)(move_offset[gi] + t) * stride;
-        double *pol = reinterpret_cast<double *>(rec + 64);
+        double *pol = rec_policy(rec);
         const double *psrc = policy + ((size_t)slot * max_moves + t) * A;
         rec_write_position(rec, A, P, M, colour, last, lane);
         for (int c = lane; c < A; c += 32) pol[c] = psrc[c];
@@ -133,14 +127,14 @@ k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, co
             for (int i = 0; i < n_steps; ++i)
                 if (t + i < T) acc = __dadd_rn(acc, __dmul_rn(dpow[i], (double)rec_final_reward(t + i, T, winner)));
             const int b = t + n_steps;
-            RecHeader h;
+            gmz_move_record h;
             h.game_seq = gi; h.t = t; h.length = T; h.winner = winner;
             h.action = acts[t]; h.to_move = colour; h.last_move = last; h.move_count = mc;
             h.reward = rec_final_reward(t, T, winner);
             h.value_target = b < T ? __fadd_rn((float)acc, __fmul_rn((float)vals[b], gn)) : (float)acc;
             h.search_value = vals[t];
-            h.game = game; h.slot = slot; h.opening = start_opening ? start_opening[slot] : 0; h.pad1 = 0;
-            *reinterpret_cast<RecHeader *>(rec) = h;
+            h.game = game; h.slot = slot; h.opening = start_opening ? start_opening[slot] : 0; h.reserved = 0;
+            *rec_header(rec) = h;
         }
     }
 }
@@ -148,15 +142,14 @@ k_traj_pack(int N, int A, size_t stride, int max_moves, const double *policy, co
 extern "C" int gmz_traj_pack(const gmz_traj *traj, int board_size, const int32_t *fin, int n_games, const int64_t *move_offset,
                              const double *discount_pow, int n_steps, void *out_records, gmz_stream stream)
 {
-    if (!traj || !fin || !move_offset || !discount_pow || !out_records) return rc_fail("gmz_traj_pack: null argument");
+    if (!traj || !fin || !move_offset || !discount_pow || !out_records) return gmz_fail("gmz_traj_pack: null argument");
     if (n_games <= 0) return 0;
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD || n_steps < 0) return rc_fail("gmz_traj_pack: bad size");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD || n_steps < 0) return gmz_fail("gmz_traj_pack: bad size");
     const int A = board_size * board_size;
     k_traj_pack<<<n_games, 128, 0, (cudaStream_t)stream>>>(board_size, A, rec_stride(A), traj->max_moves, traj->policy, traj->value,
                                                            traj->action, (const u64 *)traj->start_board, traj->start_info, traj->start_opening, fin, n_games,
                                                            move_offset, discount_pow, n_steps, (unsigned char *)out_records);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail(cudaGetErrorString(e));
+    return gmz_check_launch("k_traj_pack");
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -193,15 +186,15 @@ k_records_batch(int N, int A, size_t stride, int64_t capacity, const unsigned ch
     const int lane = threadIdx.x & 31, b = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (b >= B) return;
     const int64_t p0 = pos[b];
-    const RecHeader h0 = *reinterpret_cast<const RecHeader *>(ring + (size_t)p0 * stride);
+    const gmz_move_record h0 = *rec_header(ring + (size_t)p0 * stride);
     for (int k = 0; k <= U; ++k) {
         float *o = obs + ((size_t)b * (U + 1) + k) * 3 * A;
         double *pk = pi + ((size_t)b * (U + 1) + k) * A;
         if (h0.t + k < h0.length) {
-            const unsigned char *rec = ring + (size_t)((p0 + k) % capacity) * stride;
-            const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
-            const double *pol = reinterpret_cast<const double *>(rec + 64);
-            const float *ob = reinterpret_cast<const float *>(rec + 64 + (size_t)8 * A);
+            const unsigned char *rec = rec_at(ring, stride, capacity, p0, k);
+            const gmz_move_record *h = rec_header(rec);
+            const double *pol = rec_policy(rec);
+            const float *ob = rec_obs(rec, A);
             for (int c = lane; c < A; c += 32) {
                 const int d = rec_sym_cell(c, N, rk, fl);
                 o[d] = ob[c]; o[A + d] = ob[A + c]; o[2 * A + d] = ob[2 * A + c];
@@ -224,28 +217,20 @@ k_records_batch(int N, int A, size_t stride, int64_t capacity, const unsigned ch
 extern "C" int gmz_records_batch(const void *ring, int64_t capacity, int board_size, const int64_t *positions, int batch, int unroll,
                                  int rot_k, int flip, float *obs, int32_t *act, float *rew, double *pi, float *val, gmz_stream stream)
 {
-    if (!ring || !positions || !obs || !act || !rew || !pi || !val) return rc_fail("gmz_records_batch: null argument");
+    if (!ring || !positions || !obs || !act || !rew || !pi || !val) return gmz_fail("gmz_records_batch: null argument");
     if (batch <= 0) return 0;
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD || unroll < 0 || capacity < 1) return rc_fail("gmz_records_batch: bad size");
-    if (rot_k < 0 || rot_k > 3) return rc_fail("gmz_records_batch: rot_k must be 0..3");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD || unroll < 0 || capacity < 1) return gmz_fail("gmz_records_batch: bad size");
+    if (rot_k < 0 || rot_k > 3) return gmz_fail("gmz_records_batch: rot_k must be 0..3");
     const int A = board_size * board_size;
     k_records_batch<<<(batch + 3) / 4, 128, 0, (cudaStream_t)stream>>>(board_size, A, rec_stride(A), capacity, (const unsigned char *)ring,
                                                                        positions, batch, unroll, rot_k, flip ? 1 : 0, obs, act, rew, pi, val);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail(cudaGetErrorString(e));
+    return gmz_check_launch("k_records_batch");
 }
 
 // ---------------------------------------------------------------------------------------------------------
 // Re-analysis of a stretch of the ring in place (workers.py:243-305): record k of the stretch sits at ring position
 // (first + k) % capacity.  gmz_set_roots_from_records (gmz_engine.cu) loads the roots, the search runs, then the two
 // kernels below put the results back.
-static int rc_fail2(const char *name, const char *m)
-{
-    char buf[256];
-    snprintf(buf, sizeof(buf), "%s: %s", name, m);
-    gmz_set_error_(buf);
-    return 1;
-}
 
 // The re-searched policy row k and root value k replace the record's policy bytes and header search_value; nothing
 // else in the record is written.  One warp per record.
@@ -256,26 +241,24 @@ k_records_writeback(unsigned char *ring, size_t stride, int64_t capacity, int64_
     const int lane = threadIdx.x & 31;
     const int64_t k = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
     if (k >= n) return;
-    unsigned char *rec = ring + (size_t)((first + k) % capacity) * stride;
-    double *pol = reinterpret_cast<double *>(rec + 64);
+    unsigned char *rec = rec_at(ring, stride, capacity, first, k);
+    double *pol = rec_policy(rec);
     const double *src = policy + (size_t)k * A;
     for (int c = lane; c < A; c += 32) pol[c] = src[c];
-    if (lane == 0) reinterpret_cast<RecHeader *>(rec)->search_value = value[k];
+    if (lane == 0) rec_header(rec)->search_value = value[k];
 }
 
 extern "C" int gmz_records_writeback(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *policy,
                                      const double *value, gmz_stream stream)
 {
-    const char *name = "gmz_records_writeback";
-    if (!ring || !policy || !value) return rc_fail2(name, "null argument");
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
-    if (const char *m = rec_stretch_check(capacity, first, n)) return rc_fail2(name, m);
+    if (!ring || !policy || !value) return gmz_fail("gmz_records_writeback: null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return gmz_fail("gmz_records_writeback: board_size out of range (1..19)");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return gmz_fail("gmz_records_writeback: %s", m);
     if (n == 0) return 0;
     const int A = board_size * board_size;
     k_records_writeback<<<(unsigned)((n + 3) / 4), 128, 0, (cudaStream_t)stream>>>((unsigned char *)ring, rec_stride(A), capacity,
                                                                                    first, n, A, policy, value);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+    return gmz_check_launch("k_records_writeback");
 }
 
 // New n-step value targets from the re-searched root values, with re-analysis arithmetic (reanalysis.reanalyse ->
@@ -288,14 +271,14 @@ k_records_retarget(unsigned char *ring, size_t stride, int64_t capacity, int64_t
 {
     const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
-    const int64_t p = (first + k) % capacity;
-    RecHeader *h = reinterpret_cast<RecHeader *>(ring + (size_t)p * stride);
+    const int64_t p = (first + k) % capacity;         // record k and its bootstrap record: records 0 and n_steps from p
+    gmz_move_record *h = rec_header(rec_at(ring, stride, capacity, p, 0));
     const int t = h->t, T = h->length, winner = h->winner;
     float acc = 0.0f;
     for (int i = 0; i < n_steps && t + i < T; ++i) acc = __fadd_rn(acc, __fmul_rn((float)dpow[i], rec_final_reward(t + i, T, winner)));
     float boot = 0.0f;
     if ((int64_t)t + n_steps < T) {
-        const RecHeader *hb = reinterpret_cast<const RecHeader *>(ring + (size_t)((p + n_steps) % capacity) * stride);
+        const gmz_move_record *hb = rec_header(rec_at(ring, stride, capacity, p, n_steps));
         boot = __fmul_rn((float)hb->search_value, (float)dpow[n_steps]);
     }
     h->value_target = __fadd_rn(acc, boot);
@@ -304,17 +287,15 @@ k_records_retarget(unsigned char *ring, size_t stride, int64_t capacity, int64_t
 extern "C" int gmz_records_retarget(void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, const double *discount_pow,
                                     int n_steps, gmz_stream stream)
 {
-    const char *name = "gmz_records_retarget";
-    if (!ring || !discount_pow) return rc_fail2(name, "null argument");
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
-    if (const char *m = rec_stretch_check(capacity, first, n)) return rc_fail2(name, m);
-    if (n_steps < 0) return rc_fail2(name, "n_steps must be >= 0");
+    if (!ring || !discount_pow) return gmz_fail("gmz_records_retarget: null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return gmz_fail("gmz_records_retarget: board_size out of range (1..19)");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return gmz_fail("gmz_records_retarget: %s", m);
+    if (n_steps < 0) return gmz_fail("gmz_records_retarget: n_steps must be >= 0");
     if (n == 0) return 0;
     const int A = board_size * board_size;
     k_records_retarget<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>((unsigned char *)ring, rec_stride(A), capacity,
                                                                                      first, n, discount_pow, n_steps);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+    return gmz_check_launch("k_records_retarget");
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -339,25 +320,25 @@ k_records_compact(const unsigned char *ring, size_t stride, int64_t capacity, in
     const int lane = threadIdx.x & 31;
     const int64_t k = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
     if (k >= n) return;
-    const unsigned char *rec = ring + (size_t)((first + k) % capacity) * stride;
-    const RecHeader *h = reinterpret_cast<const RecHeader *>(rec);
-    if (lane < 16) reinterpret_cast<uint32_t *>(out_headers + (size_t)k * 64)[lane] = reinterpret_cast<const uint32_t *>(rec)[lane];
-    const double *pol = reinterpret_cast<const double *>(rec + 64);
+    const unsigned char *rec = rec_at(ring, stride, capacity, first, k);
+    const gmz_move_record *h = rec_header(rec);
+    rec_copy_header(out_headers + (size_t)k * REC_HEADER, rec, lane);
+    const double *pol = rec_policy(rec);
     double *dst = out_policy + (size_t)k * A;
     for (int c = lane; c < A; c += 32) dst[c] = pol[c];
 
     const bool start = k == 0 || h->t == 0;
     const int own = h->to_move > 0 ? 1 : -1, last = h->last_move;
-    const uint32_t *obs = reinterpret_cast<const uint32_t *>(rec + 64 + (size_t)8 * A);
-    const int8_t *brd = reinterpret_cast<const int8_t *>(rec + 64 + (size_t)20 * A);
+    const uint32_t *obs = reinterpret_cast<const uint32_t *>(rec_obs(rec, A));
+    const int8_t *brd = rec_board(rec, A);
     const int8_t *pbrd = nullptr;
     int pa = -1, pown = 0;
     if (!start) {
-        const unsigned char *prv = ring + (size_t)((first + k - 1) % capacity) * stride;
-        const RecHeader *hp = reinterpret_cast<const RecHeader *>(prv);
+        const unsigned char *prv = rec_at(ring, stride, capacity, first, k - 1);
+        const gmz_move_record *hp = rec_header(prv);
         pa = hp->action;
         pown = hp->to_move > 0 ? 1 : -1;
-        pbrd = reinterpret_cast<const int8_t *>(prv + 64 + (size_t)20 * A);
+        pbrd = rec_board(prv, A);
     }
     const uint32_t one = 0x3f800000u;                   // 1.0f
     bool bad = false;
@@ -376,17 +357,15 @@ k_records_compact(const unsigned char *ring, size_t stride, int64_t capacity, in
 extern "C" int gmz_records_compact(const void *ring, int64_t capacity, int board_size, int64_t first, int64_t n, void *out_headers,
                                    double *out_policy, uint8_t *out_flags, gmz_stream stream)
 {
-    const char *name = "gmz_records_compact";
-    if (!ring || !out_headers || !out_policy || !out_flags) return rc_fail2(name, "null argument");
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
-    if (const char *m = rec_stretch_check(capacity, first, n)) return rc_fail2(name, m);
+    if (!ring || !out_headers || !out_policy || !out_flags) return gmz_fail("gmz_records_compact: null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return gmz_fail("gmz_records_compact: board_size out of range (1..19)");
+    if (const char *m = rec_stretch_check(capacity, first, n)) return gmz_fail("gmz_records_compact: %s", m);
     if (n == 0) return 0;
     const int A = board_size * board_size;
     k_records_compact<<<(unsigned)((n + 3) / 4), 128, 0, (cudaStream_t)stream>>>((const unsigned char *)ring, rec_stride(A), capacity,
                                                                                  first, n, A, (unsigned char *)out_headers, out_policy,
                                                                                  out_flags);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+    return gmz_check_launch("k_records_compact");
 }
 
 // Loading: one CTA per segment, segment s = records [seg_start[s], seg_start[s+1]) (the last one up to n), clamped to
@@ -416,19 +395,19 @@ k_records_expand(const unsigned char *headers, const double *policy, int64_t n, 
         }
         if (lane == w) { P = pw; M = mw; }
     }
-    const size_t body = (size_t)64 + (size_t)21 * A;
+    const size_t body = rec_body(A);
     int64_t m = lo;
     for (int64_t k = lo + wi; k < hi; k += 4) {
         for (; m < k; ++m) {
-            const RecHeader *hm = reinterpret_cast<const RecHeader *>(headers + (size_t)m * 64);
+            const gmz_move_record *hm = rec_header(headers + (size_t)m * REC_HEADER);
             rec_apply(P, M, hm->to_move, hm->action, lane);
         }
         if (k < skip) continue;
-        const unsigned char *src = headers + (size_t)k * 64;
-        const RecHeader *hk = reinterpret_cast<const RecHeader *>(src);
-        unsigned char *rec = ring + (size_t)((first + k - skip) % capacity) * stride;
-        if (lane < 16) reinterpret_cast<uint32_t *>(rec)[lane] = reinterpret_cast<const uint32_t *>(src)[lane];
-        double *pol = reinterpret_cast<double *>(rec + 64);
+        const unsigned char *src = headers + (size_t)k * REC_HEADER;
+        const gmz_move_record *hk = rec_header(src);
+        unsigned char *rec = rec_at(ring, stride, capacity, first, k - skip);
+        rec_copy_header(rec, src, lane);
+        double *pol = rec_policy(rec);
         const double *psrc = policy + (size_t)k * A;
         for (int c = lane; c < A; c += 32) pol[c] = psrc[c];
         rec_write_position(rec, A, P, M, hk->to_move, hk->last_move, lane);
@@ -440,20 +419,18 @@ extern "C" int gmz_records_expand(const void *headers, const double *policy, int
                                   const int8_t *base_boards, int64_t n_seg, int64_t skip, int board_size, void *ring, int64_t capacity,
                                   int64_t first, gmz_stream stream)
 {
-    const char *name = "gmz_records_expand";
-    if (!headers || !policy || !seg_start || !base_boards || !ring) return rc_fail2(name, "null argument");
-    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return rc_fail2(name, "board_size out of range (1..19)");
-    if (capacity < 1) return rc_fail2(name, "capacity must be >= 1");
-    if (n < 0) return rc_fail2(name, "n must be >= 0");
-    if (skip < 0 || skip > n) return rc_fail2(name, "skip must be in 0..n");
-    if (n - skip > capacity) return rc_fail2(name, "n - skip exceeds the ring capacity");
-    if (first < 0 || first >= capacity) return rc_fail2(name, "first outside the ring [0, capacity)");
-    if (n > 0 && (n_seg < 1 || n_seg > n || n_seg > 0x7fffffff)) return rc_fail2(name, "n_seg must be in 1..n when n > 0");
+    if (!headers || !policy || !seg_start || !base_boards || !ring) return gmz_fail("gmz_records_expand: null argument");
+    if (board_size < 1 || board_size > GMZ_MAX_BOARD) return gmz_fail("gmz_records_expand: board_size out of range (1..19)");
+    if (capacity < 1) return gmz_fail("gmz_records_expand: capacity must be >= 1");
+    if (n < 0) return gmz_fail("gmz_records_expand: n must be >= 0");
+    if (skip < 0 || skip > n) return gmz_fail("gmz_records_expand: skip must be in 0..n");
+    if (n - skip > capacity) return gmz_fail("gmz_records_expand: n - skip exceeds the ring capacity");
+    if (first < 0 || first >= capacity) return gmz_fail("gmz_records_expand: first outside the ring [0, capacity)");
+    if (n > 0 && (n_seg < 1 || n_seg > n || n_seg > 0x7fffffff)) return gmz_fail("gmz_records_expand: n_seg must be in 1..n when n > 0");
     if (n == 0) return 0;
     const int A = board_size * board_size;
     k_records_expand<<<(unsigned)n_seg, 128, 0, (cudaStream_t)stream>>>((const unsigned char *)headers, policy, n, seg_start, base_boards,
                                                                         n_seg, skip, A, rec_stride(A), (unsigned char *)ring, capacity,
                                                                         first);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : rc_fail2(name, cudaGetErrorString(e));
+    return gmz_check_launch("k_records_expand");
 }

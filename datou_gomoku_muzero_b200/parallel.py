@@ -98,9 +98,9 @@ def gather_packed_games(packed, board_size, dst: int = 0, group=None, device=Non
     game tables, each padded to the largest rank.  No pickling, no per-game Python objects; with NCCL the records go
     GPU -> GPU.  `packed` may be None (this rank has nothing).  Returns a PackedGames on `dst` whose table has a
     fifth column = source rank; None elsewhere."""
-    from .trajectory import PackedGames
+    from .trajectory import PackedGames, record_dtype
     rank, world = dist.get_rank(group), dist.get_world_size(group)
-    stride = (64 + 21 * board_size * board_size + 15) // 16 * 16
+    stride = record_dtype(board_size).itemsize
     if device is None:
         device = packed.records.device if packed is not None and torch.is_tensor(packed.records) else torch.device("cpu")
     m = 0 if packed is None else packed.n_moves

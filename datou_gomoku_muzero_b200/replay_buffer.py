@@ -20,7 +20,7 @@ import torch
 from . import _lib
 from ._lib import check
 from .config import config
-from .trajectory import record_dtype
+from .trajectory import RECORD_HEADER, record_fields
 
 
 def _ptr(t):
@@ -199,7 +199,7 @@ def validate_ring_state(sd, board_size):
         return t
     seg = sd.get("seg_start")
     n_seg = int(seg.shape[0]) if torch.is_tensor(seg) and seg.dim() == 1 else -1
-    headers = tensor("headers", torch.uint8, (n, 64))
+    headers = tensor("headers", torch.uint8, (n, RECORD_HEADER.itemsize))
     tensor("policies", torch.float64, (n, A))
     seg = tensor("seg_start", torch.int64, (max(n_seg, 0),))
     base = tensor("base_boards", torch.int8, (max(n_seg, 0), A))
@@ -207,8 +207,8 @@ def validate_ring_state(sd, board_size):
     tensor("max_priority", torch.float64, ())
     if base.numel() and (base.min() < -1 or base.max() > 1):
         raise ValueError("ring state base_boards hold a value outside {-1, 0, 1}")
-    h = headers.numpy().view(np.int32)                  # gmz_move_record: game_seq, t, length, ...
-    t, T = h[:, 1].astype(np.int64), h[:, 2].astype(np.int64)
+    h = headers.numpy().view(RECORD_HEADER).reshape(-1)
+    t, T = h["t"].astype(np.int64), h["length"].astype(np.int64)
     k = np.arange(n)
     starts = (k == 0) | (t == 0)
     if not np.array_equal(seg.numpy(), np.flatnonzero(starts)):
@@ -248,8 +248,7 @@ class DeviceReplayBuffer:
         self.capacity, self.N, self.A = int(capacity), int(board_size), int(board_size) ** 2
         self.device, self.lib = self.sum_tree.device, self.sum_tree.lib
         self.stride = int(self.lib.gmz_move_record_bytes(self.N))
-        # byte range of each record field within a ring row (policy, board, header scalars, ...)
-        self._field = {name: slice(off, off + dt.itemsize) for name, (dt, off) in record_dtype(self.N).fields.items()}
+        self._field = record_fields(self.N)
         self.ring = torch.zeros((self.capacity, self.stride), dtype=torch.uint8, device=self.device)
         self.max_priority = torch.ones((), dtype=torch.float64, device=self.device)
         self.unroll = int(config.NUM_UNROLL_STEPS if unroll_steps is None else unroll_steps)
@@ -469,7 +468,7 @@ class DeviceReplayBuffer:
         predecessor and header imply (gmz_records_compact bit 1: such a record cannot be rebuilt)."""
         cap, n, wp, A, dev = self.capacity, self.sum_tree.count, self.sum_tree.write_ptr, self.A, self.device
         oldest = wp if n == cap else 0
-        headers = torch.empty((n, 64), dtype=torch.uint8, device=dev)
+        headers = torch.empty((n, RECORD_HEADER.itemsize), dtype=torch.uint8, device=dev)
         policies = torch.empty((n, A), dtype=torch.float64, device=dev)
         seg = torch.empty(0, dtype=torch.int64, device=dev)
         if n > 0:

@@ -11,6 +11,7 @@ import torch
 from . import _lib
 from ._lib import check
 from .config import config
+from .trajectory import RECORD_HEADER
 
 FIVE, OPEN_FOUR, COMBO = 1, 2, 3
 
@@ -161,10 +162,11 @@ class SelfPlayStats:
         fives, missed = _missed(record_flags(packed.records[:M], packed.N, self.n_in_row))
         self._missed += torch.stack([fives.sum(), missed.sum()])
         if self.n_openings:
-            # first record of each game: winner (bytes 12..15), to_move (20..23), opening label + 1 (56..59)
+            # first record of each game: winner, to_move and opening label + 1, int32 columns of its header
             first = torch.as_tensor(np.asarray(packed.offsets[:-1], np.int64), device=self.device)
-            hdr = packed.records[first, :64].contiguous().view(torch.int32)
-            winner, to_move, label = hdr[:, 3], hdr[:, 5], hdr[:, 14].to(torch.int64) - 1
+            hdr = packed.records[first, :RECORD_HEADER.itemsize].contiguous().view(torch.int32)
+            winner, to_move, opening = (hdr[:, RECORD_HEADER.fields[f][1] // 4] for f in ("winner", "to_move", "opening"))
+            label = opening.to(torch.int64) - 1
             outcome = torch.where(winner == 0, 1, torch.where(winner == to_move, 0, 2)).to(torch.int64)
             ok = (label >= 0) & (label < self.n_openings)
             self._by_opening.view(-1).index_add_(0, torch.where(ok, label * 3 + outcome, 0), ok.to(torch.int64))

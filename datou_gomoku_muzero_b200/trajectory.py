@@ -17,16 +17,28 @@ from .config import config
 from .data_structures import GameRecord, TrainingSlice
 
 
+# The 64-byte header of a packed move record, include/gmz.h gmz_move_record (fields packed in this order).
+RECORD_HEADER = np.dtype([("game_seq", "<i4"), ("t", "<i4"), ("length", "<i4"), ("winner", "<i4"), ("action", "<i4"),
+                          ("to_move", "<i4"), ("last_move", "<i4"), ("move_count", "<i4"), ("reward", "<f4"),
+                          ("value_target", "<f4"), ("search_value", "<f8"), ("game", "<i4"), ("slot", "<i4"),
+                          ("opening", "<i4"), ("reserved", "<i4")])
+
+
 def record_dtype(board_size):
-    """numpy view of one packed move record (include/gmz.h gmz_move_record + payload)."""
+    """numpy view of one packed move record: header | policy f64[A] | obs f32[3A] | board i8[A] | pad to 16 bytes."""
     N = int(board_size)
-    A = N * N
-    stride = (64 + 21 * A + 15) // 16 * 16
-    names = ["game_seq", "t", "length", "winner", "action", "to_move", "last_move", "move_count", "reward", "value_target",
-             "search_value", "game", "slot", "opening", "policy", "obs", "board"]
-    formats = ["<i4"] * 8 + ["<f4", "<f4", "<f8", "<i4", "<i4", "<i4", ("<f8", (A,)), ("<f4", (3, N, N)), ("i1", (N, N))]
-    offsets = [0, 4, 8, 12, 16, 20, 24, 28, 32, 36, 40, 48, 52, 56, 64, 64 + 8 * A, 64 + 20 * A]
-    return np.dtype({"names": names, "formats": formats, "offsets": offsets, "itemsize": stride})
+    fields = dict(RECORD_HEADER.fields)
+    end = RECORD_HEADER.itemsize
+    for name, fmt in (("policy", ("<f8", (N * N,))), ("obs", ("<f4", (3, N, N))), ("board", ("i1", (N, N)))):
+        fields[name] = (np.dtype(fmt), end)
+        end += fields[name][0].itemsize
+    return np.dtype({"names": list(fields), "formats": [dt for dt, _ in fields.values()],
+                     "offsets": [off for _, off in fields.values()], "itemsize": (end + 15) // 16 * 16})
+
+
+def record_fields(board_size):
+    """name -> byte slice of that field within a packed record row (uint8 [stride])."""
+    return {name: slice(off, off + dt.itemsize) for name, (dt, off) in record_dtype(board_size).fields.items()}
 
 
 class PackedGames:
@@ -62,7 +74,7 @@ class PackedGames:
         first = self.offsets[:-1]
         if self._host is None and torch.is_tensor(self.records) and self.records.is_cuda:
             idx = torch.as_tensor(first, device=self.records.device)
-            lab = self.records[idx, 56:60].contiguous().view(torch.int32).reshape(-1).cpu().numpy()
+            lab = self.records[idx, record_fields(self.N)["opening"]].contiguous().view(torch.int32).reshape(-1).cpu().numpy()
         else:
             lab = self.host()["opening"][first]
         return lab.astype(np.int32) - 1

@@ -120,11 +120,16 @@ def test_entry_points_reject_bad_arguments_without_crashing():
         ("gmz_hidden_gather", (N, N, N, 4, 20, 4, 36, 256, N, 0, N, N)), ("gmz_hidden_scatter", (N, N, 4, 20, 4, 9216, N, N)),
         ("gmz_tactics_classify", (N, N, 4, 9, 5, N, N)), ("gmz_per_update", (N, 8, N, N, 4, N)),
         ("gmz_per_add", (N, 8, 0, N, 4, N, N)), ("gmz_per_sample", (N, 8, 8, N, 4, 0.4, N, N, N, N)),
+        ("gmz_traj_pack", (N, 9, N, 1, N, N, 5, N, N)), ("gmz_records_batch", (N, 8, 9, N, 4, 5, 0, 0, N, N, N, N, N, N)),
+        ("gmz_records_tactics", (N, 4, 9, 5, N, N)), ("gmz_set_roots_from_records", (N, N, 8, 0, 4, N)),
+        ("gmz_records_writeback", (N, 8, 9, 0, 4, N, N, N)), ("gmz_records_retarget", (N, 8, 9, 0, 4, N, 5, N)),
+        ("gmz_records_compact", (N, 8, 9, 0, 4, N, N, N, N)), ("gmz_records_expand", (N, N, 4, N, N, 1, 0, 9, N, 8, 0, N)),
     ]
     for name, args in calls:
         rc = getattr(lib, name)(*args)
         assert rc != 0, f"{name} accepted null arguments"
         assert lib.gmz_last_error(), f"{name} left no error message"
+        assert name.encode() in lib.gmz_last_error(), f"{name} error message does not name it: {lib.gmz_last_error()}"
     one = (C.c_double * 1)(1.0)
     assert lib.gmz_per_add(one, 8, 9, one, 1, (C.c_int64 * 1)(0), None) != 0          # write_ptr outside the ring
     assert lib.gmz_tactics_classify((C.c_int8 * 4)(), (C.c_int8 * 1)(1), 1, 40, 5, (C.c_int8 * 4)(), None) != 0   # board too large

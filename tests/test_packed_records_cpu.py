@@ -76,6 +76,26 @@ def test_record_layout_matches_the_header():
     assert lib.gmz_move_record_bytes(0) == 0 and lib.gmz_move_record_bytes(20) == 0
 
 
+def test_header_dtype_matches_the_c_struct(tmp_path):
+    """trajectory.RECORD_HEADER has every gmz_move_record field at the C compiler's offset and size, and nothing else."""
+    import subprocess
+    from datou_gomoku_muzero_b200.trajectory import RECORD_HEADER
+    src = tmp_path / "header_layout.c"
+    src.write_text("#include <stddef.h>\n#include <stdio.h>\n#include \"gmz.h\"\nint main(void)\n{\n"
+                   "    printf(\"sizeof %zu\\n\", sizeof(gmz_move_record));\n"
+                   + "".join(f"    printf(\"{f} %zu %zu\\n\", offsetof(gmz_move_record, {f}), sizeof(((gmz_move_record *)0)->{f}));\n"
+                             for f in RECORD_HEADER.names)
+                   + "    return 0;\n}\n")
+    exe = tmp_path / "header_layout"
+    subprocess.check_call(["gcc", "-std=c11", "-I", os.path.join(ROOT, "include"), "-o", str(exe), str(src)])
+    lines = [ln.split() for ln in subprocess.check_output([str(exe)], text=True).splitlines()]
+    assert lines[0] == ["sizeof", str(RECORD_HEADER.itemsize)]
+    got = {f: (int(off), int(size)) for f, off, size in lines[1:]}
+    want = {f: (off, dt.itemsize) for f, (dt, off) in RECORD_HEADER.fields.items()}
+    assert got == want
+    assert sum(size for _, size in got.values()) == RECORD_HEADER.itemsize      # no C field left out of the dtype
+
+
 def _gather_worker(rank, world, port, out_q):
     import torch.distributed as dist
     sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
