@@ -217,7 +217,8 @@ k_records_batch(int N, int A, size_t stride, int64_t capacity, const unsigned ch
 extern "C" int gmz_records_batch(const void *ring, int64_t capacity, int board_size, const int64_t *positions, int batch, int unroll,
                                  int rot_k, int flip, float *obs, int32_t *act, float *rew, double *pi, float *val, gmz_stream stream)
 {
-    if (!ring || !positions || !obs || !act || !rew || !pi || !val) return gmz_fail("gmz_records_batch: null argument");
+    // act / rew hold B * unroll entries: none when unroll == 0 (an empty tensor's data pointer may be NULL)
+    if (!ring || !positions || !obs || !pi || !val || (unroll > 0 && (!act || !rew))) return gmz_fail("gmz_records_batch: null argument");
     if (batch <= 0) return 0;
     if (board_size < 1 || board_size > GMZ_MAX_BOARD || unroll < 0 || capacity < 1) return gmz_fail("gmz_records_batch: bad size");
     if (rot_k < 0 || rot_k > 3) return gmz_fail("gmz_records_batch: rot_k must be 0..3");

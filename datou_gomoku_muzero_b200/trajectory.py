@@ -44,8 +44,9 @@ def record_fields(board_size):
 class PackedGames:
     """Finished games as packed move records (csrc/gmz_records.cu): `records` uint8 [M, stride] (device or host
     tensor), `table` int32 [n, 4] = (slot, game, length, winner) per game, `offsets` int64 [n + 1] = first record of
-    each game.  What the reference puts on data_queue per game -- (GameRecord, [TrainingSlice], version),
-    workers.py:230 -- is a set of numpy views of these bytes."""
+    each game; a game's length is its number of records (np.diff(offsets) == table[:, 2]).  What the reference puts
+    on data_queue per game -- (GameRecord, [TrainingSlice], version), workers.py:230 -- is a set of numpy views of
+    these bytes."""
 
     def __init__(self, records, table, offsets, board_size):
         self.records, self.table, self.offsets, self.N = records, np.asarray(table), np.asarray(offsets, np.int64), int(board_size)
@@ -107,6 +108,15 @@ class PackedGames:
         return [(self.game_record(i), self.training_slices(i), model_version) for i in range(len(self))]
 
 
+def whole_games(fin, max_moves):
+    """fin_queue rows int32 [n, 4] = (slot, game, length, winner) -> the rows of the games that played at most
+    `max_moves` moves (every move recorded), and the offset of each one's first record in a pack of them, int64
+    [n_whole + 1]."""
+    fin = np.asarray(fin)
+    q = fin[fin[:, 2] <= max_moves]
+    return q, np.concatenate([[0], np.cumsum(q[:, 2], dtype=np.int64)]).astype(np.int64)
+
+
 class TrajectoryStore:
     def __init__(self, engine, extra_slots=None, max_moves=None):
         e = self.e = engine
@@ -115,6 +125,7 @@ class TrajectoryStore:
         self.max_moves = A if max_moves is None else int(max_moves)
         if self.max_moves < 1:
             raise ValueError("max_moves must be >= 1")
+        self.truncated_games = 0        # finished games pack_finished left out: longer than max_moves
         dev = e.device
         n, T = self.n_slots, self.max_moves
         self.policy = torch.zeros((n, T, A), dtype=torch.float64, device=dev)
@@ -137,9 +148,10 @@ class TrajectoryStore:
     def harvest(self, copy_policies=True, unpark=True):
         """Finished games since the last harvest -> list of dicts (host arrays).  Their slots go back on the free
         stack and (with `unpark`) parked games restart -- pass unpark=False after play(restart=False) to leave
-        finished games finished.  A game that recorded more moves than the store's `max_moves` (only possible with a
+        finished games finished.  A game that played more moves than the store's `max_moves` (only possible with a
         user-supplied max_moves below the remaining plies) comes back with `length` clamped to what was recorded and
-        `truncated` = True.  `opening` is the index of the book opening the game was dealt, -1 for none."""
+        `truncated` = True; build_game_record refuses it.  `opening` is the index of the book opening the game was
+        dealt, -1 for none."""
         e = self.e
         n = int(self.fin_count.item())
         if n == 0:
@@ -170,31 +182,39 @@ class TrajectoryStore:
         return out
 
     def pack_finished(self, recycle=True):
-        """Finished games since the last harvest / pack -> PackedGames on the DEVICE (None if there are none): one
+        """Finished games since the last harvest / pack -> PackedGames on the DEVICE (None if no whole game finished): one
         kernel expands every finished slot into fixed-stride move records (observations, policies, boards, final
         rewards, n-step value targets); nothing is computed per move on the host.  With `recycle` the slots go back
-        on the free stack and parked games restart."""
+        on the free stack and parked games restart.
+
+        Only whole games are packed.  A game longer than `max_moves` has no record of its last moves, so neither its
+        rewards (counted back from the winning move) nor the bootstraps near the cut can be computed; it is left out,
+        its slot is released like the others, and `truncated_games` counts it."""
         e = self.e
         n = int(self.fin_count.item())
         if n == 0:
             return None
-        q = self.fin_queue[:n].cpu().numpy()
-        lens = np.minimum(q[:, 2], self.max_moves).astype(np.int64)
-        off = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
-        stride = int(e.lib.gmz_move_record_bytes(e.N))
-        # allocated in power-of-two buckets (>= 8192 records): chunks of similar size then reuse the caching allocator's
-        # blocks (a fresh cudaMalloc of a few hundred MB costs ~100 ms, 300x the pack kernel itself)
-        M = int(off[-1])
-        rec = torch.empty((max(8192, 1 << (M - 1).bit_length()), stride), dtype=torch.uint8, device=e.device)[:M]
-        off_d = torch.as_tensor(off[:-1].copy(), device=e.device)
-        dpow = torch.tensor([config.DISCOUNT ** i for i in range(config.N_STEPS + 1)], dtype=torch.float64, device=e.device)
-        check(e.lib.gmz_traj_pack(C.byref(self.c), e.N, self.fin_queue.data_ptr(), n, off_d.data_ptr(), dpow.data_ptr(),
-                                  int(config.N_STEPS), rec.data_ptr(), e._stream()), "gmz_traj_pack")
-        e.launches += 1
+        fin = self.fin_queue[:n].cpu().numpy()
+        q, off = whole_games(fin, self.max_moves)
+        self.truncated_games += n - len(q)
+        packed = None
+        if len(q):
+            stride = int(e.lib.gmz_move_record_bytes(e.N))
+            # allocated in power-of-two buckets (>= 8192 records): chunks of similar size then reuse the caching allocator's
+            # blocks (a fresh cudaMalloc of a few hundred MB costs ~100 ms, 300x the pack kernel itself)
+            M = int(off[-1])
+            rec = torch.empty((max(8192, 1 << (M - 1).bit_length()), stride), dtype=torch.uint8, device=e.device)[:M]
+            off_d = torch.as_tensor(off[:-1].copy(), device=e.device)
+            fin_d = self.fin_queue if len(q) == n else torch.as_tensor(q, device=e.device)
+            dpow = torch.tensor([config.DISCOUNT ** i for i in range(config.N_STEPS + 1)], dtype=torch.float64, device=e.device)
+            check(e.lib.gmz_traj_pack(C.byref(self.c), e.N, fin_d.data_ptr(), len(q), off_d.data_ptr(), dpow.data_ptr(),
+                                      int(config.N_STEPS), rec.data_ptr(), e._stream()), "gmz_traj_pack")
+            e.launches += 1
+            packed = PackedGames(rec, q, off, e.N)
         self.fin_count.zero_()
         if recycle:
-            self.release(torch.as_tensor(q[:, 0].astype(np.int32), device=e.device))
-        return PackedGames(rec, q, off, e.N)
+            self.release(torch.as_tensor(fin[:, 0].astype(np.int32), device=e.device))
+        return packed
 
     def free_slots_left(self):
         return int(self.free_top.item())
@@ -244,7 +264,10 @@ def compute_n_step_returns(rewards, values, discount, n_steps):
 
 
 def build_game_record(rec, board_size=None):
-    """One harvested game (from an empty start) -> GameRecord (workers.py:172-206)."""
+    """One harvested game (from an empty start) -> GameRecord (workers.py:172-206).  ValueError for a truncated game
+    (harvest's `truncated`): its rewards count back from a winning move that was not recorded."""
+    if rec.get("truncated", False):
+        raise ValueError("build_game_record: the game is truncated (longer than the store's max_moves)")
     N = board_size or rec["start_board"].shape[0]
     T = rec["length"]
     board = rec["start_board"].astype(np.int8).copy()

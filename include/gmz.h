@@ -339,7 +339,7 @@ int gmz_traj_pack(const gmz_traj *traj, int board_size, const int32_t *fin, int 
  * (loss.py:37-51): planes and policies turned rot_k (0..3) quarter turns as torch.rot90 does, then flipped
  * left-right if `flip`; actions by the reference's own index formula (loss.py:46-51), padded entries stay -1.
  * Outputs: obs f32 [B,U+1,3,N,N], act i32 [B,U] (padding -1), rew f32 [B,U], pi f64 [B,U+1,A], val f32 [B,U+1]
- * -- the tuple data_loader_worker stacks (workers.py:430-433). */
+ * -- the tuple data_loader_worker stacks (workers.py:430-433).  With unroll = 0, act and rew may be NULL. */
 int gmz_records_batch(const void *ring, int64_t capacity, int board_size, const int64_t *positions, int batch, int unroll,
                       int rot_k, int flip, float *obs, int32_t *act, float *rew, double *pi, float *val, gmz_stream stream);
 /* Missed-win flags of n_records consecutive records (a packed block or a stretch of the ring), read in place: the
