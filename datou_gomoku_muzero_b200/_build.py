@@ -10,9 +10,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libgmz.so")
 SOURCES = ["gmz_engine.cu", "gmz_per.cu", "gmz_tactics.cu", "gmz_hidden.cu", "gmz_records.cu", "gmz_match.cu", "gmz_inspect.cu"]
-# the persistent play kernel: one object per (MuZero mode, float32 accumulation, opening-book variant), built in parallel
+# the persistent play kernel: one object per (MuZero mode, float32 accumulation), built in parallel
 PLAY_SOURCE = "gmz_play_inst.cu"
-PLAY_VARIANTS = [(mz, f32, book) for book in (0, 1) for mz in (0, 1) for f32 in (0, 1)]
+PLAY_VARIANTS = [(mz, f32) for mz in (0, 1) for f32 in (0, 1)]
 HEADERS = ["gmz_common.cuh", "gmz_tree.cuh", "gmz_play.cuh", "gmz_tactics.cuh", "gmz_records.cuh", "gmz_engine.cuh", "gmz_internal.h", os.path.join("..", "..", "include", "gmz.h")]
 # -fmad=false: the search's float64 / float32 arithmetic must round once per operation, like the
 # reference's Python floats / NumPy scalars (SURVEY.md App. A.7); an FMA would change visit counts.
@@ -51,9 +51,9 @@ def build(force: bool = False, verbose: bool = False, verify: bool = False, vari
     jobs = []
     for s in SOURCES:
         jobs.append((common + ["-c", os.path.join(CSRC, s), "-o", os.path.join(objdir, s[:-3] + ".o")]))
-    for mz, f32, book in PLAY_VARIANTS:
-        jobs.append(common + [f"-DGMZ_PLAY_MZ={mz}", f"-DGMZ_PLAY_F32={f32}", f"-DGMZ_PLAY_BOOK={book}", "-c",
-                              os.path.join(CSRC, PLAY_SOURCE), "-o", os.path.join(objdir, f"gmz_play_mz{mz}_f{f32}_b{book}.o")])
+    for mz, f32 in PLAY_VARIANTS:
+        jobs.append(common + [f"-DGMZ_PLAY_MZ={mz}", f"-DGMZ_PLAY_F32={f32}", "-c", os.path.join(CSRC, PLAY_SOURCE), "-o",
+                              os.path.join(objdir, f"gmz_play_mz{mz}_f{f32}.o")])
     with ThreadPoolExecutor(max_workers=min(len(jobs), os.cpu_count() or 4)) as ex:
         list(ex.map(subprocess.check_call, jobs))
     objs = [j[-1] for j in jobs]

@@ -78,7 +78,8 @@ k_set_roots_records(Params p, const unsigned char *ring, size_t stride, int64_t 
     root_load(p, g, lane, rec_board(rec, p.A), h->to_move, h->last_move, h->move_count);
 }
 
-__global__ void __launch_bounds__(CTA_THREADS) k_games_reset(Params p, BookDev book, const uint8_t *mask)
+__global__ void __launch_bounds__(CTA_THREADS)
+k_games_reset(const __grid_constant__ Params p, const __grid_constant__ BookDev book, const uint8_t *mask)
 {
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
     if (g >= p.G) return;
@@ -311,8 +312,8 @@ __global__ void k_fill_gumbel(double *out, size_t n, u64 seed, u64 offset)
 // its own -- record (policy, value, action) in the game's trajectory slot, do_move, get_game_ended,
 // hand finished games to the host queue and restart them in a fresh slot (workers.py:172-189, 230).
 __global__ void __launch_bounds__(CTA_THREADS)
-k_selfplay_step(Params p, TrajDev t, BookDev book, int use_traj, int restart, const double *policy, const double *value,
-                const int32_t *action, int32_t *out_winner)
+k_selfplay_step(const __grid_constant__ Params p, const __grid_constant__ TrajDev t, const __grid_constant__ BookDev book, int use_traj,
+                int restart, const double *policy, const double *value, const int32_t *action, int32_t *out_winner)
 {
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
     if (g >= p.G) return;
@@ -325,50 +326,20 @@ k_selfplay_step(Params p, TrajDev t, BookDev book, int use_traj, int restart, co
     int slot = -1, tl = 0;
     if (use_traj) {
         slot = s->traj_slot; tl = s->traj_len;
-        if (tl == 0) {
-            if (lane < GMZ_WORDS) {
-                t.start_board[((size_t)slot * 2 + 0) * GMZ_WORDS + lane] = s->p1[lane];
-                t.start_board[((size_t)slot * 2 + 1) * GMZ_WORDS + lane] = s->m1[lane];
-            }
-            if (lane == 0) {
-                int32_t *si = t.start_info + (size_t)slot * 4;
-                si[0] = s->to_move; si[1] = s->move_count; si[2] = s->last_move; si[3] = g;
-                if (t.start_opening) t.start_opening[slot] = s->opening;
-            }
-        }
+        if (tl == 0) traj_open(t, s, slot, g, s->to_move, s->last_move, lane);
         if (tl < t.max_moves) {
             double *dst = t.policy + ((size_t)slot * t.max_moves + tl) * (size_t)p.A;
             for (int c = lane; c < p.A; c += 32) dst[c] = policy[(size_t)g * p.A + c];
-            if (lane == 0) { t.value[(size_t)slot * t.max_moves + tl] = value[g]; t.action[(size_t)slot * t.max_moves + tl] = a; }
         }
     }
-    __syncwarp();
-    const int wv = game_do_move(p, s, a, lane);
-    if (lane == 0) {
-        s->noise_ctr += 1; s->traj_len = tl + 1;
-        atomicAdd(&p.ctl->moves_played, 1ull);
-        if (out_winner) out_winner[g] = wv;
-    }
-    if (wv != GMZ_WINNER_NONE) {
-        int ok = 1, nslot = -1;
-        if (lane == 0) {
-            atomicAdd(&p.ctl->games_finished, 1ull);
-            if (use_traj) {
-                const int qi = atomicAdd(t.fin_count, 1);
-                if (qi < t.fin_cap) { int32_t *q = t.fin_queue + (size_t)qi * 4; q[0] = slot; q[1] = g; q[2] = tl + 1; q[3] = wv; }
-                ok = (qi < t.fin_cap) && restart && traj_pop_slot(t, nslot);
-                if (qi >= t.fin_cap) atomicSub(t.fin_count, 1);
-            } else ok = restart;
-        }
-        ok = __shfl_sync(GMZ_FULL, ok, 0); nslot = __shfl_sync(GMZ_FULL, nslot, 0);
-        __syncwarp();
-        if (ok) { game_deal(p, book, s, g, lane); if (lane == 0 && use_traj) s->traj_slot = nslot; }
-        else if (lane == 0) s->parked = use_traj ? 1 : 0;
-    }
+    const int wv = move_commit(p, t, s, use_traj, slot, tl, use_traj ? value[g] : 0.0, a, lane);   // value: null without a store
+    if (lane == 0 && out_winner) out_winner[g] = wv;
+    if (wv != GMZ_WINNER_NONE) game_finish(p, t, book, s, g, use_traj, restart, slot, tl + 1, wv, lane);
 }
 
 // parked games (finished, no free trajectory slot at the time): take a slot and restart
-__global__ void __launch_bounds__(CTA_THREADS) k_unpark(Params p, TrajDev t, BookDev book)
+__global__ void __launch_bounds__(CTA_THREADS)
+k_unpark(const __grid_constant__ Params p, const __grid_constant__ TrajDev t, const __grid_constant__ BookDev book)
 {
     const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5);
     if (g >= p.G) return;
@@ -376,10 +347,7 @@ __global__ void __launch_bounds__(CTA_THREADS) k_unpark(Params p, TrajDev t, Boo
     if (!s->parked) return;
     int ok = 0, slot = -1;
     if (lane == 0) ok = traj_pop_slot(t, slot);
-    ok = __shfl_sync(GMZ_FULL, ok, 0); slot = __shfl_sync(GMZ_FULL, slot, 0);
-    if (!ok) return;
-    game_deal(p, book, s, g, lane);
-    if (lane == 0) s->traj_slot = slot;
+    if (__shfl_sync(GMZ_FULL, ok, 0)) game_redeal(p, book, s, g, 1, slot, lane);
 }
 // give every game its initial trajectory slot (slot g) and clear the play bookkeeping
 __global__ void k_traj_init(Params p, TrajDev t)
@@ -638,17 +606,11 @@ extern "C" int gmz_e0_eval_obs(const float *obs, int batch, int board_size, uint
         obs, batch, board_size, e0_spec((u64)seed, logit_div), logits, values);
     return check_launch("k_e0_eval_obs");
 }
-// Self-play takes the book variant once a book has ever been bound, so that games dealt from it keep their labels after
-// an unbind; a search-only launch deals nothing and always takes the default variant.
 static int launch_play(gmz_engine *e, const PlayArgs &a, cudaStream_t st)
 {
-    const bool mz = e->p.mode == GMZ_MODE_MUZERO, f = e->p.f32acc != 0;
-    if (a.do_step && e->book_ever) {
-        if (mz) return f ? gmz_launch_play_mz1_f1_b1(e, a, st) : gmz_launch_play_mz1_f0_b1(e, a, st);
-        return f ? gmz_launch_play_mz0_f1_b1(e, a, st) : gmz_launch_play_mz0_f0_b1(e, a, st);
-    }
-    if (mz) return f ? gmz_launch_play_mz1_f1_b0(e, a, st) : gmz_launch_play_mz1_f0_b0(e, a, st);
-    return f ? gmz_launch_play_mz0_f1_b0(e, a, st) : gmz_launch_play_mz0_f0_b0(e, a, st);
+    const bool f = e->p.f32acc != 0;
+    if (e->p.mode == GMZ_MODE_MUZERO) return f ? gmz_launch_play_mz1_f1(e, a, st) : gmz_launch_play_mz1_f0(e, a, st);
+    return f ? gmz_launch_play_mz0_f1(e, a, st) : gmz_launch_play_mz0_f0(e, a, st);
 }
 static TrajDev traj_dev(const gmz_traj *t)
 {
@@ -735,7 +697,6 @@ extern "C" int gmz_set_openings(gmz_engine *e, const gmz_openings *book, gmz_str
     if (book) {
         e->book.n = book->n_openings; e->book.boards = book->boards; e->book.players = book->players;
         e->book.last_moves = book->last_moves; e->book.move_counts = book->move_counts;
-        e->book_ever = 1;
     }
     return 0;
 }

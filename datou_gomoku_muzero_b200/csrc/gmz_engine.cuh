@@ -5,6 +5,19 @@
 // Non-zero if `e` is a live handle (created and not yet destroyed); defined in gmz_engine.cu.
 int gmz_engine_live(const gmz_engine *e);
 
+// A new root for the GState: the bitboards (lane w < GMZ_WORDS holds word w of P, M and the valid cells V) and every
+// field a new root resets.  The opening label is left to the callers that deal games.
+__device__ __forceinline__ void root_write(GState *s, int lane, u64 P, u64 M, u64 V, int to_move, int last_move, int move_count,
+                                           bool active)
+{
+    if (lane < GMZ_WORDS) { s->p1[lane] = P; s->m1[lane] = M; s->valid[lane] = V; }
+    if (lane == 0) {
+        s->to_move = to_move; s->last_move = last_move; s->move_count = move_count; s->active = active;
+        s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
+        s->winner = GMZ_WINNER_NONE;
+    }
+}
+
 // board int8 [A] -> game g's bitboards; one warp per game, ballots pack 32 cells at a time.  b == NULL: a full board
 // of +1 stones (an inactive padding root).
 __device__ __forceinline__ void root_load(const Params &p, int g, int lane, const int8_t *b, int player, int last_move,
@@ -25,37 +38,25 @@ __device__ __forceinline__ void root_load(const Params &p, int g, int lane, cons
         if (lane == w) { P = pw; M = mw; V = vw; }
     }
     GState *s = p.gs + g;
-    if (lane < GMZ_WORDS) { s->p1[lane] = P; s->m1[lane] = M; s->valid[lane] = V; }
-    if (lane == 0) {
-        s->to_move = player >= 0 ? 1 : -1;
-        s->last_move = last_move;
-        s->move_count = move_count;
-        s->active = nvalid > 0;
-        s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
-        s->winner = GMZ_WINNER_NONE; s->opening = 0;
-    }
+    root_write(s, lane, P, M, V, player >= 0 ? 1 : -1, last_move, move_count, nvalid > 0);
+    if (lane == 0) s->opening = 0;
 }
 
 // GomokuGame.reset() on a GState (game.py:8-11).
 __device__ __forceinline__ void game_reset(const Params &p, GState *s, int lane)
 {
-    if (lane < GMZ_WORDS) {
-        u64 v = 0;
-        const int lo = 64 * lane;
-        if (lo < p.A) v = (p.A - lo >= 64) ? ~0ull : ((1ull << (p.A - lo)) - 1ull);
-        s->p1[lane] = 0; s->m1[lane] = 0; s->valid[lane] = v;
-    }
-    if (lane == 0) {
-        s->to_move = 1; s->last_move = -1; s->move_count = 0; s->active = 1;
-        s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
-        s->winner = GMZ_WINNER_NONE; s->traj_len = 0; s->parked = 0;
-    }
+    u64 v = 0;
+    const int lo = 64 * lane;
+    if (lo < p.A) v = (p.A - lo >= 64) ? ~0ull : ((1ull << (p.A - lo)) - 1ull);
+    root_write(s, lane, 0ull, 0ull, v, 1, -1, 0, true);
 }
 
 // A new self-play game for game g: its k-th deal since the book was bound (k = s->deals) takes opening (k*G + g) mod O,
 // so the games of an index depend on g and k only, not on which warp or launch deals them.  Without a book: the empty
-// board, labelled "none".  Every lane takes part (root_load ballots).
-__device__ __forceinline__ void game_deal(const Params &p, const BookDev &b, GState *s, int g, int lane)
+// board, labelled "none".  Every lane takes part (root_load ballots).  Out of line: in the play kernel a deal is rare next
+// to the simulations, and its code stays out of the simulation loop's instruction stream and registers.  Callers pass
+// __grid_constant__ kernel parameters: a by-value Params would be copied to a 360-byte stack frame for every call.
+static __device__ __noinline__ void game_deal(const Params &p, const BookDev &b, GState *s, int g, int lane)
 {
     const unsigned k = s->deals;
     int label = 0;

@@ -24,7 +24,6 @@ struct gmz_engine {
     size_t bytes;
     void *workspace;
     BookDev book;            // the bound opening book (n == 0: none)
-    int book_ever;           // a book has been bound at some point: self-play launches the play kernel's book variant
 };
 #define GMZ_ENGINE_MAGIC 0x474d5a32u
 
@@ -32,14 +31,9 @@ struct gmz_engine {
 int gmz_fail(const char *fmt, const char *a = "");
 int gmz_check_launch(const char *what);
 
-// ticketed persistent play kernel, one translation unit per (MuZero mode, float32 accumulation, book variant): _b1 deals
-// from a.book and labels each recorded game with its opening
+// ticketed persistent play kernel, one translation unit per (MuZero mode, float32 accumulation)
 struct PlayArgs;
-int gmz_launch_play_mz0_f0_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz0_f1_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz1_f0_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz1_f1_b0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz0_f0_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz0_f1_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz1_f0_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
-int gmz_launch_play_mz1_f1_b1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz0_f0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz0_f1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz1_f0(gmz_engine *e, const PlayArgs &a, cudaStream_t st);
+int gmz_launch_play_mz1_f1(gmz_engine *e, const PlayArgs &a, cudaStream_t st);

@@ -57,18 +57,6 @@ k_match_noise(int G, int A, gmz_match m, u64 seed_mixed, double *gum_a, double *
     }
 }
 
-// The root fields of a game that changes engines (what root_load writes, from bitboards instead of an int8 board).
-__device__ __forceinline__ void root_store(GState *s, int lane, u64 P, u64 M, u64 V, int to_move, int last_move, int move_count)
-{
-    const bool any = __any_sync(GMZ_FULL, lane < GMZ_WORDS && V != 0ull);
-    if (lane < GMZ_WORDS) { s->p1[lane] = P; s->m1[lane] = M; s->valid[lane] = V; }
-    if (lane == 0) {
-        s->to_move = to_move; s->last_move = last_move; s->move_count = move_count; s->active = any;
-        s->sim_count = 0; s->num_nodes = 0; s->leaf_depth = 0; s->n_surv = 0; s->n_init = 0;
-        s->winner = GMZ_WINNER_NONE;
-    }
-}
-
 __global__ void __launch_bounds__(MATCH_THREADS)
 k_match_step(Params pa, Params pb, gmz_match m, const int32_t *act_a, const int32_t *act_b)
 {
@@ -109,7 +97,8 @@ k_match_step(Params pa, Params pb, gmz_match m, const int32_t *act_a, const int3
         const Params &p = q ? pb : pa;
         const int src = 1 - q;
         if (!live[src]) { slot_deal(p, m, q, g, lane); continue; }
-        root_store(p.gs + g, lane, P[src], M[src], V[src], tm[src], lm[src], mc[src]);
+        root_write(p.gs + g, lane, P[src], M[src], V[src], tm[src], lm[src], mc[src],
+                   __any_sync(GMZ_FULL, lane < GMZ_WORDS && V[src] != 0ull));
         if (lane == 0) { m.slot_ticket[(size_t)q * G + g] = tk[src]; m.slot_ply[(size_t)q * G + g] = ply[src]; }
     }
 }

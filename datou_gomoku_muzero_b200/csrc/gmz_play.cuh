@@ -188,15 +188,82 @@ struct PlayArgs {
     double *out_policy; double *out_value; int32_t *out_action; int32_t *out_visits;   // search-only outputs
     int32_t *trace_a, *trace_d;   // [G][S] leaf action / depth per evaluation (search-only, optional)
     TrajDev traj;
-    BookDev book;         // self-play deals (book variant of k_play_e0 only)
+    BookDev book;         // self-play deals (game_deal)
 };
 
+// The self-play move commit (workers.py:172-189), shared by k_play_e0, k_selfplay_step and k_unpark.  Each caller
+// writes the move's policy row itself; to_move / last_move are the root's, passed in by the caller.
+
+// First recorded move of the game in `slot`: remember the position it started from and its opening label.
+__device__ __forceinline__ void traj_open(const TrajDev &t, const GState *s, int slot, int g, int to_move, int last_move,
+                                          int lane)
+{
+    if (lane < GMZ_WORDS) {
+        t.start_board[((size_t)slot * 2 + 0) * GMZ_WORDS + lane] = s->p1[lane];
+        t.start_board[((size_t)slot * 2 + 1) * GMZ_WORDS + lane] = s->m1[lane];
+    }
+    if (lane == 0) {
+        int32_t *si = t.start_info + (size_t)slot * 4;
+        si[0] = to_move; si[1] = s->move_count; si[2] = last_move; si[3] = g;
+        if (t.start_opening) t.start_opening[slot] = s->opening;
+    }
+}
+
+// Record value and action as move tl of `slot` (moves past max_moves are played, not recorded), play the move and count
+// it.  Returns game_do_move's winner.
+__device__ __forceinline__ int move_commit(const Params &p, const TrajDev &t, GState *s, int use_traj, int slot, int tl,
+                                           double value, int action, int lane)
+{
+    if (use_traj && lane == 0 && tl < t.max_moves) {
+        t.value[(size_t)slot * t.max_moves + tl] = value;
+        t.action[(size_t)slot * t.max_moves + tl] = action;
+    }
+    __syncwarp();
+    const int wv = game_do_move(p, s, action, lane);
+    if (lane == 0) {
+        s->noise_ctr += 1; s->traj_len = tl + 1;
+        atomicAdd(&p.ctl->moves_played, 1ull);
+    }
+    return wv;
+}
+
+// Pop a free trajectory slot (lane 0); false when the free stack is empty.
 __device__ __forceinline__ bool traj_pop_slot(const TrajDev &t, int &slot)
 {
     const int idx = atomicSub(t.free_top, 1) - 1;
     if (idx < 0) { atomicAdd(t.free_top, 1); return false; }
     slot = t.free_slots[idx];
     return true;
+}
+
+// Deal game g a new game, recorded into `slot` when there is a store.
+__device__ __forceinline__ void game_redeal(const Params &p, const BookDev &b, GState *s, int g, int use_traj, int slot, int lane)
+{
+    game_deal(p, b, s, g, lane);
+    if (lane == 0 && use_traj) s->traj_slot = slot;
+}
+
+// Game g has ended (winner wv after len moves): hand its slot to the host through the finish queue, then deal it a new
+// game if `restart` and a free slot allow.  Otherwise it parks with a store (k_unpark deals it once slots are released)
+// and stays finished without one.  A full finish queue drops the row and parks the game.
+__device__ __forceinline__ void game_finish(const Params &p, const TrajDev &t, const BookDev &b, GState *s, int g,
+                                            int use_traj, int restart, int slot, int len, int wv, int lane)
+{
+    int ok = 1, nslot = -1;
+    if (lane == 0) {
+        atomicAdd(&p.ctl->games_finished, 1ull);
+        if (use_traj) {
+            const int qi = atomicAdd(t.fin_count, 1);
+            if (qi < t.fin_cap) { int32_t *q = t.fin_queue + (size_t)qi * 4; q[0] = slot; q[1] = g; q[2] = len; q[3] = wv; }
+            ok = (qi < t.fin_cap) && restart && traj_pop_slot(t, nslot);
+            if (qi >= t.fin_cap) atomicSub(t.fin_count, 1);
+        } else ok = restart;
+    }
+    ok = __shfl_sync(GMZ_FULL, ok, 0);
+    nslot = __shfl_sync(GMZ_FULL, nslot, 0);
+    __syncwarp();
+    if (ok) game_redeal(p, b, s, g, use_traj, nslot, lane);
+    else if (lane == 0) s->parked = use_traj ? 1 : 0;
 }
 
 struct PlayArgs;
@@ -240,18 +307,9 @@ __device__ __noinline__ u64 play_root(const Params &p, const PlayArgs &a, WG &w,
     return h;
 }
 
-// The book variant's deal (game_deal), out of line like play_root: a restart is rare next to the simulations, and its
-// code stays out of the simulation loop's instruction stream and registers.
-static __device__ __noinline__ void play_deal(const Params &p, const BookDev &b, GState *s, int g, int lane)
-{
-    game_deal(p, b, s, g, lane);
-}
-
 // One search (mcts.py:197-280) -- and in self-play mode one whole move (workers.py:168-189) --
-// per ticket, one game per warp, E0 inlined.  BOOK: self-play deals through play_deal from the bound opening book and
-// records each game's opening label; the launcher takes it once a book has ever been bound on the engine, and the
-// default variant (BOOK = false) is the kernel as it was before books existed.
-template <int NC, bool MZ, bool F32, bool BOOK>
+// per ticket, one game per warp, E0 inlined.
+template <int NC, bool MZ, bool F32>
 __global__ void __launch_bounds__(32 * GMZ_PLAY_WARPS, GMZ_PLAY_MIN_CTAS)
 k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
 {
@@ -304,8 +362,7 @@ k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
         int2 *path = p.path + (size_t)g * (p.S + 2);    // descent path past depth 31 (rare)
 
         if (a.do_step && s->winner != GMZ_WINNER_NONE) {   // finished earlier, could not restart then
-            if constexpr (BOOK) play_deal(p, a.book, s, g, lane);
-            else game_reset(p, s, lane);
+            game_deal(p, a.book, s, g, lane);
             __syncwarp();
         }
         WG &w = s_wg[wi];
@@ -368,17 +425,7 @@ k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
         if (a.do_step) {
             if (a.use_traj) {
                 slot = s->traj_slot; tl = s->traj_len;
-                if (tl == 0 && w.active) {     // first recorded move of this game: remember where it started
-                    if (lane < GMZ_WORDS) {
-                        a.traj.start_board[((size_t)slot * 2 + 0) * GMZ_WORDS + lane] = s->p1[lane];
-                        a.traj.start_board[((size_t)slot * 2 + 1) * GMZ_WORDS + lane] = s->m1[lane];
-                    }
-                    if (lane == 0) {
-                        int32_t *si = a.traj.start_info + (size_t)slot * 4;
-                        si[0] = w.to_move; si[1] = s->move_count; si[2] = w.last_move; si[3] = g;
-                        if constexpr (BOOK) { if (a.traj.start_opening) a.traj.start_opening[slot] = s->opening; }
-                    }
-                }
+                if (tl == 0 && w.active) traj_open(a.traj, s, slot, g, w.to_move, w.last_move, lane);
                 if (tl < a.traj.max_moves) pol = a.traj.policy + ((size_t)slot * a.traj.max_moves + tl) * (size_t)p.A;
             }
         } else {
@@ -391,39 +438,8 @@ k_play_e0(const __grid_constant__ Params p, const __grid_constant__ PlayArgs a)
         } else if (action < 0) {
             if (lane == 0) atomicAdd(&p.ctl->tickets_idle, 1ull);
         } else {
-            if (a.use_traj && lane == 0 && tl < a.traj.max_moves) {
-                a.traj.value[(size_t)slot * a.traj.max_moves + tl] = value;
-                a.traj.action[(size_t)slot * a.traj.max_moves + tl] = action;
-            }
-            __syncwarp();
-            const int wv = game_do_move(p, s, action, lane);
-            if (lane == 0) {
-                s->noise_ctr += 1; s->traj_len = tl + 1;
-                atomicAdd(&p.ctl->moves_played, 1ull);
-            }
-            if (wv != GMZ_WINNER_NONE) {      // game over: hand the trajectory to the host, restart
-                int ok = 1, nslot = -1;
-                if (lane == 0) {
-                    atomicAdd(&p.ctl->games_finished, 1ull);
-                    if (a.use_traj) {
-                        const int qi = atomicAdd(a.traj.fin_count, 1);
-                        if (qi < a.traj.fin_cap) {
-                            int32_t *q = a.traj.fin_queue + (size_t)qi * 4;
-                            q[0] = slot; q[1] = g; q[2] = tl + 1; q[3] = wv;
-                        }
-                        ok = (qi < a.traj.fin_cap) && a.restart && traj_pop_slot(a.traj, nslot);
-                        if (qi >= a.traj.fin_cap) atomicSub(a.traj.fin_count, 1);
-                    } else ok = a.restart;
-                }
-                ok = __shfl_sync(GMZ_FULL, ok, 0);
-                nslot = __shfl_sync(GMZ_FULL, nslot, 0);
-                __syncwarp();
-                if (ok) {
-                    if constexpr (BOOK) play_deal(p, a.book, s, g, lane);
-                    else game_reset(p, s, lane);
-                    if (lane == 0 && a.use_traj) s->traj_slot = nslot;
-                } else if (lane == 0) s->parked = a.use_traj ? 1 : 0;
-            }
+            const int wv = move_commit(p, a.traj, s, a.use_traj, slot, tl, value, action, lane);
+            if (wv != GMZ_WINNER_NONE) game_finish(p, a.traj, a.book, s, g, a.use_traj, a.restart, slot, tl + 1, wv, lane);
         }
         __syncwarp();
         __threadfence();                    // release

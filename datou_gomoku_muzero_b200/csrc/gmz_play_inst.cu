@@ -1,26 +1,24 @@
-// gmz_play_inst.cu -- one instantiation family of the persistent play kernel k_play_e0<NC, MZ, F32, BOOK>.
-// Compiled eight times (-DGMZ_PLAY_MZ=0|1 -DGMZ_PLAY_F32=0|1 -DGMZ_PLAY_BOOK=0|1) so the big kernels build in parallel.
-// The book variants get translation units of their own: next to a BOOK = true instantiation, ptxas allocates the
-// shared out-of-line helpers (play_root, finalize_root, ...) differently and the default kernel's code changes.
+// gmz_play_inst.cu -- one instantiation family of the persistent play kernel k_play_e0<NC, MZ, F32>.
+// Compiled four times (-DGMZ_PLAY_MZ=0|1 -DGMZ_PLAY_F32=0|1) so the big kernels build in parallel.
 #include "gmz_internal.h"
 #include "gmz_tree.cuh"
 #include "gmz_play.cuh"
 
-#if !defined(GMZ_PLAY_MZ) || !defined(GMZ_PLAY_F32) || !defined(GMZ_PLAY_BOOK)
-#error "compile with -DGMZ_PLAY_MZ=0|1 -DGMZ_PLAY_F32=0|1 -DGMZ_PLAY_BOOK=0|1"
+#if !defined(GMZ_PLAY_MZ) || !defined(GMZ_PLAY_F32)
+#error "compile with -DGMZ_PLAY_MZ=0|1 -DGMZ_PLAY_F32=0|1"
 #endif
-#define GMZ_CAT_(a, b, c, d, e, f) a##b##c##d##e##f
-#define GMZ_CAT(a, b, c, d, e, f) GMZ_CAT_(a, b, c, d, e, f)
-#define GMZ_LAUNCH_NAME GMZ_CAT(gmz_launch_play_mz, GMZ_PLAY_MZ, _f, GMZ_PLAY_F32, _b, GMZ_PLAY_BOOK)
+#define GMZ_CAT_(a, b, c, d) a##b##c##d
+#define GMZ_CAT(a, b, c, d) GMZ_CAT_(a, b, c, d)
+#define GMZ_LAUNCH_NAME GMZ_CAT(gmz_launch_play_mz, GMZ_PLAY_MZ, _f, GMZ_PLAY_F32)
 
 // grid = what fits on the GPU at once (persistent), capped by the game count.  The occupancy is a
-// property of (device, NC) for this translation unit's (MZ, F32, BOOK): cached per device, filled under a mutex.
+// property of (device, NC) for this translation unit's (MZ, F32): cached per device, filled under a mutex.
 #include <mutex>
 #include <stdlib.h>
 template <int NC>
 static int launch_t(gmz_engine *e, const PlayArgs &a, cudaStream_t st)
 {
-    constexpr bool MZ = GMZ_PLAY_MZ != 0, F32 = GMZ_PLAY_F32 != 0, BOOK = GMZ_PLAY_BOOK != 0;
+    constexpr bool MZ = GMZ_PLAY_MZ != 0, F32 = GMZ_PLAY_F32 != 0;
     static std::mutex mu;
     static int cache[64];                    // resident CTAs per device ordinal, 0 = unknown
     int dev = 0;
@@ -32,7 +30,7 @@ static int launch_t(gmz_engine *e, const PlayArgs &a, cudaStream_t st)
         if (!resident) {
             int occ = 0, sms = 0;
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_play_e0<NC, MZ, F32, BOOK>, 32 * GMZ_PLAY_WARPS, 0);
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_play_e0<NC, MZ, F32>, 32 * GMZ_PLAY_WARPS, 0);
             resident = (occ > 0 ? occ : 1) * (sms > 0 ? sms : 148);
             if (dev >= 0 && dev < 64) cache[dev] = resident;
         }
@@ -41,7 +39,7 @@ static int launch_t(gmz_engine *e, const PlayArgs &a, cudaStream_t st)
     if (grid > resident) grid = resident;
     if (const char *cap = getenv("GMZ_PLAY_GRID_CAP")) { const int c = atoi(cap); if (c > 0 && c < grid) grid = c; }   // development: occupancy sweeps
     if (cudaMemsetAsync(&e->p.ctl->next_ticket, 0, 2 * sizeof(unsigned long long), st) != cudaSuccess) return gmz_fail("cudaMemsetAsync(ctl)");
-    k_play_e0<NC, MZ, F32, BOOK><<<grid, 32 * GMZ_PLAY_WARPS, 0, st>>>(e->p, a);
+    k_play_e0<NC, MZ, F32><<<grid, 32 * GMZ_PLAY_WARPS, 0, st>>>(e->p, a);
     return gmz_check_launch("k_play_e0");
 }
 

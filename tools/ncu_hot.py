@@ -8,7 +8,7 @@ rep, sims = sys.argv[1], float(sys.argv[2])
 kern = sys.argv[3] if len(sys.argv) > 3 else "_Z9k_play_e0ILi2ELb0ELb0EEv6Params8PlayArgs"
 # the four play-kernel cubins inside libgmz.so share one file name, so read the object of the instantiation instead
 so = sys.argv[4] if len(sys.argv) > 4 else os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "datou_gomoku_muzero_b200",
-                                                       "build", "release", "gmz_play_mz0_f0_b0.o")
+                                                       "build", "release", "gmz_play_mz0_f0.o")
 tmp = tempfile.mkdtemp()
 subprocess.run(["cuobjdump", "-xelf", "all", os.path.abspath(so)], cwd=tmp, capture_output=True)
 dis, start = [], None

@@ -1,13 +1,13 @@
-"""Check that the default persistent play kernel compiles to the same machine code as at another commit.
+"""Check that the persistent play kernel compiles to the same machine code as at another commit.
 
     python tools/play_sass_diff.py [REV]        (default REV: HEAD~1)
 
 Builds gmz_play_inst.cu of REV (from `git archive`) and of the working tree into a temporary directory, with
-_build.NVCC_FLAGS and -Xptxas -v, for every (MZ, F32) pair; the working tree also for GMZ_PLAY_BOOK=1.  Every
-k_play_e0 instantiation of REV is matched with the working tree's one of the same NC / MZ / F32 and BOOK = false (a
-REV kernel without the BOOK parameter matches that one too); their `cuobjdump -sass` bodies are compared without the
-mangled names, and ptxas's registers, stack and spill bytes of both are printed and compared.  The book variants'
-ptxas figures are printed too.  Exit status 1 on any difference.  Needs nvcc and cuobjdump, no GPU."""
+_build.NVCC_FLAGS and -Xptxas -v, for every (MZ, F32) pair.  Every k_play_e0<NC, MZ, F32> of the working tree is matched
+with REV's one of the same NC / MZ / F32 (a REV that still has the opening-book parameter is built with
+-DGMZ_PLAY_BOOK=1 and its BOOK = true kernel is the match); their `cuobjdump -sass` bodies are compared without the
+mangled names, and ptxas's registers, stack and spill bytes of both are printed and compared.  Exit status 1 on any
+difference.  Needs nvcc and cuobjdump, no GPU."""
 from __future__ import annotations
 
 import os
@@ -59,19 +59,20 @@ def ptxas_props(text):
 
 
 def kernels(obj, log):
-    """(NC, MZ, F32, BOOK) -> (sass body, ptxas figures) of the k_play_e0 instantiations in one object."""
+    """(NC, MZ, F32) -> (sass body, ptxas figures) of the k_play_e0 instantiations in one object (BOOK = true only, where
+    the kernel still has that parameter)."""
     props = ptxas_props(log)
     out = {}
     for name, body in sass_functions(obj).items():
         m = KERNEL.fullmatch(name)
-        if m:
-            out[(int(m.group(1)), int(m.group(2)), int(m.group(3)), int(m.group(4) or 0))] = (body, props.get(name))
+        if m and m.group(4) != "0":
+            out[(int(m.group(1)), int(m.group(2)), int(m.group(3)))] = (body, props.get(name))
     return out
 
 
-def compile_obj(src_root, mz, f32, book, out):
+def compile_obj(src_root, mz, f32, out):
     cmd = [os.path.join(CUDA, "bin", "nvcc"), *NVCC_FLAGS, "-Xptxas", "-v", f"-DGMZ_PLAY_MZ={mz}", f"-DGMZ_PLAY_F32={f32}",
-           f"-DGMZ_PLAY_BOOK={book}", "-c", os.path.join(src_root, "datou_gomoku_muzero_b200", "csrc", "gmz_play_inst.cu"),
+           "-DGMZ_PLAY_BOOK=1", "-c", os.path.join(src_root, "datou_gomoku_muzero_b200", "csrc", "gmz_play_inst.cu"),
            "-o", out]
     r = subprocess.run(cmd, check=True, capture_output=True, text=True)
     return out, r.stdout + r.stderr
@@ -84,37 +85,26 @@ def main(rev):
         tar = subprocess.run(["git", "-C", ROOT, "archive", rev, "datou_gomoku_muzero_b200/csrc", "include"], check=True,
                              capture_output=True).stdout
         subprocess.run(["tar", "x", "-C", old_root], input=tar, check=True)
-        jobs = []
-        for mz in (0, 1):
-            for f in (0, 1):
-                jobs.append(("old", mz, f, 0, old_root))
-                jobs.append(("new", mz, f, 0, ROOT))
-                jobs.append(("new", mz, f, 1, ROOT))
+        jobs = [(side, mz, f, src) for mz in (0, 1) for f in (0, 1) for side, src in (("old", old_root), ("new", ROOT))]
         with ThreadPoolExecutor(max_workers=min(len(jobs), os.cpu_count() or 4)) as ex:
-            res = list(ex.map(lambda j: compile_obj(j[4], j[1], j[2], j[3], os.path.join(tmp, f"{j[0]}_mz{j[1]}_f{j[2]}_b{j[3]}.o")),
-                              jobs))
+            res = list(ex.map(lambda j: compile_obj(j[3], j[1], j[2], os.path.join(tmp, f"{j[0]}_mz{j[1]}_f{j[2]}.o")), jobs))
         found = {}
         for (side, *_), (obj, log) in zip(jobs, res):
             for k, v in kernels(obj, log).items():
                 found[(side,) + k] = v
     bad = 0
-    for (side, nc, mz, f, book), (body, props) in sorted(found.items()):
-        if side != "old":
+    for (side, nc, mz, f), (body, props) in sorted(found.items()):
+        if side != "new":
             continue
-        new = found.get(("new", nc, mz, f, 0))
-        if new is None:
-            print(f"NC={nc} MZ={mz} F32={f}: no default kernel in the working tree")
+        old = found.get(("old", nc, mz, f))
+        if old is None:
+            print(f"NC={nc} MZ={mz} F32={f}: no kernel at {rev}")
             bad = 1
             continue
-        same = body == new[0] and props == new[1]
-        print(f"NC={nc} MZ={mz} F32={f} BOOK=0: {len(body)} SASS lines {'identical' if body == new[0] else 'DIFFERENT'}; "
-              f"ptxas (registers, stack, spill stores, spill loads) {props} -> {new[1]}")
-        bad |= not same
-    for (side, nc, mz, f, book), (body, props) in sorted(found.items()):
-        if side == "new" and book:
-            print(f"NC={nc} MZ={mz} F32={f} BOOK=1: {len(body)} SASS lines; ptxas {props}")
+        print(f"NC={nc} MZ={mz} F32={f}: {len(body)} SASS lines {'identical' if body == old[0] else 'DIFFERENT'}; "
+              f"ptxas (registers, stack, spill stores, spill loads) {old[1]} -> {props}")
+        bad |= body != old[0] or props != old[1]
     return bad
-
 
 if __name__ == "__main__":
     if len(sys.argv) > 2:
