@@ -9,7 +9,8 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libgmz.so")
-SOURCES = ["gmz_engine.cu", "gmz_per.cu", "gmz_tactics.cu", "gmz_hidden.cu", "gmz_records.cu", "gmz_match.cu", "gmz_inspect.cu"]
+SOURCES = ["gmz_engine.cu", "gmz_per.cu", "gmz_tactics.cu", "gmz_hidden.cu", "gmz_records.cu", "gmz_match.cu", "gmz_inspect.cu",
+           "gmz_vcf.cu"]
 # the persistent play kernel: one object per (MuZero mode, float32 accumulation), built in parallel
 PLAY_SOURCE = "gmz_play_inst.cu"
 PLAY_VARIANTS = [(mz, f32) for mz in (0, 1) for f32 in (0, 1)]

@@ -113,6 +113,23 @@ def random_openings(n, stones, board_size=15, seed=0, n_in_row=5):
     return Openings(boards, players, last, np.full(n, stones, np.int32))
 
 
+def opening_vcf(book, max_attacks=8, node_budget=20_000, n_in_row=5, board_size=None):
+    """Which openings of a book are already decided by a forced win (tactics.find_vcf on the GPU): int32 arrays
+    (mover [O], opponent [O]) = the VCF length of the side to move, and the length the other side would have if it were
+    to move (0: none within `max_attacks` stones, -1: the node budget ran out).  A balanced book keeps
+    `(mover == 0) & (opponent == 0)`."""
+    from .tactics import find_vcf
+    boards, players = np.asarray(book.boards), np.asarray(book.players)
+    O = boards.shape[0]
+    N = int(board_size) if board_size else (boards.shape[1] if boards.ndim == 3 else int(round(math.sqrt(boards.shape[1]))))
+    boards = np.ascontiguousarray(boards.reshape(O, N * N), np.int8)
+    side = np.where(players >= 0, 1, -1).astype(np.int8)
+    length, _, _ = find_vcf(np.concatenate([boards, boards]), np.concatenate([side, -side]), max_attacks, node_budget,
+                            n_in_row=n_in_row, board_size=N)
+    length = length.cpu().numpy()
+    return length[:O], length[O:]
+
+
 def elo_of(score):
     """Elo difference of an expected score: -400 log10(1/s - 1), -inf / +inf at 0 / 1."""
     if score <= 0.0:

@@ -1,6 +1,8 @@
 """Tactical move classifier on the device (reference workers.py:49-123) and the missed-win statistics
 built on it (workers.py:191-203): per host GameRecord (`missed_win_stats`), and straight from the packed move
-records of device self-play (`missed_win_counts`, `SelfPlayStats`)."""
+records of device self-play (`missed_win_counts`, `SelfPlayStats`).  Forced wins beyond the next stone: the VCF
+solver (`find_vcf`) and the missed-VCF statistics built on it (`vcf_record_flags`, `missed_vcf_counts`,
+`SelfPlayStats(vcf_attacks=k)`)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -100,6 +102,18 @@ def missed_win_counts(packed, n_in_row=None):
     [len(packed), 2] on the device, the counts `missed_win_stats` gives for `packed.game_record(i)` (one kernel over all
     records and one reduction, no loop over games).  Records held on the host (e.g. gathered over gloo) are copied
     to the current device once."""
+    rec, game = _game_records(packed)
+    out = torch.zeros((len(packed), 2), dtype=torch.int64, device=rec.device)
+    if rec.shape[0] == 0:
+        return out
+    fives, missed = _missed(record_flags(rec, packed.N, n_in_row))
+    out.index_add_(0, game, torch.stack([fives, missed], dim=1).to(torch.int64))
+    return out
+
+
+def _game_records(packed):
+    """(the records of every game of a trajectory.PackedGames on the current device -- host records are copied there
+    once --, the game index of each record int64 [M])."""
     dev = torch.device(f"cuda:{torch.cuda.current_device()}")
     off = np.asarray(packed.offsets, np.int64)
     n, M = len(packed), int(off[-1] - off[0])
@@ -107,14 +121,77 @@ def missed_win_counts(packed, n_in_row=None):
     if rec.device.type != "cuda":
         rec = rec.to(dev)
     rec = rec.reshape(-1, int(_lib.load().gmz_move_record_bytes(packed.N)))[int(off[0]):int(off[-1])]
-    out = torch.zeros((n, 2), dtype=torch.int64, device=rec.device)
-    if M == 0:
-        return out
-    fives, missed = _missed(record_flags(rec, packed.N, n_in_row))
     # record -> game from the offsets (the header's game_seq restarts on every rank, so it repeats after a gather)
     game = torch.repeat_interleave(torch.arange(n, device=rec.device), torch.as_tensor(np.diff(off), device=rec.device),
                                    output_size=M)
-    out.index_add_(0, game, torch.stack([fives, missed], dim=1).to(torch.int64))
+    return rec, game
+
+
+# Forced wins: the VCF solver (include/gmz.h gmz_vcf_solve states the definition, the visiting order and the budget).
+VCF_ATTACKS, VCF_BUDGET = 8, 20_000
+# Bits of the per-record flags gmz_records_vcf writes.
+VCF_AVAILABLE, PLAYED_VCF, VCF_UNKNOWN = 1, 2, 4
+
+
+def find_vcf(boards, players, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None, board_size=None,
+             device=None):
+    """Forced wins by continuous fours for the side to move.  boards int8 [B,N,N] or [B,A], players +-1 [B] -> device
+    tensors (length int32 [B], first bool [B,A], nodes int32 [B]): the fewest attacker stones of a VCF of at most
+    `max_attacks` stones (0: none, -1: the node budget ran out), every first move that starts one, and the positions
+    expanded."""
+    if not torch.cuda.is_available():
+        raise _lib.GmzError("find_vcf needs a CUDA device (there is no CPU fallback)")
+    lib = _lib.load()
+    dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    b = torch.as_tensor(boards).to(device=dev, dtype=torch.int8)
+    B = b.shape[0]
+    N = board_size or (b.shape[1] if b.dim() == 3 else int(round(b.shape[1] ** 0.5)))
+    A = N * N
+    b = b.reshape(B, A).contiguous()
+    p = torch.as_tensor(players).to(device=dev, dtype=torch.int8).reshape(B).contiguous()
+    length = torch.empty(B, dtype=torch.int32, device=dev)
+    nodes = torch.empty(B, dtype=torch.int32, device=dev)
+    first = torch.empty((B, 6), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.gmz_vcf_solve(C.c_void_p(b.data_ptr()), C.c_void_p(p.data_ptr()), B, N,
+                                int(config.N_IN_ROW if n_in_row is None else n_in_row), int(max_attacks), int(node_budget),
+                                C.c_void_p(length.data_ptr()), C.c_void_p(first.data_ptr()), C.c_void_p(nodes.data_ptr()),
+                                C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "gmz_vcf_solve")
+    bits = (first.unsqueeze(-1) >> torch.arange(64, device=dev)) & 1
+    return length, bits.reshape(B, 6 * 64)[:, :A].bool(), nodes
+
+
+def vcf_record_flags(records, board_size, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None):
+    """The VCF twin of record_flags: packed move records (uint8 device tensor [M, stride], a trajectory.PackedGames
+    block or a stretch of the DeviceReplayBuffer ring) solved where they lie for the side in each record's to_move ->
+    uint8 [M] (bits VCF_AVAILABLE, PLAYED_VCF = the played action starts a VCF, VCF_UNKNOWN = the budget ran out)."""
+    lib = _lib.load()
+    N = int(board_size)
+    stride = int(lib.gmz_move_record_bytes(N))
+    if not torch.is_tensor(records) or records.device.type != "cuda":
+        raise _lib.GmzError("vcf_record_flags needs the records in a CUDA tensor (there is no CPU fallback)")
+    if records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != stride or not records.is_contiguous():
+        raise ValueError(f"records must be a contiguous uint8 tensor [M, {stride}] of {N}x{N} move records")
+    M = int(records.shape[0])
+    out = torch.empty(M, dtype=torch.uint8, device=records.device)
+    if M == 0:
+        return out
+    with torch.cuda.device(records.device):
+        check(lib.gmz_records_vcf(C.c_void_p(records.data_ptr()), M, N, int(config.N_IN_ROW if n_in_row is None else n_in_row),
+                                  int(max_attacks), int(node_budget), C.c_void_p(out.data_ptr()),
+                                  C.c_void_p(torch.cuda.current_stream(records.device).cuda_stream)), "gmz_records_vcf")
+    return out
+
+
+def missed_vcf_counts(packed, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None):
+    """Per game of a trajectory.PackedGames, in `packed.table` order: int64 [len(packed)] on the device, the moves at
+    which the mover had a VCF of at most `max_attacks` stones and played a move that does not start one."""
+    rec, game = _game_records(packed)
+    out = torch.zeros(len(packed), dtype=torch.int64, device=rec.device)
+    if rec.shape[0] == 0:
+        return out
+    flags = vcf_record_flags(rec, packed.N, max_attacks, node_budget, n_in_row)
+    out.index_add_(0, game, ((flags & (VCF_AVAILABLE | PLAYED_VCF)) == VCF_AVAILABLE).to(torch.int64))
     return out
 
 
@@ -127,9 +204,14 @@ class SelfPlayStats:
 
     n_openings = O > 0 also keeps, per opening of a self-play book (SearchEngine.set_openings), how often the side to
     move at the opening won, drew and lost, from each game's first record on the device; `by_opening()` reads them.
-    Games without a label in [0, O) count in the totals only."""
+    Games without a label in [0, O) count in the totals only.
 
-    def __init__(self, n_in_row=None, device=None, n_openings=0):
+    vcf_attacks = k > 0 also solves every record for forced wins of at most k attacker stones (gmz_records_vcf, at most
+    `vcf_budget` positions each) and adds to `summary()` the moves at which the mover had one (vcf_available), those
+    at which it played a move that starts none (missed_vcf, and missed_vcf_per_game) and the records the budget left
+    undecided (vcf_unknown).  0 leaves the statistics and the summary's keys as they are without it."""
+
+    def __init__(self, n_in_row=None, device=None, n_openings=0, vcf_attacks=0, vcf_budget=VCF_BUDGET):
         if not torch.cuda.is_available():
             raise _lib.GmzError("SelfPlayStats needs a CUDA device (there is no CPU fallback)")
         self.n_in_row = n_in_row
@@ -137,12 +219,17 @@ class SelfPlayStats:
         self._missed = torch.zeros(2, dtype=torch.int64, device=self.device)      # missed fives, missed wins
         self.n_openings = int(n_openings)
         self._by_opening = torch.zeros((self.n_openings, 3), dtype=torch.int64, device=self.device)
+        self.vcf_attacks, self.vcf_budget = int(vcf_attacks), int(vcf_budget)
+        if self.vcf_attacks < 0:
+            raise ValueError("vcf_attacks must be >= 0")
+        self._vcf = torch.zeros(3, dtype=torch.int64, device=self.device)        # available, missed, unknown
         self.reset()
 
     def reset(self):
         self.games = self.moves = self.wins_black = self.wins_white = self.draws = 0
         self._missed.zero_()
         self._by_opening.zero_()
+        self._vcf.zero_()
 
     def add(self, packed):
         """Count the games of a trajectory.PackedGames whose records are on this device.  Launches one kernel and a
@@ -161,6 +248,10 @@ class SelfPlayStats:
             return
         fives, missed = _missed(record_flags(packed.records[:M], packed.N, self.n_in_row))
         self._missed += torch.stack([fives.sum(), missed.sum()])
+        if self.vcf_attacks:
+            f = vcf_record_flags(packed.records[:M], packed.N, self.vcf_attacks, self.vcf_budget, self.n_in_row)
+            self._vcf += torch.stack([(f & VCF_AVAILABLE).bool().sum(), ((f & (VCF_AVAILABLE | PLAYED_VCF)) == VCF_AVAILABLE).sum(),
+                                      (f & VCF_UNKNOWN).bool().sum()])
         if self.n_openings:
             # first record of each game: winner, to_move and opening label + 1, int32 columns of its header
             first = torch.as_tensor(np.asarray(packed.offsets[:-1], np.int64), device=self.device)
@@ -180,7 +271,12 @@ class SelfPlayStats:
         """dict of the counts plus avg_game_length and per-game rates (one device -> host copy)."""
         fives, missed = (int(x) for x in self._missed.tolist())
         g = self.games
-        return {"games": g, "moves": self.moves, "wins_black": self.wins_black, "wins_white": self.wins_white,
-                "draws": self.draws, "missed_fives": fives, "missed_all_wins": missed,
-                "avg_game_length": self.moves / g if g else 0.0,
-                "missed_fives_per_game": fives / g if g else 0.0, "missed_all_wins_per_game": missed / g if g else 0.0}
+        out = {"games": g, "moves": self.moves, "wins_black": self.wins_black, "wins_white": self.wins_white,
+               "draws": self.draws, "missed_fives": fives, "missed_all_wins": missed,
+               "avg_game_length": self.moves / g if g else 0.0,
+               "missed_fives_per_game": fives / g if g else 0.0, "missed_all_wins_per_game": missed / g if g else 0.0}
+        if self.vcf_attacks:
+            available, missed_vcf, unknown = (int(x) for x in self._vcf.tolist())
+            out.update(vcf_available=available, missed_vcf=missed_vcf, missed_vcf_per_game=missed_vcf / g if g else 0.0,
+                       vcf_unknown=unknown)
+        return out

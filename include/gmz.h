@@ -392,6 +392,37 @@ int gmz_records_expand(const void *headers, const double *policy, int64_t n, con
 int gmz_tactics_classify(const int8_t *boards, const int8_t *players, int batch, int board_size, int n_in_row,
                          int8_t *out_cls, gmz_stream stream);
 
+/* ---- forced wins: VCF (victory by continuous fours) solver ---- */
+/* Freestyle rules as game_do_move plays them: a run of >= n_in_row stones wins.  For a side X on a board, a COMPLETION
+ * CELL is an empty cell where an X stone would make such a run.  Attacker X is to move, Y defends; vcf(B, L) = "X wins
+ * with at most L attacker stones":
+ *   1. X has a completion cell: true (1 stone).  Else, if L <= 1: false.
+ *   2. Y has >= 2 completion cells: false.  Y has exactly one: X's only candidate is that cell, and only if it is a four
+ *      move.  Otherwise X's candidates are all its FOUR MOVES: empty cells m after which X has >= 1 completion cell.
+ *   3. Candidates m in ascending action order; C = X's completion cells after X plays m.  |C| >= 2: true (2 stones).
+ *      |C| = 1: Y is forced to play c in C; the branch fails if Y's stone at c completes a run for Y or the board is
+ *      then full; else the branch is vcf(B + X@m + Y@c, L - 1).  The first candidate that succeeds decides: true.
+ * Per position (side to move = X): length = the least L <= max_attacks with vcf true, 0 if none; first = bitmask u64[6]
+ * (bit a of word a/64) of every first move that starts a VCF of <= max_attacks stones: the completion cells if X has
+ * one, else the root candidates whose branch succeeds at some L <= max_attacks; nodes = positions expanded.
+ * VISITING ORDER (it fixes the node count, and with it where a budget cuts): the root is expanded (1 node); if rules 1-2
+ * do not decide it, its candidates are taken in ascending order and a |C| = 1 candidate's reply position is searched
+ * by iterative deepening, vcf(B', L - 1) for L = 2, 3, ... max_attacks, stopping at the first true or after an
+ * iteration in which no position was refused by "L <= 1" (a deeper one would search the same tree).  Each vcf() call
+ * expands one position, depth first, candidates ascending, and returns at its first success.  Before a position is
+ * expanded, nodes == node_budget cuts the search: length = -1, first empty, nodes = node_budget.
+ * Limits: 1 <= max_attacks <= 32, node_budget >= 1, n_in_row >= 1, 1 <= board_size <= GMZ_MAX_BOARD. */
+/* boards int8 [batch][A] (+1 / -1 / 0), players int8 [batch] (the side to move, >= 0 counts as +1) -> out_length int32
+ * [batch], out_first uint64 [batch][6], out_nodes int32 [batch].  One warp per position.  batch = 0 is a no-op. */
+int gmz_vcf_solve(const int8_t *boards, const int8_t *players, int batch, int board_size, int n_in_row, int max_attacks,
+                  int node_budget, int32_t *out_length, uint64_t *out_first, int32_t *out_nodes, gmz_stream stream);
+/* The same solver on n_records consecutive packed move records (a block or a stretch of the ring), read in place: the
+ * record's board for the side in its to_move.  out_flags uint8 [n_records] = bit 0: the mover had a VCF (length > 0),
+ * bit 1: the played action (outside [0, A): never) is in `first`, bit 2: the node budget was exhausted.  A missed VCF is
+ * bit 0 without bit 1.  n_records = 0 is a no-op. */
+int gmz_records_vcf(const void *records, int64_t n_records, int board_size, int n_in_row, int max_attacks, int node_budget,
+                    uint8_t *out_flags, gmz_stream stream);
+
 /* ---- prioritized replay: SumTree (replay_buffer.py:4-106) ------------------- */
 /* tree f64 [2*capacity-1] lives in caller memory, 1 <= capacity <= 2^32 (all three calls refuse
  * any other capacity before looking at n / batch).  Sequential reference semantics are preserved
