@@ -96,6 +96,8 @@ SIGNATURES = {
     "gmz_tactics_classify": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gmz_vcf_solve": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "gmz_records_vcf": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "gmz_vct_solve": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
+    "gmz_records_vct": (C.c_int, [_P, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gmz_per_update": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int, _P]),
     "gmz_per_add": (C.c_int, [_P, C.c_int64, C.c_int64, _P, C.c_int, _P, _P]),
     "gmz_per_sample": (C.c_int, [_P, C.c_int64, C.c_int64, _P, C.c_int, C.c_double, _P, _P, _P, _P]),

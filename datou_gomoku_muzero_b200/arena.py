@@ -113,21 +113,35 @@ def random_openings(n, stones, board_size=15, seed=0, n_in_row=5):
     return Openings(boards, players, last, np.full(n, stones, np.int32))
 
 
+def _opening_lengths(solve, book, max_attacks, node_budget, n_in_row, board_size):
+    """(mover [O], opponent [O]) int32: `solve`'s length for the side to move of each opening and for the other side."""
+    boards, players = np.asarray(book.boards), np.asarray(book.players)
+    O = boards.shape[0]
+    N = int(board_size) if board_size else (boards.shape[1] if boards.ndim == 3 else int(round(math.sqrt(boards.shape[1]))))
+    boards = np.ascontiguousarray(boards.reshape(O, N * N), np.int8)
+    side = np.where(players >= 0, 1, -1).astype(np.int8)
+    length, _, _ = solve(np.concatenate([boards, boards]), np.concatenate([side, -side]), max_attacks, node_budget,
+                         n_in_row=n_in_row, board_size=N)
+    length = length.cpu().numpy()
+    return length[:O], length[O:]
+
+
 def opening_vcf(book, max_attacks=8, node_budget=20_000, n_in_row=5, board_size=None):
     """Which openings of a book are already decided by a forced win (tactics.find_vcf on the GPU): int32 arrays
     (mover [O], opponent [O]) = the VCF length of the side to move, and the length the other side would have if it were
     to move (0: none within `max_attacks` stones, -1: the node budget ran out).  A balanced book keeps
     `(mover == 0) & (opponent == 0)`."""
     from .tactics import find_vcf
-    boards, players = np.asarray(book.boards), np.asarray(book.players)
-    O = boards.shape[0]
-    N = int(board_size) if board_size else (boards.shape[1] if boards.ndim == 3 else int(round(math.sqrt(boards.shape[1]))))
-    boards = np.ascontiguousarray(boards.reshape(O, N * N), np.int8)
-    side = np.where(players >= 0, 1, -1).astype(np.int8)
-    length, _, _ = find_vcf(np.concatenate([boards, boards]), np.concatenate([side, -side]), max_attacks, node_budget,
-                            n_in_row=n_in_row, board_size=N)
-    length = length.cpu().numpy()
-    return length[:O], length[O:]
+    return _opening_lengths(find_vcf, book, max_attacks, node_budget, n_in_row, board_size)
+
+
+def opening_vct(book, max_attacks=None, node_budget=None, n_in_row=5, board_size=None):
+    """opening_vcf through threats of three (tactics.find_vct, defaults VCT_ATTACKS / VCT_BUDGET): (mover [O],
+    opponent [O]) VCT lengths, 0 none, -1 the budget ran out.  It flags every opening opening_vcf decides where neither
+    search is cut, and the openings won by threes besides; a balanced book keeps `(mover == 0) & (opponent == 0)`."""
+    from .tactics import VCT_ATTACKS, VCT_BUDGET, find_vct
+    return _opening_lengths(find_vct, book, VCT_ATTACKS if max_attacks is None else max_attacks,
+                            VCT_BUDGET if node_budget is None else node_budget, n_in_row, board_size)
 
 
 def elo_of(score):

@@ -2,7 +2,8 @@
 built on it (workers.py:191-203): per host GameRecord (`missed_win_stats`), and straight from the packed move
 records of device self-play (`missed_win_counts`, `SelfPlayStats`).  Forced wins beyond the next stone: the VCF
 solver (`find_vcf`) and the missed-VCF statistics built on it (`vcf_record_flags`, `missed_vcf_counts`,
-`SelfPlayStats(vcf_attacks=k)`)."""
+`SelfPlayStats(vcf_attacks=k)`), and the VCT solver through threats of three (`find_vct`, `vct_record_flags`,
+`missed_vct_counts`) for offline use and samples."""
 from __future__ import annotations
 
 import ctypes as C
@@ -133,14 +134,10 @@ VCF_ATTACKS, VCF_BUDGET = 8, 20_000
 VCF_AVAILABLE, PLAYED_VCF, VCF_UNKNOWN = 1, 2, 4
 
 
-def find_vcf(boards, players, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None, board_size=None,
-             device=None):
-    """Forced wins by continuous fours for the side to move.  boards int8 [B,N,N] or [B,A], players +-1 [B] -> device
-    tensors (length int32 [B], first bool [B,A], nodes int32 [B]): the fewest attacker stones of a VCF of at most
-    `max_attacks` stones (0: none, -1: the node budget ran out), every first move that starts one, and the positions
-    expanded."""
+def _solve(entry, name, boards, players, max_attacks, node_budget, n_in_row, board_size, device):
+    """gmz_vcf_solve / gmz_vct_solve on a batch -> device tensors (length int32 [B], first bool [B,A], nodes int32 [B])."""
     if not torch.cuda.is_available():
-        raise _lib.GmzError("find_vcf needs a CUDA device (there is no CPU fallback)")
+        raise _lib.GmzError(f"{name} needs a CUDA device (there is no CPU fallback)")
     lib = _lib.load()
     dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
     b = torch.as_tensor(boards).to(device=dev, dtype=torch.int8)
@@ -153,23 +150,21 @@ def find_vcf(boards, players, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n
     nodes = torch.empty(B, dtype=torch.int32, device=dev)
     first = torch.empty((B, 6), dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):
-        check(lib.gmz_vcf_solve(C.c_void_p(b.data_ptr()), C.c_void_p(p.data_ptr()), B, N,
-                                int(config.N_IN_ROW if n_in_row is None else n_in_row), int(max_attacks), int(node_budget),
-                                C.c_void_p(length.data_ptr()), C.c_void_p(first.data_ptr()), C.c_void_p(nodes.data_ptr()),
-                                C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "gmz_vcf_solve")
+        check(getattr(lib, entry)(C.c_void_p(b.data_ptr()), C.c_void_p(p.data_ptr()), B, N,
+                                  int(config.N_IN_ROW if n_in_row is None else n_in_row), int(max_attacks), int(node_budget),
+                                  C.c_void_p(length.data_ptr()), C.c_void_p(first.data_ptr()), C.c_void_p(nodes.data_ptr()),
+                                  C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), entry)
     bits = (first.unsqueeze(-1) >> torch.arange(64, device=dev)) & 1
     return length, bits.reshape(B, 6 * 64)[:, :A].bool(), nodes
 
 
-def vcf_record_flags(records, board_size, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None):
-    """The VCF twin of record_flags: packed move records (uint8 device tensor [M, stride], a trajectory.PackedGames
-    block or a stretch of the DeviceReplayBuffer ring) solved where they lie for the side in each record's to_move ->
-    uint8 [M] (bits VCF_AVAILABLE, PLAYED_VCF = the played action starts a VCF, VCF_UNKNOWN = the budget ran out)."""
+def _solver_flags(entry, name, records, board_size, max_attacks, node_budget, n_in_row):
+    """gmz_records_vcf / gmz_records_vct on packed move records where they lie -> uint8 [M] flags."""
     lib = _lib.load()
     N = int(board_size)
     stride = int(lib.gmz_move_record_bytes(N))
     if not torch.is_tensor(records) or records.device.type != "cuda":
-        raise _lib.GmzError("vcf_record_flags needs the records in a CUDA tensor (there is no CPU fallback)")
+        raise _lib.GmzError(f"{name} needs the records in a CUDA tensor (there is no CPU fallback)")
     if records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != stride or not records.is_contiguous():
         raise ValueError(f"records must be a contiguous uint8 tensor [M, {stride}] of {N}x{N} move records")
     M = int(records.shape[0])
@@ -177,22 +172,72 @@ def vcf_record_flags(records, board_size, max_attacks=VCF_ATTACKS, node_budget=V
     if M == 0:
         return out
     with torch.cuda.device(records.device):
-        check(lib.gmz_records_vcf(C.c_void_p(records.data_ptr()), M, N, int(config.N_IN_ROW if n_in_row is None else n_in_row),
+        check(getattr(lib, entry)(C.c_void_p(records.data_ptr()), M, N, int(config.N_IN_ROW if n_in_row is None else n_in_row),
                                   int(max_attacks), int(node_budget), C.c_void_p(out.data_ptr()),
-                                  C.c_void_p(torch.cuda.current_stream(records.device).cuda_stream)), "gmz_records_vcf")
+                                  C.c_void_p(torch.cuda.current_stream(records.device).cuda_stream)), entry)
     return out
+
+
+def _missed_forced(flags_fn, packed, max_attacks, node_budget, n_in_row):
+    """Per game of a PackedGames: the records whose flags have bit 0 (a forced win) without bit 1 (the move played
+    starts one)."""
+    rec, game = _game_records(packed)
+    out = torch.zeros(len(packed), dtype=torch.int64, device=rec.device)
+    if rec.shape[0] == 0:
+        return out
+    flags = flags_fn(rec, packed.N, max_attacks, node_budget, n_in_row)
+    out.index_add_(0, game, ((flags & (VCF_AVAILABLE | PLAYED_VCF)) == VCF_AVAILABLE).to(torch.int64))
+    return out
+
+
+def find_vcf(boards, players, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None, board_size=None,
+             device=None):
+    """Forced wins by continuous fours for the side to move.  boards int8 [B,N,N] or [B,A], players +-1 [B] -> device
+    tensors (length int32 [B], first bool [B,A], nodes int32 [B]): the fewest attacker stones of a VCF of at most
+    `max_attacks` stones (0: none, -1: the node budget ran out), every first move that starts one, and the positions
+    expanded."""
+    return _solve("gmz_vcf_solve", "find_vcf", boards, players, max_attacks, node_budget, n_in_row, board_size, device)
+
+
+def vcf_record_flags(records, board_size, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None):
+    """The VCF twin of record_flags: packed move records (uint8 device tensor [M, stride], a trajectory.PackedGames
+    block or a stretch of the DeviceReplayBuffer ring) solved where they lie for the side in each record's to_move ->
+    uint8 [M] (bits VCF_AVAILABLE, PLAYED_VCF = the played action starts a VCF, VCF_UNKNOWN = the budget ran out)."""
+    return _solver_flags("gmz_records_vcf", "vcf_record_flags", records, board_size, max_attacks, node_budget, n_in_row)
 
 
 def missed_vcf_counts(packed, max_attacks=VCF_ATTACKS, node_budget=VCF_BUDGET, n_in_row=None):
     """Per game of a trajectory.PackedGames, in `packed.table` order: int64 [len(packed)] on the device, the moves at
     which the mover had a VCF of at most `max_attacks` stones and played a move that does not start one."""
-    rec, game = _game_records(packed)
-    out = torch.zeros(len(packed), dtype=torch.int64, device=rec.device)
-    if rec.shape[0] == 0:
-        return out
-    flags = vcf_record_flags(rec, packed.N, max_attacks, node_budget, n_in_row)
-    out.index_add_(0, game, ((flags & (VCF_AVAILABLE | PLAYED_VCF)) == VCF_AVAILABLE).to(torch.int64))
-    return out
+    return _missed_forced(vcf_record_flags, packed, max_attacks, node_budget, n_in_row)
+
+
+# Forced wins through threats of three: the VCT solver (include/gmz.h gmz_vct_solve).  Its flag bits are the VCF ones.
+# Defaults from profiles/r12_vct.json (one B200, 1000 W limit), on 100,000 15x15 E0 self-play records: a 5,000-node
+# budget cuts 22.0 % of them at 23.3 k positions/s, a 20,000-node budget still cuts 21.0 % at 6.2 k/s; max_attacks 16
+# cuts more than 8 (22.7 % against 22.0 % at 5,000 nodes).
+VCT_ATTACKS, VCT_BUDGET = 8, 5_000
+
+
+def find_vct(boards, players, max_attacks=VCT_ATTACKS, node_budget=VCT_BUDGET, n_in_row=None, board_size=None,
+             device=None):
+    """Forced wins by threats of three or four (VCT) for the side to move, as find_vcf: device tensors (length int32
+    [B], first bool [B,A], nodes int32 [B]) -- the fewest attacker stones, forced blocks included, of a VCT of at most
+    `max_attacks` stones (0: none, -1: the node budget ran out), every first move that starts one, and the positions
+    expanded.  Every VCF is a VCT, so it finds at least what find_vcf finds where neither is cut."""
+    return _solve("gmz_vct_solve", "find_vct", boards, players, max_attacks, node_budget, n_in_row, board_size, device)
+
+
+def vct_record_flags(records, board_size, max_attacks=VCT_ATTACKS, node_budget=VCT_BUDGET, n_in_row=None):
+    """The VCT twin of vcf_record_flags -> uint8 [M] (bits VCF_AVAILABLE = the mover had a VCT, PLAYED_VCF = the played
+    action starts one, VCF_UNKNOWN = the budget ran out)."""
+    return _solver_flags("gmz_records_vct", "vct_record_flags", records, board_size, max_attacks, node_budget, n_in_row)
+
+
+def missed_vct_counts(packed, max_attacks=VCT_ATTACKS, node_budget=VCT_BUDGET, n_in_row=None):
+    """Per game of a trajectory.PackedGames, in `packed.table` order: int64 [len(packed)] on the device, the moves at
+    which the mover had a VCT of at most `max_attacks` stones and played a move that does not start one."""
+    return _missed_forced(vct_record_flags, packed, max_attacks, node_budget, n_in_row)
 
 
 class SelfPlayStats:

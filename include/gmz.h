@@ -423,6 +423,42 @@ int gmz_vcf_solve(const int8_t *boards, const int8_t *players, int batch, int bo
 int gmz_records_vcf(const void *records, int64_t n_records, int board_size, int n_in_row, int max_attacks, int node_budget,
                     uint8_t *out_flags, gmz_stream stream);
 
+/* ---- forced wins: VCT (victory by threats of three) solver ---- */
+/* The VCF terms stay.  X attacks and is to move at the root, Y defends; C_X(B) / C_Y(B) are X's / Y's completion cells.
+ * When C_X(B) is empty, F2(B) = the empty cells f where an X stone leaves |C_X| >= 2 (an open four or a double four).
+ * FOUR MOVE of X: an empty m with C_X(B+X@m) non-empty.  THREE MOVE: an empty m with C_X(B+X@m) empty and F2(B+X@m)
+ * non-empty.  THREAT MOVE: either.  L counts X stones, forced blocks included.  Each xnode / ynode call expands one
+ * position: nodes == node_budget cuts it, else nodes += 1, then:
+ *   xnode(B, L), X to move: 1. C_X non-empty: true.  2. L <= 1: refused (a "refusal"), false.  3. C_Y empty and F2
+ *     non-empty: true.  4. |C_Y| >= 2: false.  5. The threat moves in ascending order -- if |C_Y| = 1 only Y's
+ *     completion cell, and only if it is a threat move -- each m tried as ynode(B+X@m, L - 1): the first true returns
+ *     true.  6. Otherwise false.
+ *   ynode(B, L), Y to move (C_Y is empty here): 1. |C_X| >= 2: true.  2. |C_X| = 1 at c: Y must play c; false if that
+ *     stone completes a Y run or fills the board, else xnode(B+Y@c, L).  3. F2 empty: false.  4. L < 2: refused,
+ *     false.  5. The replies R = D | K in ascending order: D = the empty d with C_X(B+Y@d) and F2(B+Y@d) both empty,
+ *     K = the empty k with C_Y(B+Y@k) non-empty (counter-fours).  After Y plays r: the board full, false; |C_Y| >= 2,
+ *     false; |C_Y| = 1 at c', X blocks c' -- the board then full, false, else ynode(...+X@c', L - 1); else
+ *     xnode(..., L).  The first false returns false.  6. Every reply true, or R empty: true.
+ *   Root (1 node): C_X non-empty: length 1, first = C_X.  max_attacks = 1: length 0.  C_Y empty and F2 non-empty:
+ *     length 2, first = F2.  |C_Y| >= 2: length 0.  Else the root's threat moves (restricted as in xnode 5) in
+ *     ascending order, each by iterative deepening: ynode(B+X@m, L - 1) for L = 2 ... max_attacks, stopping at the
+ *     first true or after an iteration without a refusal.  length = the least successful L (0: none), first = every
+ *     candidate that succeeded.  A budget cut: length -1, first empty, nodes = node_budget.
+ * Guarantees: length > 0 means X wins against every defence within length stones (a Y move outside R leaves X a
+ * completion cell or an F2 cell while Y has no completion cell).  Every VCF is a VCT: for the same max_attacks and
+ * neither search cut, a VCF length > 0 implies 0 < VCT length <= VCF length, and when the root has no completion cell
+ * and F2 is empty every VCF first move is a VCT first move.  No Renju or exact-five rules, no threat weaker than a
+ * three, no proof-number search.
+ * Limits: 1 <= max_attacks <= 32 (the shared-memory stack holds 2 * max_attacks plies), node_budget >= 1,
+ * n_in_row >= 1, 1 <= board_size <= GMZ_MAX_BOARD; anything else is refused.  Arguments, outputs and batch = 0 as
+ * gmz_vcf_solve. */
+int gmz_vct_solve(const int8_t *boards, const int8_t *players, int batch, int board_size, int n_in_row, int max_attacks,
+                  int node_budget, int32_t *out_length, uint64_t *out_first, int32_t *out_nodes, gmz_stream stream);
+/* The VCT solver on packed move records, as gmz_records_vcf: out_flags bit 0 the mover had a VCT, bit 1 the played
+ * action is in `first`, bit 2 the budget was cut. */
+int gmz_records_vct(const void *records, int64_t n_records, int board_size, int n_in_row, int max_attacks, int node_budget,
+                    uint8_t *out_flags, gmz_stream stream);
+
 /* ---- prioritized replay: SumTree (replay_buffer.py:4-106) ------------------- */
 /* tree f64 [2*capacity-1] lives in caller memory, 1 <= capacity <= 2^32 (all three calls refuse
  * any other capacity before looking at n / batch).  Sequential reference semantics are preserved
